@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SLOD offline phase (BASELINE.json metric: SLOD basis patches/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over the whole synthetic problem: per-patch basis computation
 (source/LOD.cc:296-768) for every patch, then the coarse stiffness matrix (source/LOD.cc:860-973).
@@ -13,6 +13,12 @@ the coarse matrix and one of the K row blocks after it; timing = max over ranks 
 value : patches/s with the coefficient already resident in HBM (device-buffer entry points).
 e2e   : the same through the host-buffer C ABI (slod_set_coefficient -> slod_compute_basis ->
         slod_assemble_coarse -> slod_get_coarse_csr + slod_get_all_basis), host<->device copies inside the timed region.
+
+--dump-outputs DIR writes what the timed path computed in its last step (see dump_outputs) so that two builds can be
+compared output for output on identical, seeded inputs.
+
+bench.py writes nothing into the repository (it may be read-only): it runs the libraries that __graft_entry__.build()
+left in the tree, so rebuild after changing the CUDA sources.
 """
 from __future__ import annotations
 
@@ -27,6 +33,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # before the project's modules are imported: no __pycache__ in the repository
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -257,6 +264,39 @@ def config_of(w, wname):
             "parallelism": "patches"}
 
 
+DUMP_PATCHES = 1024       # patches sampled by --dump-outputs (all of them on smaller meshes)
+DUMP_SEED = 20261020
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ctx, phi, aphi, K):
+    """Write the outputs of the last timed step for a fixed, seeded sample of patches (the full arrays exceed 1 GB on
+    the default workload), all float64:
+      patch_ids.npy [P]             sampled patch ids, ascending
+      phi.npy       [P, s, F]       basis functions; F = largest n_fine of the sample, zero past each patch's n_fine
+      aphi.npy      [P, s, F]       A * basis functions, same layout
+      K_ell.npy     [P * s, W]      block-ELL rows spacedim*patch + comp of the coarse matrix (layout: include/slod.h)"""
+    import torch
+    n, s = ctx.n_patches, phi.shape[1]
+    rs = np.random.default_rng(DUMP_SEED)
+    ids = np.sort(rs.choice(n, size=min(n, DUMP_PATCHES), replace=False))
+    nf = np.array([ctx.patch_info(int(p))["n_fine"] for p in ids])
+    width = int(nf.max())
+    keep = torch.from_numpy(np.arange(width)[None, :] < nf[:, None]).to(phi.device)[:, None, :]
+    sel = torch.from_numpy(ids).to(phi.device)
+    rows = torch.from_numpy((ids[:, None] * s + np.arange(s)[None, :]).ravel()).to(K.device)
+    arrays = {"patch_ids": ids.astype(np.float64),
+              "phi": torch.where(keep, phi[sel, :, :width], 0.0).cpu().numpy(),
+              "aphi": torch.where(keep, aphi[sel, :, :width], 0.0).cpu().numpy(),
+              "K_ell": K[rows].cpu().numpy()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------------
 def _dbg(*a):
     if os.environ.get("SLOD_BENCH_DEBUG"):
@@ -272,7 +312,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (one GPU only)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w, args.workload)
@@ -281,10 +325,11 @@ def main():
     import torch
     import torch.distributed as dist
     pkg = importlib.import_module("dealii-slod_b200")
-    pkg.build_library()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single-process run: phi is not gathered across ranks")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (no CPU fallback)")
     torch.cuda.set_device(local)
@@ -343,6 +388,8 @@ def main():
         barrier()
     ms_total = e0.elapsed_time(e1)
     _dbg("timed done", ms_total)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ctx, phi, aphi, K)
     launches = ctx.launch_count - l0
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
