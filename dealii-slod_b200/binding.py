@@ -29,7 +29,8 @@ EXPORTS = [
     "slod_free_host", "slod_fine_size", "slod_coarse_rhs", "slod_coarse_solve", "slod_prolongate",
     "slod_fem_solve", "slod_fine_norms", "slod_synchronize", "slod_measure_fp64_peak", "slod_owned_range",
     "slod_comm_unique_id", "slod_comm_init", "slod_offline_distributed", "slod_save_state", "slod_load_state",
-    "slod_fine_norms_reference", "slod_set_host_outputs",
+    "slod_fine_norms_reference", "slod_set_host_outputs", "slod_coarse_rhs_batch", "slod_coarse_solve_batch",
+    "slod_prolongate_batch",
 ]
 
 
@@ -73,6 +74,9 @@ def load_library(path=None):
     lib.slod_coarse_rhs.argtypes = [vp, P(dbl), P(dbl)]
     lib.slod_coarse_solve.argtypes = [vp, P(dbl), P(dbl), i32, dbl, dbl, P(i32), P(dbl)]
     lib.slod_prolongate.argtypes = [vp, P(dbl), P(dbl)]
+    lib.slod_coarse_rhs_batch.argtypes = [vp, i32, P(dbl), P(dbl)]
+    lib.slod_coarse_solve_batch.argtypes = [vp, i32, P(dbl), P(dbl), i32, dbl, dbl, P(i32), P(dbl)]
+    lib.slod_prolongate_batch.argtypes = [vp, i32, P(dbl), P(dbl)]
     lib.slod_fem_solve.argtypes = [vp, P(dbl), P(dbl), i32, dbl, dbl, P(i32), P(dbl)]
     lib.slod_fine_norms.argtypes = [vp, P(dbl), P(dbl), P(dbl), P(dbl)]
     lib.slod_get_patch_info.argtypes = [vp, i64] + [P(i32)] * 6 + [P(i32), P(i32)]
@@ -331,6 +335,40 @@ class SlodContext:
             raise ValueError("coarse vector has the wrong size")
         out = np.empty(self.n_fine)
         self._ck(self.lib.slod_prolongate(self.h, _dp(u), _dp(out)))
+        return out
+
+    # -- batched online phase: k vectors per call, one per row of a (k, n) array --
+    def _block(self, a, n, what):
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if a.ndim != 2 or a.shape[0] < 1 or a.shape[1] != n:
+            raise ValueError(f"{what} must be a 2-D array of shape (k, {n}) with k >= 1, got {a.shape}")
+        return a
+
+    # reuse: as in all_basis (benchmark loops: the output block of the previous call of the same shape is overwritten)
+    def coarse_rhs_batch(self, F, reuse=False):
+        """B = C^T F row by row: F (k, n_fine) -> (k, n_coarse)."""
+        f = self._block(F, self.n_fine, "fine block")
+        b = self._out("rhs_batch", (f.shape[0], self.n_patches * self.s), reuse=reuse)
+        self._ck(self.lib.slod_coarse_rhs_batch(self.h, f.shape[0], _dp(f), _dp(b)))
+        return b
+
+    def coarse_solve_batch(self, B, max_steps=10000, tolerance=1e-10, reduction=1e-10, reuse=False):
+        """Per-row CG: B (k, n_coarse) -> (U (k, n_coarse), steps int32[k], residual[k]); raises SlodError
+        (SLOD_ERR_NUMERIC) when a row does not converge."""
+        b = self._block(B, self.n_patches * self.s, "coarse block")
+        k = b.shape[0]
+        u = self._out("u_batch", b.shape, reuse=reuse)
+        steps = self._out("steps_batch", k, np.int32, reuse=reuse)
+        res = self._out("res_batch", k, reuse=reuse)
+        self._ck(self.lib.slod_coarse_solve_batch(self.h, k, _dp(b), _dp(u), max_steps, tolerance, reduction,
+                                                  steps.ctypes.data_as(C.POINTER(C.c_int32)), _dp(res)))
+        return u, steps, res
+
+    def prolongate_batch(self, U, reuse=False):
+        """U_fine = C U row by row: U (k, n_coarse) -> (k, n_fine)."""
+        u = self._block(U, self.n_patches * self.s, "coarse block")
+        out = self._out("uf_batch", (u.shape[0], self.n_fine), reuse=reuse)
+        self._ck(self.lib.slod_prolongate_batch(self.h, u.shape[0], _dp(u), _dp(out)))
         return out
 
     # -- fine-scale reference problem (assemble_and_solve_fem_problem, source/LOD.cc:1004-1094) and norms (:1252) --

@@ -103,6 +103,8 @@ struct slod_ctx {
   bool coarse_timing_pending = false;
   double *d_online = nullptr;    // scratch of the online / fine-problem entry points, allocated on first use
   size_t online_doubles = 0;
+  double *d_batch = nullptr;     // scratch of the batched online entry points (one group of kBatch columns)
+  size_t batch_doubles = 0;
   double *d_val = nullptr;
   int64_t csr_nnz = 0;
   // multi-GPU: (a) n_gpus > 1: this handle is rank 0 and owns one sub-handle per further device; (b) slod_comm_init
@@ -400,7 +402,7 @@ void free_dev(slod_ctx *c) {
     p = nullptr;
   };
   F(c->d_coef); F(c->d_phi); F(c->d_aphi); F(c->d_Kell); F(c->d_diag); F(c->d_status);
-  F(c->d_perm); F(c->d_val); F(c->d_online);
+  F(c->d_perm); F(c->d_val); F(c->d_online); F(c->d_batch);
   free_workspace(c);
 }
 
@@ -1750,6 +1752,155 @@ int slod_prolongate(slod_ctx *ctx, const double *u_coarse, double *u_fine) {
   if (e == cudaSuccess) e = cudaStreamSynchronize(0);
   ctx->launches += 1;
   if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_prolongate: ") + cudaGetErrorString(e));
+  return SLOD_OK;
+}
+
+// ---- batched online phase: groups of at most kBatch right-hand sides (online_batch.cuh) ----
+// One scratch block, allocated on first use and regrown when too small; its size depends on kBatch, not on n_rhs:
+// [fine staging | fine interleaved | coarse staging | coarse interleaved a | b | CG workspace].  A group's host block
+// ([kb][n], contiguous in the caller's [n_rhs][n] array) is copied in one piece to the staging block and transposed on
+// the device; results go the other way.
+struct BatchScratch {
+  double *fine_stage, *fine, *coarse_stage, *coarse_a, *coarse_b, *work;
+};
+static int batch_scratch(slod_ctx *ctx, BatchScratch *b) {
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const size_t nc = (size_t)ctx->n_patches * ctx->P.s;
+  const size_t need = 2 * (size_t)kBatch * n_fine + 3 * (size_t)kBatch * nc + cg_multi_workspace_doubles((int)nc) + 8;
+  if (ctx->batch_doubles < need) {
+    if (ctx->d_batch) cudaFree(ctx->d_batch);
+    ctx->d_batch = nullptr;
+    ctx->batch_doubles = 0;
+    CK(cudaMalloc(&ctx->d_batch, sizeof(double) * need));
+    ctx->batch_doubles = need;
+  }
+  double *p = ctx->d_batch;
+  b->fine_stage = p;
+  b->fine = p + (size_t)kBatch * n_fine;
+  b->coarse_stage = b->fine + (size_t)kBatch * n_fine;
+  b->coarse_a = b->coarse_stage + (size_t)kBatch * nc;
+  b->coarse_b = b->coarse_a + (size_t)kBatch * nc;
+  b->work = b->coarse_b + (size_t)kBatch * nc;
+  return SLOD_OK;
+}
+
+int slod_coarse_rhs_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, double *rhs_coarse) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  if (!ctx->basis_done) return fail(ctx, SLOD_ERR_STATE, "slod_compute_basis has not run");
+  if (!f_fine || !rhs_coarse) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  if (n_rhs < 1) return fail(ctx, SLOD_ERR_INVALID, "n_rhs must be at least 1");
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const size_t nc = (size_t)ctx->n_patches * ctx->P.s;
+  BatchScratch w{};
+  int rc = batch_scratch(ctx, &w);
+  if (rc) return rc;
+  cudaError_t e = cudaSuccess;
+  for (int j0 = 0; j0 < n_rhs && e == cudaSuccess; j0 += kBatch) {
+    const int kb = std::min(kBatch, n_rhs - j0);
+    e = cudaMemcpyAsync(w.fine_stage, f_fine + (size_t)j0 * n_fine, sizeof(double) * kb * (size_t)n_fine,
+                        cudaMemcpyHostToDevice, 0);
+    if (e == cudaSuccess) e = launch_interleave(0, n_fine, kb, w.fine_stage, w.fine, true);
+    if (e == cudaSuccess)
+      e = launch_coarse_rhs_multi(0, (int)ctx->n_patches, ctx->P.s, kb, ctx->d_phi, w.fine, w.coarse_a, ctx->P.NfMax);
+    if (e == cudaSuccess) e = launch_interleave(0, (long long)nc, kb, w.coarse_a, w.coarse_stage, false);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(rhs_coarse + (size_t)j0 * nc, w.coarse_stage, sizeof(double) * kb * nc,
+                          cudaMemcpyDeviceToHost, 0);
+    ctx->launches += 3;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_coarse_rhs_batch: ") + cudaGetErrorString(e));
+  return SLOD_OK;
+}
+
+int slod_coarse_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *rhs_coarse, double *u_coarse,
+                            int32_t max_steps, double tolerance, double reduction, int32_t *steps, double *residual) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  if (!ctx->coarse_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse has not run");
+  if (!rhs_coarse || !u_coarse) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  if (n_rhs < 1) return fail(ctx, SLOD_ERR_INVALID, "n_rhs must be at least 1");
+  if (max_steps < 0 || !(tolerance >= 0.0) || !(reduction >= 0.0))
+    return fail(ctx, SLOD_ERR_INVALID, "solver control: max_steps, tolerance and reduction must be non-negative");
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  const int nrows = (int)(ctx->n_patches * ctx->P.s);
+  BatchScratch w{};
+  int rc = batch_scratch(ctx, &w);
+  if (rc) return rc;
+  std::vector<int> st_steps(n_rhs, 0), flag(n_rhs, 0);
+  std::vector<double> res(n_rhs, 0.0);
+  cudaError_t e = cudaSuccess;
+  long long n_launch = 0;
+  for (int j0 = 0; j0 < n_rhs && e == cudaSuccess; j0 += kBatch) {
+    const int kb = std::min(kBatch, n_rhs - j0);
+    e = cudaMemcpyAsync(w.coarse_stage, rhs_coarse + (size_t)j0 * nrows, sizeof(double) * kb * (size_t)nrows,
+                        cudaMemcpyHostToDevice, 0);
+    if (e == cudaSuccess) e = launch_interleave(0, nrows, kb, w.coarse_stage, w.coarse_a, true);
+    if (e == cudaSuccess)
+      e = run_cg_multi(0, nrows, ctx->d_Kell, kb, w.coarse_a, w.coarse_b, w.work, max_steps, tolerance, reduction,
+                       &st_steps[j0], &res[j0], &flag[j0], &n_launch);
+    if (e == cudaSuccess) e = launch_interleave(0, nrows, kb, w.coarse_b, w.coarse_stage, false);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(u_coarse + (size_t)j0 * nrows, w.coarse_stage, sizeof(double) * kb * (size_t)nrows,
+                          cudaMemcpyDeviceToHost, 0);
+    n_launch += 2;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  ctx->launches += n_launch;
+  for (int j = 0; j < n_rhs; ++j) {
+    if (steps) steps[j] = st_steps[j];
+    if (residual) residual[j] = res[j];
+  }
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_coarse_solve_batch: ") + cudaGetErrorString(e));
+  for (int j = 0; j < n_rhs; ++j) {
+    if (flag[j] == 1) continue;
+    char buf[200];
+    if (flag[j] == 2)
+      std::snprintf(buf, sizeof buf, "coarse CG broke down in column %d after %d steps (residual %.3e): the coarse "
+                    "matrix is not positive definite", j, st_steps[j], res[j]);
+    else
+      std::snprintf(buf, sizeof buf, "coarse CG did not converge in column %d: %d steps, residual %.3e", j, st_steps[j],
+                    res[j]);
+    return fail(ctx, SLOD_ERR_NUMERIC, buf);   // the first failing column; every column's u / steps / residual is written
+  }
+  return SLOD_OK;
+}
+
+int slod_prolongate_batch(slod_ctx *ctx, int32_t n_rhs, const double *u_coarse, double *u_fine) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  if (!ctx->basis_done) return fail(ctx, SLOD_ERR_STATE, "slod_compute_basis has not run");
+  if (!u_coarse || !u_fine) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  if (n_rhs < 1) return fail(ctx, SLOD_ERR_INVALID, "n_rhs must be at least 1");
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const size_t nc = (size_t)ctx->n_patches * ctx->P.s;
+  BatchScratch w{};
+  int rc = batch_scratch(ctx, &w);
+  if (rc) return rc;
+  cudaError_t e = cudaSuccess;
+  for (int j0 = 0; j0 < n_rhs && e == cudaSuccess; j0 += kBatch) {
+    const int kb = std::min(kBatch, n_rhs - j0);
+    e = cudaMemcpyAsync(w.coarse_stage, u_coarse + (size_t)j0 * nc, sizeof(double) * kb * nc, cudaMemcpyHostToDevice,
+                        0);
+    if (e == cudaSuccess) e = launch_interleave(0, (long long)nc, kb, w.coarse_stage, w.coarse_a, true);
+    if (e == cudaSuccess) e = launch_prolongate_multi(0, n_fine, kb, ctx->d_phi, w.coarse_a, w.fine, ctx->P.NfMax);
+    if (e == cudaSuccess) e = launch_interleave(0, n_fine, kb, w.fine, w.fine_stage, false);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(u_fine + (size_t)j0 * n_fine, w.fine_stage, sizeof(double) * kb * (size_t)n_fine,
+                          cudaMemcpyDeviceToHost, 0);
+    ctx->launches += 3;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_prolongate_batch: ") + cudaGetErrorString(e));
   return SLOD_OK;
 }
 

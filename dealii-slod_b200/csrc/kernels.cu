@@ -1204,6 +1204,7 @@ cudaError_t launch_gather(cudaStream_t st, const double *src, const long long *p
 }
 }  // namespace slod
 #include "online.cuh"
+#include "online_batch.cuh"
 namespace slod {
 
 cudaError_t launch_coarse_rhs(cudaStream_t st, int n_patches, int s, const double *phi, const double *f, double *b,
@@ -1277,6 +1278,77 @@ cudaError_t launch_fine_quadratic_form(cudaStream_t st, int op, long long n_node
   const int nb = (int)((n_nodes + kCgThreads - 1) / kCgThreads);
   *n_partial = nb;
   if (partial) k_fine_apply<<<nb, kCgThreads, 0, st>>>(op, n_nodes, d_coef, x, nullptr, nullptr, partial, nullptr);
+  return cudaGetLastError();
+}
+
+// ---- batched online phase (online_batch.cuh) ----
+cudaError_t launch_interleave(cudaStream_t st, long long n, int kb, const double *src, double *dst, bool to_interleaved) {
+  const long long blocks = (n * kb + 255) / 256;
+  const int grid = (int)(blocks < 148 * 16 ? blocks : 148 * 16);
+  if (to_interleaved) k_interleave<<<grid, 256, 0, st>>>(n, kb, src, dst);
+  else k_deinterleave<<<grid, 256, 0, st>>>(n, kb, src, dst);
+  return cudaGetLastError();
+}
+cudaError_t launch_coarse_rhs_multi(cudaStream_t st, int n_patches, int s, int kb, const double *phi, const double *F,
+                                    double *B, int nf_max) {
+  const int rows = n_patches * s, per = kCgThreads / 32;
+  k_coarse_rhs_multi<<<(rows + per - 1) / per, kCgThreads, 0, st>>>(n_patches, kb, phi, F, B, nf_max);
+  return cudaGetLastError();
+}
+cudaError_t launch_prolongate_multi(cudaStream_t st, long long n_fine, int kb, const double *phi, const double *U,
+                                    double *Uf, int nf_max) {
+  const long long blocks = (n_fine + kCgThreads - 1) / kCgThreads;
+  k_prolongate_multi<<<(int)(blocks < 148 * 16 ? blocks : 148 * 16), kCgThreads, 0, st>>>(n_fine, kb, phi, U, Uf,
+                                                                                          nf_max);
+  return cudaGetLastError();
+}
+// Grids depend on nrows only (never on kb): the partial-sum arrays, and so every column's sums, have the same shape
+// whatever the group holds.
+static int cg_multi_apply_blocks(int nrows) {
+  const int per = kCgThreads / 32, want = (nrows + per - 1) / per;
+  return want < 148 * 8 ? want : 148 * 8;
+}
+size_t cg_multi_workspace_doubles(int nrows) {
+  const size_t nb_apply = cg_multi_apply_blocks(nrows), nb_vec = (nrows + kVecRows - 1) / kVecRows;
+  // R, P, Q | dinv | partial p.q | partial r.z, r.r | states
+  return 3 * (size_t)kBatch * nrows + nrows + kBatch * (nb_apply + 2 * nb_vec) + (kBatch * sizeof(CgState) + 7) / 8;
+}
+// The host loop of run_cg for kb columns: every 16 steps it reads the kb states back (kb x 56 bytes) and stops when all
+// columns are done or at max_steps.
+cudaError_t run_cg_multi(cudaStream_t st, int nrows, const double *Kell, int kb, const double *B, double *X,
+                         double *work, int max_steps, double tol, double reduction, int *steps, double *residual,
+                         int *flag, long long *launches) {
+  const int nb_apply = cg_multi_apply_blocks(nrows), nb_vec = (nrows + kVecRows - 1) / kVecRows;
+  const size_t nv = (size_t)kBatch * nrows;
+  double *R = work, *P = R + nv, *Q = P + nv, *dinv = Q + nv;
+  double *ppq = dinv + nrows, *prz = ppq + (size_t)kBatch * nb_apply, *prr = prz + (size_t)kBatch * nb_vec;
+  CgState *state = reinterpret_cast<CgState *>(prr + (size_t)kBatch * nb_vec);
+  CgState h[kBatch];
+  cudaError_t e;
+  k_cg_init_multi<<<kb, 1024, 0, st>>>(nrows, kb, Kell, B, X, R, P, dinv, state, tol, reduction);
+  *launches += 1;
+  const int check_every = 16;
+  int it = 0;
+  for (;;) {
+    if ((e = cudaMemcpyAsync(h, state, sizeof(CgState) * kb, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
+    bool all = true;
+    for (int j = 0; j < kb; ++j) all = all && h[j].done;
+    if (all || it >= max_steps) break;
+    const int upto = (it + check_every < max_steps) ? it + check_every : max_steps;
+    for (; it < upto; ++it) {
+      k_cg_spmm<<<nb_apply, kCgThreads, 0, st>>>(nrows, kb, Kell, P, Q, ppq, state);
+      k_cg_update_multi<<<nb_vec, kCgThreads, 0, st>>>(nrows, kb, it, P, Q, dinv, X, R, ppq, nb_apply, prz, prr, state);
+      k_cg_direction_multi<<<nb_vec, kCgThreads, 0, st>>>(nrows, kb, it, R, dinv, P, prz, prr, nb_vec, state);
+      *launches += 3;
+    }
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  }
+  for (int j = 0; j < kb; ++j) {
+    steps[j] = h[j].steps;
+    residual[j] = sqrt(h[j].rr);
+    flag[j] = h[j].done;
+  }
   return cudaGetLastError();
 }
 

@@ -148,6 +148,21 @@ size_t cg_workspace_doubles(const CgOperator &A, int nrows);
 cudaError_t run_cg(cudaStream_t st, int nrows, const CgOperator &A, const double *b, double *x, double *work,
                    int max_steps, double tol, double reduction, int *steps, double *residual, int *flag,
                    long long *launches);
+// batched online phase (online_batch.cuh): right-hand sides in groups of at most kBatch columns, interleaved [n][kb].
+// 16: the values of one row form one 128-byte line, and the scratch of a group stays small (about 70 MB of fine
+// vectors at the 32^3-cell workload) whatever the number of right-hand sides.
+constexpr int kBatch = 16;
+// [kb][n] <-> [n][kb]; to_interleaved selects the direction
+cudaError_t launch_interleave(cudaStream_t st, long long n, int kb, const double *src, double *dst, bool to_interleaved);
+cudaError_t launch_coarse_rhs_multi(cudaStream_t st, int n_patches, int s, int kb, const double *phi, const double *F,
+                                    double *B, int nf_max);
+cudaError_t launch_prolongate_multi(cudaStream_t st, long long n_fine, int kb, const double *phi, const double *U,
+                                    double *Uf, int nf_max);
+size_t cg_multi_workspace_doubles(int nrows);
+// per-column CG on the block-ELL matrix for kb <= kBatch interleaved columns; steps / residual / flag: kb entries each
+cudaError_t run_cg_multi(cudaStream_t st, int nrows, const double *Kell, int kb, const double *B, double *X,
+                         double *work, int max_steps, double tol, double reduction, int *steps, double *residual,
+                         int *flag, long long *launches);
 cudaError_t launch_fine_quadratic_form(cudaStream_t st, int op, long long n_nodes, const double *d_coef, const double *x,
                                        double *partial, int *n_partial);
 cudaError_t launch_fine_norms_reference(cudaStream_t st, long long n_cells, int nq, const double *gauss_x,

@@ -150,6 +150,21 @@ int slod_coarse_solve(slod_ctx *ctx, const double *rhs_coarse, double *u_coarse,
                       double reduction, int32_t *steps, double *residual);
 /* lod_solution = C u  (basis_matrix_transposed.vmult(lod_solution, solution), source/LOD.cc:1251). */
 int slod_prolongate(slod_ctx *ctx, const double *u_coarse, double *u_fine);
+/* Batched online phase: n_rhs >= 1 vectors per call, each one contiguous ([n_rhs][n_fine] / [n_rhs][n_coarse]).
+ * Column j of every result is bit-identical to what the same call computes for that vector alone.
+ * The per-vector semantics are those of the three calls above (source/LOD.cc:981, :991-998, :1251): same call-order
+ * checks, same device (the first one of an n_gpus > 1 handle), and they serve handles restored by slod_load_state.
+ * phi and K are read once per group of columns instead of once per vector.  n_rhs < 1 or a NULL buffer ->
+ * SLOD_ERR_INVALID.  The reference solves one system per run; these calls are an extension.
+ * slod_coarse_solve_batch runs one CG per column, each with its own step count and ReductionControl test; a column that
+ * has stopped is no longer updated.  If any column breaks down or does not converge within max_steps the call returns
+ * SLOD_ERR_NUMERIC and slod_last_error names the first such column with its steps and residual; u_coarse, steps and
+ * residual (may be NULL, else [n_rhs]) are written for all columns in every case. */
+int slod_coarse_rhs_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, double *rhs_coarse);
+int slod_coarse_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *rhs_coarse, double *u_coarse,
+                            int32_t max_steps, double tolerance, double reduction,
+                            int32_t *steps /* [n_rhs] or NULL */, double *residual /* [n_rhs] or NULL */);
+int slod_prolongate_batch(slod_ctx *ctx, int32_t n_rhs, const double *u_coarse, double *u_fine);
 
 /* ---- fine-scale reference problem (SURVEY 8f row 2; the solve of LOD::assemble_and_solve_fem_problem,
  * source/LOD.cc:1004-1094, and the norms of compare_lod_with_fem, source/LOD.cc:1252).  Needs only the coefficient.
