@@ -30,7 +30,8 @@ EXPORTS = [
     "slod_fem_solve", "slod_fine_norms", "slod_synchronize", "slod_measure_fp64_peak", "slod_owned_range",
     "slod_comm_unique_id", "slod_comm_init", "slod_offline_distributed", "slod_save_state", "slod_load_state",
     "slod_fine_norms_reference", "slod_set_host_outputs", "slod_coarse_rhs_batch", "slod_coarse_solve_batch",
-    "slod_prolongate_batch",
+    "slod_prolongate_batch", "slod_assemble_coarse_mass", "slod_get_coarse_mass_csr", "slod_l2_project_batch",
+    "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve",
 ]
 
 
@@ -78,6 +79,12 @@ def load_library(path=None):
     lib.slod_coarse_solve_batch.argtypes = [vp, i32, P(dbl), P(dbl), i32, dbl, dbl, P(i32), P(dbl)]
     lib.slod_prolongate_batch.argtypes = [vp, i32, P(dbl), P(dbl)]
     lib.slod_fem_solve.argtypes = [vp, P(dbl), P(dbl), i32, dbl, dbl, P(i32), P(dbl)]
+    lib.slod_assemble_coarse_mass.argtypes = [vp]
+    lib.slod_get_coarse_mass_csr.argtypes = [vp, P(i64), P(i64), P(dbl), P(i64), P(i64)]
+    lib.slod_l2_project_batch.argtypes = [vp, i32, P(dbl), P(dbl), i32, dbl, dbl, P(i32), P(dbl)]
+    lib.slod_heat_solve.argtypes = [vp, P(dbl), P(dbl), dbl, i32, i32, P(dbl), i32, dbl, dbl, P(i32)]
+    lib.slod_heat_solve_batch.argtypes = [vp, i32, P(dbl), P(dbl), dbl, i32, i32, P(dbl), i32, dbl, dbl, P(i32)]
+    lib.slod_fem_heat_solve.argtypes = [vp, P(dbl), P(dbl), dbl, i32, i32, P(dbl), i32, dbl, dbl, P(i32)]
     lib.slod_fine_norms.argtypes = [vp, P(dbl), P(dbl), P(dbl), P(dbl)]
     lib.slod_get_patch_info.argtypes = [vp, i64] + [P(i32)] * 6 + [P(i32), P(i32)]
     lib.slod_get_patch_cells.argtypes = [vp, i64, P(C.c_uint32), P(i32)]
@@ -293,14 +300,17 @@ class SlodContext:
         self._ck(self.lib.slod_assemble_coarse(self.h))
 
     def coarse_csr(self, reuse=False):
+        return self._csr(self.lib.slod_get_coarse_csr, "", reuse)
+
+    def _csr(self, getter, key, reuse):
         nr, nnz = C.c_int64(), C.c_int64()
-        self._ck(self.lib.slod_get_coarse_csr(self.h, None, None, None, C.byref(nr), C.byref(nnz)))
-        rowptr = self._out("rowptr", nr.value + 1, np.int64, reuse=reuse)
-        col = self._out("col", nnz.value, np.int64, reuse=reuse)
-        val = self._out("val", nnz.value, reuse=reuse)
+        self._ck(getter(self.h, None, None, None, C.byref(nr), C.byref(nnz)))
+        rowptr = self._out(key + "rowptr", nr.value + 1, np.int64, reuse=reuse)
+        col = self._out(key + "col", nnz.value, np.int64, reuse=reuse)
+        val = self._out(key + "val", nnz.value, reuse=reuse)
         i64p = C.POINTER(C.c_int64)
-        self._ck(self.lib.slod_get_coarse_csr(self.h, rowptr.ctypes.data_as(i64p), col.ctypes.data_as(i64p),
-                                              _dp(val), C.byref(nr), C.byref(nnz)))
+        self._ck(getter(self.h, rowptr.ctypes.data_as(i64p), col.ctypes.data_as(i64p), _dp(val), C.byref(nr),
+                        C.byref(nnz)))
         return rowptr, col, val
 
     # -- online phase (LOD::solve, source/LOD.cc:975-1001; prolongation :1251) --
@@ -370,6 +380,78 @@ class SlodContext:
         out = self._out("uf_batch", (u.shape[0], self.n_fine), reuse=reuse)
         self._ck(self.lib.slod_prolongate_batch(self.h, u.shape[0], _dp(u), _dp(out)))
         return out
+
+    # -- coarse mass matrix, L2 projection and backward Euler on the SLOD space (an extension of the reference) --
+    def assemble_coarse_mass(self):
+        self._ck(self.lib.slod_assemble_coarse_mass(self.h))
+
+    def coarse_mass_csr(self, reuse=False):
+        """CSR of M_H = C^T M_h C: (rowptr, col, val), the pattern of coarse_csr()."""
+        return self._csr(self.lib.slod_get_coarse_mass_csr, "mass_", reuse)
+
+    def l2_project_batch(self, V, max_steps=10000, tolerance=1e-12, reduction=1e-12, reuse=False):
+        """M_H u = C^T M_h v row by row: V (k, n_fine) -> (U (k, n_coarse), steps int32[k], residual[k])."""
+        v = self._block(V, self.n_fine, "fine block")
+        k = v.shape[0]
+        u = self._out("l2_u", (k, self.n_patches * self.s), reuse=reuse)
+        steps = self._out("l2_steps", k, np.int32, reuse=reuse)
+        res = self._out("l2_res", k, reuse=reuse)
+        self._ck(self.lib.slod_l2_project_batch(self.h, k, _dp(v), _dp(u), max_steps, tolerance, reduction,
+                                                steps.ctypes.data_as(C.POINTER(C.c_int32)), _dp(res)))
+        return u, steps, res
+
+    def _vec_or_none(self, a, n, what):
+        if a is None:
+            return None
+        a = np.ascontiguousarray(a, dtype=np.float64).ravel()
+        if a.size != n:
+            raise ValueError(f"{what} has {a.size} entries, expected {n}")
+        return a
+
+    def heat_solve(self, f_fine, u0_coarse, dt, n_steps, out_every=1, max_steps=10000, tolerance=0.0,
+                   reduction=1e-12):
+        """Backward Euler on the SLOD space (f_fine / u0_coarse may be None: zero).  Returns (U (n_steps // out_every,
+        n_coarse), cg_steps int32[n_steps])."""
+        nc = self.n_patches * self.s
+        f = self._vec_or_none(f_fine, self.n_fine, "fine vector")
+        u0 = self._vec_or_none(u0_coarse, nc, "coarse vector")
+        out = np.empty((max(n_steps // max(out_every, 1), 1), nc))
+        steps = np.zeros(max(n_steps, 1), dtype=np.int32)
+        self._ck(self.lib.slod_heat_solve(self.h, None if f is None else _dp(f), None if u0 is None else _dp(u0), dt,
+                                          n_steps, out_every, _dp(out), max_steps, tolerance, reduction,
+                                          steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out, steps
+
+    def heat_solve_batch(self, F, U0, dt, n_steps, out_every=1, max_steps=10000, tolerance=0.0, reduction=1e-12):
+        """k trajectories at once: F (k, n_fine), U0 (k, n_coarse) (either may be None: zero).  Returns
+        (U (n_steps // out_every, k, n_coarse), cg_steps int32 (n_steps, k))."""
+        nc = self.n_patches * self.s
+        f = None if F is None else self._block(F, self.n_fine, "fine block")
+        u0 = None if U0 is None else self._block(U0, nc, "coarse block")
+        if f is not None and u0 is not None and f.shape[0] != u0.shape[0]:
+            raise ValueError("F and U0 must have the same number of rows")
+        if f is None and u0 is None:
+            raise ValueError("give F or U0 (the number of trajectories)")
+        k = (f if f is not None else u0).shape[0]
+        out = np.empty((max(n_steps // max(out_every, 1), 1), k, nc))
+        steps = np.zeros((max(n_steps, 1), k), dtype=np.int32)
+        self._ck(self.lib.slod_heat_solve_batch(self.h, k, None if f is None else _dp(f),
+                                                None if u0 is None else _dp(u0), dt, n_steps, out_every, _dp(out),
+                                                max_steps, tolerance, reduction,
+                                                steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out, steps
+
+    def fem_heat_solve(self, f_fine, u0_fine, dt, n_steps, out_every=1, max_steps=200000, tolerance=0.0,
+                       reduction=1e-12):
+        """The fine-scale reference trajectory.  Returns (U (n_steps // out_every, n_fine), cg_steps int32[n_steps])."""
+        f = self._vec_or_none(f_fine, self.n_fine, "fine vector")
+        u0 = self._vec_or_none(u0_fine, self.n_fine, "fine vector")
+        out = np.empty((max(n_steps // max(out_every, 1), 1), self.n_fine))
+        steps = np.zeros(max(n_steps, 1), dtype=np.int32)
+        self._ck(self.lib.slod_fem_heat_solve(self.h, None if f is None else _dp(f), None if u0 is None else _dp(u0),
+                                              dt, n_steps, out_every, _dp(out), max_steps, tolerance, reduction,
+                                              steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out, steps
 
     # -- fine-scale reference problem (assemble_and_solve_fem_problem, source/LOD.cc:1004-1094) and norms (:1252) --
     def fem_solve(self, f_fine, max_steps=200000, tolerance=1e-12, reduction=1e-10):

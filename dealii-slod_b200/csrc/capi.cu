@@ -82,7 +82,7 @@ struct slod_ctx {
   int coarse_nu = 0;   // > 0: blocked coarse kernel with this common-box width
   int grid_solve = 0, grid_dense = 0, grid_finish = 0, grid_coarse = 0;
   int bw_max = 0, nb_max = 0;
-  cudaEvent_t ev[10]{};
+  cudaEvent_t ev[12]{};   // [8]..[10]: the coarse mass matrix (slod_get_timings [6], [7])
   std::vector<cudaEvent_t> chunk_ev;   // 5 per chunk of the last run_basis
   size_t chunks_pending = 0;
   bool basis_pending = false;
@@ -107,6 +107,13 @@ struct slod_ctx {
   size_t batch_doubles = 0;
   double *d_val = nullptr;
   int64_t csr_nnz = 0;
+  // heat equation on the SLOD space: M_H in block-ELL form and its CSR values, S = M_H + dt K for the dt of the last
+  // time-stepping call (s_dt == 0: not formed), and the scratch of the time steppers
+  double *d_Mell = nullptr, *d_Mval = nullptr, *d_Sell = nullptr;
+  bool mass_done = false;
+  double s_dt = 0.0;
+  double *d_heat = nullptr;
+  size_t heat_doubles = 0;
   // multi-GPU: (a) n_gpus > 1: this handle is rank 0 and owns one sub-handle per further device; (b) slod_comm_init
   std::vector<slod_ctx *> subs;   // sub-handles of ranks 1 .. n_gpus-1 (owned)
   ncclComm_t comm = nullptr;
@@ -389,6 +396,12 @@ void patch_cells_rel(const Params &P, const Geom &g, std::vector<std::array<int,
   }
 }
 
+// M_H and S are derived from the basis and from K: a new basis, a restored checkpoint or a new K make them stale
+void invalidate_mass(slod_ctx *c) {
+  c->mass_done = false;
+  c->s_dt = 0.0;
+}
+
 int check_patch(const slod_ctx *ctx, int64_t patch) {
   if (!ctx) return SLOD_ERR_INVALID;
   if (patch < 0 || patch >= ctx->n_patches) return fail(ctx, SLOD_ERR_INVALID, "patch id out of range");
@@ -403,6 +416,7 @@ void free_dev(slod_ctx *c) {
   };
   F(c->d_coef); F(c->d_phi); F(c->d_aphi); F(c->d_Kell); F(c->d_diag); F(c->d_status);
   F(c->d_perm); F(c->d_val); F(c->d_online); F(c->d_batch);
+  F(c->d_Mell); F(c->d_Mval); F(c->d_Sell); F(c->d_heat);
   free_workspace(c);
 }
 
@@ -1413,6 +1427,7 @@ int slod_compute_basis(slod_ctx *ctx) {
     CK(cudaMalloc(&ctx->d_aphi, sizeof(double) * n));
   }
   ctx->basis_done = ctx->coarse_done = false;
+  invalidate_mass(ctx);
   if (!ctx->subs.empty()) return multi_basis(ctx);
   int rc = run_basis(ctx, 0, ctx->n_patches, ctx->d_phi, ctx->d_aphi, 0);
   if (rc) return rc;
@@ -1601,6 +1616,7 @@ int slod_assemble_coarse(slod_ctx *ctx) {
   // the matrix is stream ordered behind them, and an execution error surfaces at that consumer's synchronisation.
   int rc = build_csr_cache(ctx);   // first call only: host-side integer geometry, before the kernels are in flight
   if (rc) return rc;
+  invalidate_mass(ctx);
   if (!ctx->subs.empty())
     rc = multi_coarse(ctx);   // row blocks on N devices + NCCL all-gather; the matrix is complete on return
   else
@@ -1612,8 +1628,9 @@ int slod_assemble_coarse(slod_ctx *ctx) {
   return SLOD_OK;
 }
 
-int slod_get_coarse_csr(const slod_ctx *cctx, int64_t *rowptr, int64_t *col, double *val, int64_t *n_rows,
-                        int64_t *nnz) {
+// CSR of K (mass == false) or of M_H (mass == true): the same pattern, values gathered on the device
+static int get_csr(const slod_ctx *cctx, bool mass, int64_t *rowptr, int64_t *col, double *val, int64_t *n_rows,
+                   int64_t *nnz) {
   if (!cctx) return SLOD_ERR_INVALID;
   slod_ctx *ctx = const_cast<slod_ctx *>(cctx);   // the pattern cache is filled lazily
   if (!rowptr) {
@@ -1625,16 +1642,23 @@ int slod_get_coarse_csr(const slod_ctx *cctx, int64_t *rowptr, int64_t *col, dou
     return ell_to_csr(ctx, nullptr, nullptr, nullptr, nullptr, n_rows, nnz);
   }
   NEED_DEVICE();
-  if (!ctx->coarse_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse has not run");
+  if (!mass && !ctx->coarse_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse has not run");
+  if (mass && !ctx->mass_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse_mass has not run");
   if (!col || !val) return fail(ctx, SLOD_ERR_INVALID, "null output buffer");
   CK(cudaSetDevice(ctx->device));
   if (n_rows) *n_rows = (int64_t)ctx->csr_rowptr.size() - 1;
   if (nnz) *nnz = ctx->csr_nnz;
-  CK(cudaMemcpyAsync(val, ctx->d_val, sizeof(double) * (size_t)ctx->csr_nnz, cudaMemcpyDeviceToHost, 0));
+  CK(cudaMemcpyAsync(val, mass ? ctx->d_Mval : ctx->d_val, sizeof(double) * (size_t)ctx->csr_nnz,
+                     cudaMemcpyDeviceToHost, 0));
   std::memcpy(rowptr, ctx->csr_rowptr.data(), sizeof(int64_t) * ctx->csr_rowptr.size());
   parallel_copy(col, ctx->csr_col.data(), sizeof(int64_t) * ctx->csr_col.size());
   CK(cudaStreamSynchronize(0));
   return SLOD_OK;
+}
+
+int slod_get_coarse_csr(const slod_ctx *ctx, int64_t *rowptr, int64_t *col, double *val, int64_t *n_rows,
+                        int64_t *nnz) {
+  return get_csr(ctx, false, rowptr, col, val, n_rows, nnz);
 }
 
 // ---- online phase on the handle's own basis and coarse matrix (SURVEY 8f row 1) ----
@@ -2059,6 +2083,395 @@ int slod_fine_norms_reference(slod_ctx *ctx, const double *v_fine, double *l2, d
   return SLOD_OK;
 }
 
+// ---- heat equation on the SLOD space: coarse mass matrix, L2 projection, backward Euler ----
+// M_H = C^T (M_h C) is formed like K: k_mass_apply writes M_h phi in the layout of A phi (a temporary the size of A phi)
+// and the coarse-matrix kernel takes it in place of A phi.  The time steppers solve (M_H + dt K) u^k = M_H u^{k-1} + dt b
+// in increment form, r = dt (b - K u^{k-1}), S delta = r, u^k = u^{k-1} + delta: the CG drivers start from zero, which is
+// the previous step here.
+int slod_assemble_coarse_mass(slod_ctx *ctx) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  if (!ctx->basis_done) return fail(ctx, SLOD_ERR_STATE, "slod_compute_basis has not run");
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  int rc = build_csr_cache(ctx);
+  if (rc) return rc;
+  invalidate_mass(ctx);
+  const Params &P = ctx->P;
+  const size_t nb = (size_t)ctx->n_patches * P.s * P.NfMax, nk = (size_t)ctx->n_patches * P.s * P.ell_width;
+  if (!ctx->d_Mell) CK(cudaMalloc(&ctx->d_Mell, sizeof(double) * nk));
+  if (!ctx->d_Mval) CK(cudaMalloc(&ctx->d_Mval, sizeof(double) * std::max<size_t>(1, (size_t)ctx->csr_nnz)));
+  double *d_mphi = nullptr;
+  CK(cudaMalloc(&d_mphi, sizeof(double) * nb));
+  cudaError_t e = cudaEventRecord(ctx->ev[8], 0);
+  if (e == cudaSuccess) e = launch_mass_apply(0, (int)ctx->n_patches, P.s, ctx->d_phi, d_mphi, P.NfMax);
+  if (e == cudaSuccess) e = cudaEventRecord(ctx->ev[9], 0);
+  if (e == cudaSuccess) {
+    if (ctx->coarse_nu > 0)
+      e = launch_coarse_blocked(P.dim, P.s, ctx->n_sm, ctx->smem_coarse_blk, 0, 0, (int)ctx->n_patches, ctx->d_phi,
+                                d_mphi, ctx->d_Mell, ctx->fl, ctx->coarse_nu);
+    else
+      e = launch_coarse((int)std::min<int64_t>(ctx->n_patches, ctx->grid_coarse), ctx->smem_coarse, 0, 0,
+                        (int)ctx->n_patches, ctx->d_phi, d_mphi, ctx->d_Mell, ctx->fl);
+  }
+  if (e == cudaSuccess) e = cudaEventRecord(ctx->ev[10], 0);
+  if (e == cudaSuccess) e = launch_gather(0, ctx->d_Mell, ctx->d_perm, ctx->d_Mval, ctx->csr_nnz);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  ctx->launches += 3;
+  cudaFree(d_mphi);
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_assemble_coarse_mass: ") + cudaGetErrorString(e));
+  float ms[2] = {0, 0};
+  CK(cudaEventElapsedTime(&ms[0], ctx->ev[8], ctx->ev[9]));
+  CK(cudaEventElapsedTime(&ms[1], ctx->ev[9], ctx->ev[10]));
+  ctx->tm.ms[6] = ms[0];
+  ctx->tm.ms[7] = ms[1];
+  ctx->mass_done = true;
+  return SLOD_OK;
+}
+
+int slod_get_coarse_mass_csr(const slod_ctx *ctx, int64_t *rowptr, int64_t *col, double *val, int64_t *n_rows,
+                             int64_t *nnz) {
+  return get_csr(ctx, true, rowptr, col, val, n_rows, nnz);
+}
+
+static int check_solver_control(slod_ctx *ctx, int32_t max_steps, double tolerance, double reduction) {
+  if (max_steps < 0 || !(tolerance >= 0.0) || !(reduction >= 0.0))
+    return fail(ctx, SLOD_ERR_INVALID, "solver control: max_steps, tolerance and reduction must be non-negative");
+  return SLOD_OK;
+}
+
+static int check_time_steps(slod_ctx *ctx, double dt, int32_t n_steps, int32_t out_every) {
+  if (!(dt > 0.0) || !std::isfinite(dt)) return fail(ctx, SLOD_ERR_INVALID, "dt must be positive and finite");
+  if (n_steps < 1) return fail(ctx, SLOD_ERR_INVALID, "n_steps must be at least 1");
+  if (out_every < 1 || out_every > n_steps) return fail(ctx, SLOD_ERR_INVALID, "out_every must be in [1, n_steps]");
+  return SLOD_OK;
+}
+
+// scratch of the time steppers, allocated on first use and regrown when too small
+static int heat_scratch(slod_ctx *ctx, size_t doubles, double **out) {
+  if (ctx->heat_doubles < doubles) {
+    if (ctx->d_heat) cudaFree(ctx->d_heat);
+    ctx->d_heat = nullptr;
+    ctx->heat_doubles = 0;
+    CK(cudaMalloc(&ctx->d_heat, sizeof(double) * doubles));
+    ctx->heat_doubles = doubles;
+  }
+  *out = ctx->d_heat;
+  return SLOD_OK;
+}
+
+// the common preconditions of the two coarse time steppers, and S = M_H + dt K (kept until dt changes)
+static int heat_prepare(slod_ctx *ctx, double dt, int32_t n_steps, int32_t out_every, const double *u_out,
+                        int32_t max_steps, double tolerance, double reduction) {
+  if (!ctx->coarse_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse has not run");
+  if (!ctx->mass_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse_mass has not run");
+  if (!u_out) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  int rc = check_time_steps(ctx, dt, n_steps, out_every);
+  if (rc) return rc;
+  rc = check_solver_control(ctx, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  if (ctx->s_dt == dt) return SLOD_OK;
+  const size_t nk = (size_t)ctx->n_patches * ctx->P.s * ctx->P.ell_width;
+  if (!ctx->d_Sell) CK(cudaMalloc(&ctx->d_Sell, sizeof(double) * nk));
+  CK(launch_lincomb(0, (long long)nk, 1.0, ctx->d_Mell, dt, ctx->d_Kell, ctx->d_Sell));
+  ctx->launches += 1;
+  ctx->s_dt = dt;
+  return SLOD_OK;
+}
+
+static int heat_cg_failure(slod_ctx *ctx, int step, int column, int flag, int steps, double res) {
+  char buf[240];
+  const std::string col = column >= 0 ? " column " + std::to_string(column) : std::string();
+  if (flag == 2)
+    std::snprintf(buf, sizeof buf, "time step %d%s: CG on M_H + dt K broke down after %d steps (residual %.3e): the "
+                  "matrix is not positive definite", step, col.c_str(), steps, res);
+  else
+    std::snprintf(buf, sizeof buf, "time step %d%s: CG on M_H + dt K did not converge: %d steps, residual %.3e", step,
+                  col.c_str(), steps, res);
+  return fail(ctx, SLOD_ERR_NUMERIC, buf);
+}
+
+int slod_l2_project_batch(slod_ctx *ctx, int32_t n_rhs, const double *v_fine, double *u_coarse, int32_t max_steps,
+                          double tolerance, double reduction, int32_t *steps, double *residual) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  if (!ctx->mass_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse_mass has not run");
+  if (!v_fine || !u_coarse) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  if (n_rhs < 1) return fail(ctx, SLOD_ERR_INVALID, "n_rhs must be at least 1");
+  int rc = check_solver_control(ctx, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const long long n_nodes = n_fine / ctx->P.s;
+  const int nrows = (int)(ctx->n_patches * ctx->P.s);
+  BatchScratch w{};
+  rc = batch_scratch(ctx, &w);
+  if (rc) return rc;
+  std::vector<int> st_steps(n_rhs, 0), flag(n_rhs, 0);
+  std::vector<double> res(n_rhs, 0.0);
+  cudaError_t e = cudaSuccess;
+  long long n_launch = 0;
+  for (int j0 = 0; j0 < n_rhs && e == cudaSuccess; j0 += kBatch) {
+    const int kb = std::min(kBatch, n_rhs - j0);
+    e = cudaMemcpyAsync(w.fine_stage, v_fine + (size_t)j0 * n_fine, sizeof(double) * kb * (size_t)n_fine,
+                        cudaMemcpyHostToDevice, 0);
+    for (int j = 0; j < kb && e == cudaSuccess; ++j)   // M_h v, column by column, [kb][n_fine]
+      e = launch_fine_apply(0, kFineMass, 0.0, n_nodes, nullptr, w.fine_stage + (size_t)j * n_fine,
+                            w.fine + (size_t)j * n_fine);
+    if (e == cudaSuccess) e = launch_interleave(0, n_fine, kb, w.fine, w.fine_stage, true);
+    if (e == cudaSuccess)
+      e = launch_coarse_rhs_multi(0, (int)ctx->n_patches, ctx->P.s, kb, ctx->d_phi, w.fine_stage, w.coarse_a,
+                                  ctx->P.NfMax);
+    if (e == cudaSuccess)
+      e = run_cg_multi(0, nrows, ctx->d_Mell, kb, w.coarse_a, w.coarse_b, w.work, max_steps, tolerance, reduction,
+                       &st_steps[j0], &res[j0], &flag[j0], &n_launch);
+    if (e == cudaSuccess) e = launch_interleave(0, nrows, kb, w.coarse_b, w.coarse_stage, false);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(u_coarse + (size_t)j0 * nrows, w.coarse_stage, sizeof(double) * kb * (size_t)nrows,
+                          cudaMemcpyDeviceToHost, 0);
+    n_launch += kb + 3;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  ctx->launches += n_launch;
+  for (int j = 0; j < n_rhs; ++j) {
+    if (steps) steps[j] = st_steps[j];
+    if (residual) residual[j] = res[j];
+  }
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_l2_project_batch: ") + cudaGetErrorString(e));
+  for (int j = 0; j < n_rhs; ++j) {
+    if (flag[j] == 1) continue;
+    char buf[200];
+    std::snprintf(buf, sizeof buf, "CG on M_H %s in column %d: %d steps, residual %.3e",
+                  flag[j] == 2 ? "broke down" : "did not converge", j, st_steps[j], res[j]);
+    return fail(ctx, SLOD_ERR_NUMERIC, buf);
+  }
+  return SLOD_OK;
+}
+
+int slod_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_coarse, double dt, int32_t n_steps,
+                    int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
+                    int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  int rc = heat_prepare(ctx, dt, n_steps, out_every, u_out, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const int nrows = (int)(ctx->n_patches * ctx->P.s);
+  double *d_f = nullptr, *d_r = nullptr, *d_delta = nullptr, *d_work = nullptr, *d_u = nullptr;
+  rc = online_scratch(ctx, &d_f, nullptr, &d_r, &d_delta, &d_work);
+  if (rc) return rc;
+  rc = heat_scratch(ctx, 2 * (size_t)nrows, &d_u);
+  if (rc) return rc;
+  double *d_b = d_u + nrows;
+  cudaError_t e = cudaSuccess;
+  if (f_fine) {
+    e = cudaMemcpyAsync(d_f, f_fine, sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+    if (e == cudaSuccess) e = launch_coarse_rhs(0, (int)ctx->n_patches, ctx->P.s, ctx->d_phi, d_f, d_b, ctx->P.NfMax);
+    ctx->launches += 1;
+  } else {
+    e = cudaMemsetAsync(d_b, 0, sizeof(double) * nrows, 0);
+  }
+  if (e == cudaSuccess)
+    e = u0_coarse ? cudaMemcpyAsync(d_u, u0_coarse, sizeof(double) * nrows, cudaMemcpyHostToDevice, 0)
+                  : cudaMemsetAsync(d_u, 0, sizeof(double) * nrows, 0);
+  const CgOperator S{ctx->d_Sell, nullptr, 0};
+  long long n_launch = 0;
+  int failed_step = 0, flag = 0, st_steps = 0;
+  double res = 0.0;
+  for (int k = 1; k <= n_steps && e == cudaSuccess; ++k) {
+    e = launch_ell_residual(0, nrows, 1, ctx->d_Kell, d_u, d_b, dt, d_r);
+    if (e == cudaSuccess)
+      e = run_cg(0, nrows, S, d_r, d_delta, d_work, max_steps, tolerance, reduction, &st_steps, &res, &flag, &n_launch);
+    if (e != cudaSuccess) break;
+    if (cg_steps) cg_steps[k - 1] = st_steps;
+    if (flag != 1) {
+      failed_step = k;
+      break;
+    }
+    e = launch_lincomb(0, nrows, 1.0, d_u, 1.0, d_delta, d_u);
+    if (e == cudaSuccess && k % out_every == 0)
+      e = cudaMemcpyAsync(u_out + (size_t)(k / out_every - 1) * nrows, d_u, sizeof(double) * nrows,
+                          cudaMemcpyDeviceToHost, 0);
+    n_launch += 2;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  ctx->launches += n_launch;
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_heat_solve: ") + cudaGetErrorString(e));
+  if (failed_step) return heat_cg_failure(ctx, failed_step, -1, flag, st_steps, res);
+  return SLOD_OK;
+}
+
+int slod_heat_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, const double *u0_coarse, double dt,
+                          int32_t n_steps, int32_t out_every, double *u_out, int32_t max_steps, double tolerance,
+                          double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  if (n_rhs < 1) return fail(ctx, SLOD_ERR_INVALID, "n_rhs must be at least 1");
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  int rc = heat_prepare(ctx, dt, n_steps, out_every, u_out, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const int nrows = (int)(ctx->n_patches * ctx->P.s);
+  const int n_groups = (n_rhs + kBatch - 1) / kBatch;
+  const size_t gsz = (size_t)kBatch * nrows;   // one interleaved group
+  BatchScratch w{};
+  rc = batch_scratch(ctx, &w);
+  if (rc) return rc;
+  double *d_U = nullptr;   // [group][nrows][kb] states, then the right-hand sides C^T f in the same layout
+  rc = heat_scratch(ctx, 2 * (size_t)n_groups * gsz, &d_U);
+  if (rc) return rc;
+  double *d_B = d_U + (size_t)n_groups * gsz;
+  cudaError_t e = cudaSuccess;
+  long long n_launch = 0;
+  for (int g = 0; g < n_groups && e == cudaSuccess; ++g) {
+    const int j0 = g * kBatch, kb = std::min(kBatch, n_rhs - j0);
+    double *U = d_U + g * gsz, *B = d_B + g * gsz;
+    if (f_fine) {
+      e = cudaMemcpyAsync(w.fine_stage, f_fine + (size_t)j0 * n_fine, sizeof(double) * kb * (size_t)n_fine,
+                          cudaMemcpyHostToDevice, 0);
+      if (e == cudaSuccess) e = launch_interleave(0, n_fine, kb, w.fine_stage, w.fine, true);
+      if (e == cudaSuccess)
+        e = launch_coarse_rhs_multi(0, (int)ctx->n_patches, ctx->P.s, kb, ctx->d_phi, w.fine, B, ctx->P.NfMax);
+      n_launch += 2;
+    } else {
+      e = cudaMemsetAsync(B, 0, sizeof(double) * kb * (size_t)nrows, 0);
+    }
+    if (e == cudaSuccess && u0_coarse) {
+      e = cudaMemcpyAsync(w.coarse_stage, u0_coarse + (size_t)j0 * nrows, sizeof(double) * kb * (size_t)nrows,
+                          cudaMemcpyHostToDevice, 0);
+      if (e == cudaSuccess) e = launch_interleave(0, nrows, kb, w.coarse_stage, U, true);
+      n_launch += 1;
+    } else if (e == cudaSuccess) {
+      e = cudaMemsetAsync(U, 0, sizeof(double) * kb * (size_t)nrows, 0);
+    }
+  }
+  std::vector<int> st_steps(n_rhs, 0), flag(n_rhs, 0);
+  std::vector<double> res(n_rhs, 0.0);
+  int failed_step = 0, failed_col = -1;
+  for (int k = 1; k <= n_steps && e == cudaSuccess && !failed_step; ++k) {
+    for (int g = 0; g < n_groups && e == cudaSuccess; ++g) {
+      const int j0 = g * kBatch, kb = std::min(kBatch, n_rhs - j0);
+      double *U = d_U + g * gsz, *B = d_B + g * gsz;
+      e = launch_ell_residual(0, nrows, kb, ctx->d_Kell, U, B, dt, w.coarse_a);
+      if (e == cudaSuccess)
+        e = run_cg_multi(0, nrows, ctx->d_Sell, kb, w.coarse_a, w.coarse_b, w.work, max_steps, tolerance, reduction,
+                         &st_steps[j0], &res[j0], &flag[j0], &n_launch);
+      if (e != cudaSuccess) break;
+      for (int j = 0; j < kb; ++j) {
+        if (cg_steps) cg_steps[(size_t)(k - 1) * n_rhs + j0 + j] = st_steps[j0 + j];
+        if (flag[j0 + j] != 1 && !failed_step) {
+          failed_step = k;
+          failed_col = j0 + j;
+        }
+      }
+      if (failed_step) break;
+      e = launch_lincomb(0, (long long)kb * nrows, 1.0, U, 1.0, w.coarse_b, U);
+      n_launch += 2;
+    }
+    if (e != cudaSuccess || failed_step || k % out_every != 0) continue;
+    for (int g = 0; g < n_groups && e == cudaSuccess; ++g) {
+      const int j0 = g * kBatch, kb = std::min(kBatch, n_rhs - j0);
+      e = launch_interleave(0, nrows, kb, d_U + g * gsz, w.coarse_stage, false);
+      if (e == cudaSuccess)
+        e = cudaMemcpyAsync(u_out + ((size_t)(k / out_every - 1) * n_rhs + j0) * nrows, w.coarse_stage,
+                            sizeof(double) * kb * (size_t)nrows, cudaMemcpyDeviceToHost, 0);
+      n_launch += 1;
+    }
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  ctx->launches += n_launch;
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_heat_solve_batch: ") + cudaGetErrorString(e));
+  if (failed_step)
+    return heat_cg_failure(ctx, failed_step, failed_col, flag[failed_col], st_steps[failed_col], res[failed_col]);
+  return SLOD_OK;
+}
+
+// the fine-scale reference trajectory: the same scheme with M_h + dt A_h on the global grid (homogeneous Dirichlet rows)
+int slod_fem_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_fine, double dt, int32_t n_steps,
+                        int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
+                        int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  if (!u_out) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  int rc = check_time_steps(ctx, dt, n_steps, out_every);
+  if (rc) return rc;
+  rc = check_solver_control(ctx, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  CK(cudaSetDevice(ctx->device));
+  rc = prepare_coefficients(ctx);
+  if (rc) return rc;
+  BIND_PARAMS((cudaStream_t)0);
+  const Params &P = ctx->P;
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const long long n_nodes = n_fine / P.s;
+  // homogeneous Dirichlet conditions: the boundary rows of f and u0 are zero
+  std::vector<double> f(n_fine, 0.0), u0(n_fine, 0.0);
+  if (f_fine) std::copy(f_fine, f_fine + n_fine, f.begin());
+  if (u0_fine) std::copy(u0_fine, u0_fine + n_fine, u0.begin());
+  const long long G = P.nsub + 1;
+  for (long long node = 0; node < n_nodes; ++node) {
+    long long r = node;
+    bool bd = false;
+    for (int a = 0; a < P.dim; ++a) {
+      const long long i = r % G;
+      r /= G;
+      bd = bd || i == 0 || i == G - 1;
+    }
+    if (bd)
+      for (int c = 0; c < P.s; ++c) f[node * P.s + c] = u0[node * P.s + c] = 0.0;
+  }
+  double *d_r = nullptr, *d_delta = nullptr, *d_work = nullptr, *d_f = nullptr;
+  rc = online_scratch(ctx, &d_r, &d_delta, nullptr, nullptr, &d_work);
+  if (rc) return rc;
+  rc = heat_scratch(ctx, 3 * (size_t)n_fine, &d_f);
+  if (rc) return rc;
+  double *d_u = d_f + n_fine, *d_q = d_u + n_fine;
+  CgOperator A{nullptr, ctx->d_coef, n_nodes};
+  A.op = kFineHeatDirichlet;
+  A.tau = dt;
+  cudaError_t e = cudaMemcpyAsync(d_f, f.data(), sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_u, u0.data(), sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+  long long n_launch = 0;
+  int failed_step = 0, flag = 0, st_steps = 0;
+  double res = 0.0;
+  for (int k = 1; k <= n_steps && e == cudaSuccess; ++k) {
+    e = launch_fine_apply(0, kFineStiffDirichlet, 0.0, n_nodes, ctx->d_coef, d_u, d_q);
+    if (e == cudaSuccess) e = launch_lincomb(0, n_fine, dt, d_f, -dt, d_q, d_r);   // dt (f - A u), zero boundary rows
+    if (e == cudaSuccess)
+      e = run_cg(0, (int)n_fine, A, d_r, d_delta, d_work, max_steps, tolerance, reduction, &st_steps, &res, &flag,
+                 &n_launch);
+    if (e != cudaSuccess) break;
+    if (cg_steps) cg_steps[k - 1] = st_steps;
+    if (flag != 1) {
+      failed_step = k;
+      break;
+    }
+    e = launch_lincomb(0, n_fine, 1.0, d_u, 1.0, d_delta, d_u);
+    if (e == cudaSuccess && k % out_every == 0)
+      e = cudaMemcpyAsync(u_out + (size_t)(k / out_every - 1) * n_fine, d_u, sizeof(double) * (size_t)n_fine,
+                          cudaMemcpyDeviceToHost, 0);
+    n_launch += 3;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  ctx->launches += n_launch;
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_fem_heat_solve: ") + cudaGetErrorString(e));
+  if (failed_step) {
+    char buf[200];
+    std::snprintf(buf, sizeof buf, "time step %d: fine CG on M_h + dt A_h %s: %d steps, residual %.3e", failed_step,
+                  flag == 2 ? "broke down" : "did not converge", st_steps, res);
+    return fail(ctx, SLOD_ERR_NUMERIC, buf);
+  }
+  return SLOD_OK;
+}
+
 // ---- checkpoint: parameters + phi + A*phi (+ block-ELL coarse matrix) --------------------------------------------
 namespace {
 struct StateHeader {
@@ -2135,6 +2548,7 @@ int slod_load_state(slod_ctx *ctx, const char *path) {
   }
   ctx->basis_done = ok;
   ctx->coarse_done = false;
+  invalidate_mass(ctx);
   if (ok && h.has_coarse) {
     if (!ctx->d_Kell) CK(cudaMalloc(&ctx->d_Kell, sizeof(double) * nk));
     ok = std::fread(buf.data(), sizeof(double), nk, f) == nk;

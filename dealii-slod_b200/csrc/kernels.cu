@@ -1205,6 +1205,7 @@ cudaError_t launch_gather(cudaStream_t st, const double *src, const long long *p
 }  // namespace slod
 #include "online.cuh"
 #include "online_batch.cuh"
+#include "heat.cuh"
 namespace slod {
 
 cudaError_t launch_coarse_rhs(cudaStream_t st, int n_patches, int s, const double *phi, const double *f, double *b,
@@ -1232,7 +1233,7 @@ size_t cg_workspace_doubles(const CgOperator &A, int nrows) {
 }
 // Runs diag-preconditioned CG until the device-side stopping test fires or max_steps is reached; the host looks at the
 // state every `check_every` steps (one 64-byte copy).  A.Kell != nullptr: block-ELL coarse matrix; else the fine
-// Dirichlet stiffness operator applied matrix free.  Returns the state in *steps / *residual / *flag.
+// Dirichlet operator A.op applied matrix free.  Returns the state in *steps / *residual / *flag.
 cudaError_t run_cg(cudaStream_t st, int nrows, const CgOperator &A, const double *b, double *x, double *work,
                    int max_steps, double tol, double reduction, int *steps, double *residual, int *flag,
                    long long *launches) {
@@ -1243,7 +1244,7 @@ cudaError_t run_cg(cudaStream_t st, int nrows, const CgOperator &A, const double
   CgState h{};
   cudaError_t e;
   if (!A.Kell) {
-    k_fine_apply<<<nb_apply, kCgThreads, 0, st>>>(kFineStiffDirichlet, A.n_nodes, A.d_coef, nullptr, nullptr, dinv, nullptr,
+    k_fine_apply<<<nb_apply, kCgThreads, 0, st>>>(A.op, A.tau, A.n_nodes, A.d_coef, nullptr, nullptr, dinv, nullptr,
                                                  nullptr);
     *launches += 1;
   }
@@ -1260,7 +1261,7 @@ cudaError_t run_cg(cudaStream_t st, int nrows, const CgOperator &A, const double
       if (A.Kell)
         k_cg_spmv<<<nb_apply, kCgThreads, 0, st>>>(nrows, A.Kell, p, q, ppq, state);
       else
-        k_fine_apply<<<nb_apply, kCgThreads, 0, st>>>(kFineStiffDirichlet, A.n_nodes, A.d_coef, p, q, nullptr, ppq, state);
+        k_fine_apply<<<nb_apply, kCgThreads, 0, st>>>(A.op, A.tau, A.n_nodes, A.d_coef, p, q, nullptr, ppq, state);
       k_cg_update<<<nb_vec, kCgThreads, 0, st>>>(nrows, it, p, q, dinv, x, r, ppq, nb_apply, prz, prr, state);
       k_cg_direction<<<nb_vec, kCgThreads, 0, st>>>(nrows, it, r, dinv, p, prz, prr, nb_vec, state);
       *launches += 3;
@@ -1277,7 +1278,7 @@ cudaError_t launch_fine_quadratic_form(cudaStream_t st, int op, long long n_node
                                        double *partial, int *n_partial) {
   const int nb = (int)((n_nodes + kCgThreads - 1) / kCgThreads);
   *n_partial = nb;
-  if (partial) k_fine_apply<<<nb, kCgThreads, 0, st>>>(op, n_nodes, d_coef, x, nullptr, nullptr, partial, nullptr);
+  if (partial) k_fine_apply<<<nb, kCgThreads, 0, st>>>(op, 0.0, n_nodes, d_coef, x, nullptr, nullptr, partial, nullptr);
   return cudaGetLastError();
 }
 
@@ -1349,6 +1350,29 @@ cudaError_t run_cg_multi(cudaStream_t st, int nrows, const double *Kell, int kb,
     residual[j] = sqrt(h[j].rr);
     flag[j] = h[j].done;
   }
+  return cudaGetLastError();
+}
+
+// ---- heat equation on the SLOD space (heat.cuh) ----
+cudaError_t launch_mass_apply(cudaStream_t st, int n_patches, int s, const double *phi, double *mphi, int nf_max) {
+  const int rows = n_patches * s;
+  k_mass_apply<<<rows < 148 * 16 ? rows : 148 * 16, 256, 0, st>>>(n_patches, phi, mphi, nf_max);
+  return cudaGetLastError();
+}
+cudaError_t launch_ell_residual(cudaStream_t st, int nrows, int kb, const double *Kell, const double *U, const double *B,
+                                double tau, double *R) {
+  k_ell_residual<<<cg_multi_apply_blocks(nrows), kCgThreads, 0, st>>>(nrows, kb, Kell, U, B, tau, R);
+  return cudaGetLastError();
+}
+cudaError_t launch_lincomb(cudaStream_t st, long long n, double a, const double *x, double b, const double *y, double *z) {
+  const long long blocks = (n + 255) / 256;
+  k_lincomb<<<(int)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, st>>>(n, a, x, b, y, z);
+  return cudaGetLastError();
+}
+cudaError_t launch_fine_apply(cudaStream_t st, int op, double tau, long long n_nodes, const double *d_coef,
+                              const double *x, double *y) {
+  const int nb = (int)((n_nodes + kCgThreads - 1) / kCgThreads);
+  k_fine_apply<<<nb, kCgThreads, 0, st>>>(op, tau, n_nodes, d_coef, x, y, nullptr, nullptr, nullptr);
   return cudaGetLastError();
 }
 

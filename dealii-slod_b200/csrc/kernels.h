@@ -137,12 +137,15 @@ enum FineOp {
   kFineStiffDirichlet = 0,  // coefficient-weighted stiffness, identity on the domain-boundary rows, boundary columns dropped
   kFineEnergy = 1,          // the same without the boundary treatment: x.y = energy norm^2
   kFineMass = 2,            // mass matrix: x.y = L2 norm^2
-  kFineLaplace = 3          // component-wise unweighted Laplace: x.y = H1 seminorm^2
+  kFineLaplace = 3,         // component-wise unweighted Laplace: x.y = H1 seminorm^2
+  kFineHeatDirichlet = 4    // mass + tau * stiffness (backward Euler), with the boundary treatment of op 0
 };
 struct CgOperator {
-  const double *Kell;     // block-ELL coarse matrix, or nullptr for the fine Dirichlet stiffness operator
+  const double *Kell;     // block-ELL coarse matrix, or nullptr for a fine Dirichlet operator
   const double *d_coef;   // fine operator: sub-cell coefficients
   long long n_nodes;      // fine operator: nodes of the global grid
+  int op = kFineStiffDirichlet;   // fine operator: kFineStiffDirichlet or kFineHeatDirichlet
+  double tau = 0.0;               // fine operator kFineHeatDirichlet: the time step
 };
 size_t cg_workspace_doubles(const CgOperator &A, int nrows);
 cudaError_t run_cg(cudaStream_t st, int nrows, const CgOperator &A, const double *b, double *x, double *work,
@@ -163,6 +166,17 @@ size_t cg_multi_workspace_doubles(int nrows);
 cudaError_t run_cg_multi(cudaStream_t st, int nrows, const double *Kell, int kb, const double *B, double *X,
                          double *work, int max_steps, double tol, double reduction, int *steps, double *residual,
                          int *flag, long long *launches);
+// heat equation on the SLOD space (heat.cuh)
+// M_h phi of every patch on its own node box, the [n_patches][s][nf_max] layout of A phi
+cudaError_t launch_mass_apply(cudaStream_t st, int n_patches, int s, const double *phi, double *mphi, int nf_max);
+// R = tau (B - K U) on the block-ELL matrix for kb <= kBatch interleaved columns (kb = 1: plain vectors)
+cudaError_t launch_ell_residual(cudaStream_t st, int nrows, int kb, const double *Kell, const double *U, const double *B,
+                                double tau, double *R);
+// z = a x + b y (z may alias x or y)
+cudaError_t launch_lincomb(cudaStream_t st, long long n, double a, const double *x, double b, const double *y, double *z);
+// y = Op x for a FineOp (tau: kFineHeatDirichlet), no reduction
+cudaError_t launch_fine_apply(cudaStream_t st, int op, double tau, long long n_nodes, const double *d_coef,
+                              const double *x, double *y);
 cudaError_t launch_fine_quadratic_form(cudaStream_t st, int op, long long n_nodes, const double *d_coef, const double *x,
                                        double *partial, int *n_partial);
 cudaError_t launch_fine_norms_reference(cudaStream_t st, long long n_cells, int nq, const double *gauss_x,

@@ -145,11 +145,41 @@ k_cg_init(int nrows, const double *__restrict__ Kell, const double *__restrict__
   }
 }
 
-// q = K p, one warp per row (grid-stride over row groups); per-block partial sums of p.q.
-// The column of entry (dx, dy, dz) is dilate(cx + dx) | dilate(cy + dy) << 1 | dilate(cz + dz) << 2: each warp tabulates
-// the 3 (2w+1) dilated coordinates of its row in shared memory (sign bit = outside the domain), so an entry costs three
-// table reads and two ORs, and the sweep is bound by the 8 bytes per entry it reads.
+// Column decoding of the block-ELL rows, shared by every kernel that multiplies with K (or with a matrix of the same
+// slot convention).  The column of entry (dx, dy, dz) is dilate(cx + dx) | dilate(cy + dy) << 1 | dilate(cz + dz) << 2:
+// each warp tabulates the 3 (2w+1) dilated coordinates of its row in shared memory (sign bit = outside the domain), so
+// an entry costs three table reads and two ORs, and a sweep is bound by the 8 bytes per entry it reads.
 constexpr int kCgTab = 32;   // 2w+1 <= 32 (oversampling <= 7); larger stencils take the direct path
+__device__ __forceinline__ void ell_tabulate(int (*tab)[kCgTab], const int c[3], int lane) {
+  const int w = cP.w, ww = 2 * w + 1, dim = cP.dim;
+  __syncwarp();
+  for (int i = lane; i < 3 * ww; i += 32) {
+    const int a = i / ww, d = i - a * ww, v = c[a] + d - w;
+    int code = 0;
+    if (a < dim) code = (v >= 0 && v < cP.N) ? (int)(((dim == 3) ? dilate3(v) : dilate2(v)) << a) : (int)0x80000000;
+    tab[a][d] = code;
+  }
+  __syncwarp();
+}
+// column (coarse dof) of entry t < ell_width of the row whose centre cell is c, -1 outside the domain; `tab` is the
+// warp's table (tabulated: 2w+1 <= kCgTab), else the Morton code is computed directly
+__device__ __forceinline__ int ell_column(int t, const int (*tab)[kCgTab], const int c[3], bool tabulated) {
+  const int s = cP.s, w = cP.w, ww = 2 * w + 1, dim = cP.dim;
+  const float inv_ww = 1.0f / (float)ww;   // exact quotients for these small integers
+  const int slot = (s == 1) ? t : (t >> 1), e = (s == 1) ? 0 : (t & 1);   // spacedim is 1 or 2
+  const int s1 = (int)(((float)slot + 0.5f) * inv_ww), s2 = (int)(((float)s1 + 0.5f) * inv_ww);
+  if (tabulated) {
+    const int cc = tab[0][slot - s1 * ww] | tab[1][s1 - s2 * ww] | tab[2][s2];
+    return (cc >= 0) ? cc * s + e : -1;
+  }
+  int qc[3] = {c[0] + (slot - s1 * ww) - w, c[1] + (s1 - s2 * ww) - w, (dim == 3) ? c[2] + s2 - w : 0};
+  bool valid = true;
+#pragma unroll
+  for (int x = 0; x < 3; ++x) if (x < dim) valid = valid && (qc[x] >= 0 && qc[x] < cP.N);
+  return valid ? (int)morton_fast(qc, dim) * s + e : -1;
+}
+
+// q = K p, one warp per row (grid-stride over row groups); per-block partial sums of p.q.
 __global__ void __launch_bounds__(kCgThreads)
 k_cg_spmv(int nrows, const double *__restrict__ Kell, const double *__restrict__ p, double *__restrict__ q,
           double *__restrict__ partial, const CgState *st) {
@@ -159,7 +189,6 @@ k_cg_spmv(int nrows, const double *__restrict__ Kell, const double *__restrict__
   const int s = cP.s, w = cP.w, ww = 2 * w + 1, dim = cP.dim;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const bool tabulated = ww <= kCgTab;
-  const float inv_ww = 1.0f / (float)ww;   // exact quotients for these small integers
   double pq = 0.0;
   for (int row = blockIdx.x * (kCgThreads / 32) + warp; row < nrows; row += gridDim.x * (kCgThreads / 32)) {
     const int pid = row / s;
@@ -168,14 +197,7 @@ k_cg_spmv(int nrows, const double *__restrict__ Kell, const double *__restrict__
     const double *kr = Kell + (size_t)row * cP.ell_width;
     double acc = 0.0;
     if (tabulated) {
-      __syncwarp();
-      for (int i = lane; i < 3 * ww; i += 32) {
-        const int a = i / ww, d = i - a * ww, v = c[a] + d - w;
-        int code = 0;
-        if (a < dim) code = (v >= 0 && v < cP.N) ? (int)(((dim == 3) ? dilate3(v) : dilate2(v)) << a) : (int)0x80000000;
-        sTab[warp][a][d] = code;
-      }
-      __syncwarp();
+      ell_tabulate(sTab[warp], c, lane);
       for (int t0 = lane; t0 < cP.ell_width; t0 += 128) {   // four independent entries in flight per lane
         double kv[4];
         int col[4];
@@ -186,12 +208,8 @@ k_cg_spmv(int nrows, const double *__restrict__ Kell, const double *__restrict__
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-          const int t = t0 + 32 * u, tc = min(t, cP.ell_width - 1);   // clamped: table indices stay in range
-          const int slot = (s == 1) ? tc : (tc >> 1), e = (s == 1) ? 0 : (tc & 1);   // spacedim is 1 or 2
-          const int s1 = (int)(((float)slot + 0.5f) * inv_ww), s2 = (int)(((float)s1 + 0.5f) * inv_ww);
-          const int cc = (t < cP.ell_width)
-                             ? (sTab[warp][0][slot - s1 * ww] | sTab[warp][1][s1 - s2 * ww] | sTab[warp][2][s2]) : -1;
-          col[u] = (cc >= 0) ? cc * s + e : -1;
+          const int t = t0 + 32 * u;
+          col[u] = (t < cP.ell_width) ? ell_column(t, sTab[warp], c, true) : -1;
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u)
@@ -199,13 +217,8 @@ k_cg_spmv(int nrows, const double *__restrict__ Kell, const double *__restrict__
       }
     } else {
       for (int t = lane; t < cP.ell_width; t += 32) {
-        const int slot = (s == 1) ? t : (t >> 1), e = (s == 1) ? 0 : (t & 1);
-        const int s1 = (int)(((float)slot + 0.5f) * inv_ww), s2 = (int)(((float)s1 + 0.5f) * inv_ww);
-        int qc[3] = {c[0] + (slot - s1 * ww) - w, c[1] + (s1 - s2 * ww) - w, (dim == 3) ? c[2] + s2 - w : 0};
-        bool valid = true;
-#pragma unroll
-        for (int x = 0; x < 3; ++x) if (x < dim) valid = valid && (qc[x] >= 0 && qc[x] < cP.N);
-        if (valid) acc += kr[t] * p[(size_t)morton_fast(qc, dim) * s + e];
+        const int col = ell_column(t, nullptr, c, false);
+        if (col >= 0) acc += kr[t] * p[col];
       }
     }
     acc = warp_sum(acc);
@@ -281,9 +294,32 @@ k_cg_direction(int nrows, int it, const double *__restrict__ r, const double *__
 // use (geom.h: Kref / Klam / Kq), so the fine FEM problem of assemble_and_solve_fem_problem (source/LOD.cc:1004-1094)
 // is exactly the operator the patch problems restrict.
 
-__device__ __forceinline__ double fine_local_entry(int op, const double *__restrict__ d_coef, long long sc, long long fstride,
+__device__ __forceinline__ double fine_stiff_entry(const double *__restrict__ d_coef, long long sc, long long fstride,
                                                    int la, int lb, int ca, int cb) {
   const int dim = cP.dim, s = cP.s;
+  const int nl = (1 << dim) * s;
+  const int idx = (la * s + ca) * nl + (lb * s + cb);
+  if (!cP.gauss_coef) {
+    if (cP.problem == 0) return d_coef[sc] * cP.Kref[idx];
+    return d_coef[fstride + sc] * cP.Kref[idx] + d_coef[sc] * cP.Klam[idx];
+  }
+  const int nq = 1 << dim;
+  double v = 0.0;
+  for (int q = 0; q < nq; ++q) {
+    if (cP.problem == 0) v += d_coef[sc * nq + q] * cP.Kq[q][idx];
+    else v += d_coef[(fstride + sc) * nq + q] * cP.Kq[q][idx] + d_coef[sc * nq + q] * cP.Klamq[q][idx];
+  }
+  return v;
+}
+
+__device__ __forceinline__ double fine_local_entry(int op, double tau, const double *__restrict__ d_coef, long long sc,
+                                                   long long fstride, int la, int lb, int ca, int cb) {
+  const int dim = cP.dim;
+  if (op == kFineHeatDirichlet) {   // mass + tau * stiffness
+    double m = (ca == cb) ? 1.0 : 0.0;
+    for (int x = 0; x < dim; ++x) m *= (((la >> x) & 1) == ((lb >> x) & 1)) ? cP.h / 3.0 : cP.h / 6.0;
+    return m + tau * fine_stiff_entry(d_coef, sc, fstride, la, lb, ca, cb);
+  }
   if (op == kFineMass || op == kFineLaplace) {
     if (ca != cb) return 0.0;
     double m[3] = {1.0, 1.0, 1.0};
@@ -301,28 +337,18 @@ __device__ __forceinline__ double fine_local_entry(int op, const double *__restr
     }
     return v;
   }
-  const int nl = (1 << dim) * s;
-  const int idx = (la * s + ca) * nl + (lb * s + cb);
-  if (!cP.gauss_coef) {
-    if (cP.problem == 0) return d_coef[sc] * cP.Kref[idx];
-    return d_coef[fstride + sc] * cP.Kref[idx] + d_coef[sc] * cP.Klam[idx];
-  }
-  const int nq = 1 << dim;
-  double v = 0.0;
-  for (int q = 0; q < nq; ++q) {
-    if (cP.problem == 0) v += d_coef[sc * nq + q] * cP.Kq[q][idx];
-    else v += d_coef[(fstride + sc) * nq + q] * cP.Kq[q][idx] + d_coef[sc * nq + q] * cP.Klamq[q][idx];
-  }
-  return v;
+  return fine_stiff_entry(d_coef, sc, fstride, la, lb, ca, cb);
 }
 
-// invdiag != nullptr: write 1 / diagonal of the operator instead of applying it (Jacobi preconditioner)
+// invdiag != nullptr: write 1 / diagonal of the operator instead of applying it (Jacobi preconditioner).
+// tau: the time step of kFineHeatDirichlet, unused by the other operators.
 __global__ void __launch_bounds__(kCgThreads)
-k_fine_apply(int op, long long n_nodes, const double *__restrict__ d_coef, const double *__restrict__ x,
+k_fine_apply(int op, double tau, long long n_nodes, const double *__restrict__ d_coef, const double *__restrict__ x,
              double *__restrict__ y, double *__restrict__ invdiag, double *__restrict__ partial, const CgState *st) {
   __shared__ double sRed[kCgThreads / 32];
   if (st && st->done) return;
   const int dim = cP.dim, s = cP.s, G = cP.nsub + 1, nsub = cP.nsub;
+  const bool dirichlet = op == kFineStiffDirichlet || op == kFineHeatDirichlet;
   const long long fstride = (dim == 3) ? (long long)nsub * nsub * nsub : (long long)nsub * nsub;
   const long long node = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   double dot = 0.0;
@@ -336,7 +362,7 @@ k_fine_apply(int op, long long n_nodes, const double *__restrict__ d_coef, const
     bool on_boundary = false;
     for (int k = 0; k < dim; ++k) on_boundary = on_boundary || a[k] == 0 || a[k] == G - 1;
     double acc[2] = {0.0, 0.0};
-    if (op == kFineStiffDirichlet && on_boundary) {
+    if (dirichlet && on_boundary) {
       for (int c = 0; c < s; ++c) acc[c] = invdiag ? 1.0 : x[node * s + c];
     } else {
       for (int corner = 0; corner < (1 << dim); ++corner) {   // the sub-cell in which this node is local node `corner`
@@ -355,13 +381,13 @@ k_fine_apply(int op, long long n_nodes, const double *__restrict__ d_coef, const
             b[k] = o[k] + ((lb >> k) & 1);
             b_boundary = b_boundary || b[k] == 0 || b[k] == G - 1;
           }
-          if (op == kFineStiffDirichlet && b_boundary) continue;
+          if (dirichlet && b_boundary) continue;
           if (invdiag && lb != corner) continue;
           const long long nb = ((long long)b[2] * G + b[1]) * G + b[0];
           for (int ca = 0; ca < s; ++ca)
             for (int cb = 0; cb < s; ++cb) {
               if (invdiag && cb != ca) continue;
-              const double v = fine_local_entry(op, d_coef, sc, fstride, corner, lb, ca, cb);
+              const double v = fine_local_entry(op, tau, d_coef, sc, fstride, corner, lb, ca, cb);
               acc[ca] += invdiag ? v : v * x[nb * s + cb];
             }
         }

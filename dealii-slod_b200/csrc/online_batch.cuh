@@ -179,23 +179,13 @@ k_cg_spmm(int nrows, int kb, const double *__restrict__ Kell, const double *__re
   const int j = lane & (kBatch - 1), h = lane >> 4;
   const bool active = j < kb;
   const bool tabulated = ww <= kCgTab;
-  const float inv_ww = 1.0f / (float)ww;
   double pq = 0.0;   // lane j < kb: column j
   for (int row = blockIdx.x * (kCgThreads / 32) + warp; row < nrows; row += gridDim.x * (kCgThreads / 32)) {
     const int pid = row / s;
     int c[3];
     morton_decode((uint32_t)pid, dim, cP.ref, c);
     const double *kr = Kell + (size_t)row * cP.ell_width;
-    if (tabulated) {
-      __syncwarp();
-      for (int i = lane; i < 3 * ww; i += 32) {
-        const int a = i / ww, d = i - a * ww, v = c[a] + d - w;
-        int code = 0;
-        if (a < dim) code = (v >= 0 && v < cP.N) ? (int)(((dim == 3) ? dilate3(v) : dilate2(v)) << a) : (int)0x80000000;
-        sTab[warp][a][d] = code;
-      }
-      __syncwarp();
-    }
+    if (tabulated) ell_tabulate(sTab[warp], c, lane);
     double acc = 0.0;
     for (int t0 = 0; t0 < cP.ell_width; t0 += 128) {   // four batches of 32 entries: four K loads in flight per lane
       double kv[4];
@@ -208,21 +198,7 @@ k_cg_spmm(int nrows, int kb, const double *__restrict__ Kell, const double *__re
 #pragma unroll
       for (int b = 0; b < 4; ++b) {
         const int t = t0 + 32 * b + lane;
-        col[b] = -1;
-        if (t < cP.ell_width) {
-          const int slot = (s == 1) ? t : (t >> 1), e = (s == 1) ? 0 : (t & 1);
-          const int s1 = (int)(((float)slot + 0.5f) * inv_ww), s2 = (int)(((float)s1 + 0.5f) * inv_ww);
-          if (tabulated) {
-            const int cc = sTab[warp][0][slot - s1 * ww] | sTab[warp][1][s1 - s2 * ww] | sTab[warp][2][s2];
-            col[b] = (cc >= 0) ? cc * s + e : -1;
-          } else {
-            int qc[3] = {c[0] + (slot - s1 * ww) - w, c[1] + (s1 - s2 * ww) - w, (dim == 3) ? c[2] + s2 - w : 0};
-            bool valid = true;
-#pragma unroll
-            for (int x = 0; x < 3; ++x) if (x < dim) valid = valid && (qc[x] >= 0 && qc[x] < cP.N);
-            col[b] = valid ? (int)morton_fast(qc, dim) * s + e : -1;
-          }
-        }
+        col[b] = (t < cP.ell_width) ? ell_column(t, sTab[warp], c, tabulated) : -1;
       }
 #pragma unroll
       for (int b = 0; b < 4; ++b)

@@ -185,6 +185,46 @@ int slod_fine_norms(slod_ctx *ctx, const double *v_fine, double *l2, double *h1_
  * sqrt(L2^2 + |.|_H1^2)).  Outputs may be NULL. */
 int slod_fine_norms_reference(slod_ctx *ctx, const double *v_fine, double *l2, double *linfty, double *h1);
 
+/* ---- the coarse mass matrix and the heat equation on the SLOD space.  The reference solves one elliptic problem and has
+ * no time-dependent path: these calls are an extension.  They run on the handle's first device (n_gpus > 1: the one that
+ * holds all of phi) and serve handles restored by slod_load_state (the checkpoint does not hold M_H: assemble it again).
+ *
+ * slod_assemble_coarse_mass: M_H = C^T (M_h C) with M_h the exact Q1 mass matrix of the sub-cell grid, in the block-ELL
+ * form and on the structural pattern of the coarse matrix (the same slot convention and CSR pattern).  Needs the basis
+ * only.  slod_compute_basis, slod_load_state and slod_assemble_coarse make M_H stale: the calls that need it return
+ * SLOD_ERR_STATE until it is assembled again.  Device times of its two kernels: slod_get_timings [6] (M_h phi) and [7]
+ * (the product).  slod_get_coarse_mass_csr: the same contract as slod_get_coarse_csr. */
+int slod_assemble_coarse_mass(slod_ctx *ctx);
+int slod_get_coarse_mass_csr(const slod_ctx *ctx, int64_t *rowptr, int64_t *col, double *val, int64_t *n_rows,
+                             int64_t *nnz);
+/* L2 projection onto the SLOD space of n_rhs fine fields ([n_rhs][n_fine]): M_H u = C^T M_h v, by one CG on M_H per column
+ * (diagonal preconditioner, ReductionControl).  Errors and per-column outputs as in slod_coarse_solve_batch. */
+int slod_l2_project_batch(slod_ctx *ctx, int32_t n_rhs, const double *v_fine, double *u_coarse, int32_t max_steps,
+                          double tolerance, double reduction, int32_t *steps /* [n_rhs] or NULL */,
+                          double *residual /* [n_rhs] or NULL */);
+/* Backward Euler for du/dt - div(alpha grad u) = f (elasticity: its operator) on the SLOD space, forcing constant in time:
+ * (M_H + dt K) u^k = M_H u^{k-1} + dt C^T f, k = 1 .. n_steps, solved in increment form (r = dt (C^T f - K u^{k-1}),
+ * (M_H + dt K) delta = r by CG from zero, u^k = u^{k-1} + delta; the stopping rule applies to each increment).  Needs K
+ * and M_H.  f_fine / u0_coarse NULL: zero.  Output o (o = 0 .. n_steps / out_every - 1) is u at step (o + 1) out_every.
+ * cg_steps (may be NULL) receives the CG steps of every time step.  M_H + dt K is formed once and kept while dt stays the
+ * same.  dt <= 0, n_steps < 1, out_every < 1 or > n_steps -> SLOD_ERR_INVALID.  A time step whose CG breaks down or does
+ * not converge -> SLOD_ERR_NUMERIC naming the step (and the column); every output of the steps before it is written.
+ * slod_heat_solve_batch: n_rhs trajectories ([n_rhs][n_fine] forcings, [n_rhs][n_coarse] initial values, outputs
+ * [n_out][n_rhs][n_coarse], cg_steps [n_steps][n_rhs]); column j is bit-identical whatever n_rhs, its position and its
+ * neighbours are, and slod_heat_solve agrees with it to the solver tolerance (slod_coarse_solve / _batch). */
+int slod_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_coarse, double dt, int32_t n_steps,
+                    int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
+                    int32_t *cg_steps);
+int slod_heat_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, const double *u0_coarse, double dt,
+                          int32_t n_steps, int32_t out_every, double *u_out, int32_t max_steps, double tolerance,
+                          double reduction, int32_t *cg_steps);
+/* The fine-scale reference trajectory of the same scheme, the counterpart of slod_fem_solve: (M_h + dt A_h) on the global
+ * grid with homogeneous Dirichlet rows (boundary rows of f and u0 are ignored), matrix free, diag-preconditioned CG on
+ * each increment.  Needs only the coefficient.  u_out [n_steps / out_every][n_fine]; errors as slod_heat_solve. */
+int slod_fem_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_fine, double dt, int32_t n_steps,
+                        int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
+                        int32_t *cg_steps);
+
 /* ---- checkpoint of the offline phase (SURVEY 8f row 4; the reference has none: it recomputes every run) ----------
  * slod_save_state writes the parameters, the basis (phi, A*phi) and, if assembled, the coarse matrix to one binary
  * file; slod_load_state restores them into a handle created with the SAME parameters (else SLOD_ERR_INVALID), after
@@ -213,7 +253,8 @@ int slod_measure_fp64_peak(slod_ctx *ctx, double *dfma_tflops, double *dmma_tflo
 
 /* per-kernel device times of the last compute/assemble (CUDA events), ms:
  *   [0] patch solve  [1] dense (M, BD, Gram)  [2] selection (eigen)  [3] finish (phi, A phi)
- *   [4] coarse matrix  [5] factorisation share of [0] (split solver, first chunk)  [6], [7] reserved */
+ *   [4] coarse matrix  [5] factorisation share of [0] (split solver, first chunk)
+ *   [6] M_h phi and [7] coarse mass matrix of the last slod_assemble_coarse_mass */
 int slod_get_timings(const slod_ctx *ctx, double *ms, int n);
 
 /* the hot path, device buffers (multi-GPU plumbing) ----------------------------------------------------*/
