@@ -31,8 +31,11 @@ EXPORTS = [
     "slod_comm_unique_id", "slod_comm_init", "slod_offline_distributed", "slod_save_state", "slod_load_state",
     "slod_fine_norms_reference", "slod_set_host_outputs", "slod_coarse_rhs_batch", "slod_coarse_solve_batch",
     "slod_prolongate_batch", "slod_assemble_coarse_mass", "slod_get_coarse_mass_csr", "slod_l2_project_batch",
-    "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve",
+    "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan",
 ]
+# slod_get_plan entries, in order
+PLAN_KEYS = ["mma_variant", "split_solver", "dense_ntile", "gmem_window", "dense_coef_gmem", "coarse_blocked", "use_ql",
+             "gauss_coef"]
 
 
 class SlodParams(C.Structure):
@@ -71,6 +74,7 @@ def load_library(path=None):
     lib.slod_last_create_error.restype = C.c_char_p
     lib.slod_set_coefficient.argtypes = [vp, C.c_int, C.c_int, P(dbl), C.c_size_t]
     lib.slod_patch_count.argtypes = [vp, P(i64)]
+    lib.slod_get_plan.argtypes = [vp, P(i32)]
     lib.slod_fine_size.argtypes = [vp, P(i64)]
     lib.slod_coarse_rhs.argtypes = [vp, P(dbl), P(dbl)]
     lib.slod_coarse_solve.argtypes = [vp, P(dbl), P(dbl), i32, dbl, dbl, P(i32), P(dbl)]
@@ -223,6 +227,12 @@ class SlodContext:
     def set_coefficient(self, field, eta_refinement, values):
         v = np.ascontiguousarray(values, dtype=np.float64).ravel()
         self._ck(self.lib.slod_set_coefficient(self.h, field, eta_refinement, _dp(v), v.size))
+
+    def plan(self):
+        """The kernels slod_create chose (slod_get_plan): {key: int} over PLAN_KEYS."""
+        out = (C.c_int32 * 8)()
+        self._ck(self.lib.slod_get_plan(self.h, out))
+        return dict(zip(PLAN_KEYS, (int(x) for x in out)))
 
     # -- integer maps ----------------------------------------------------------------------------------
     @property

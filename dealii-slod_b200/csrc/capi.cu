@@ -1062,7 +1062,9 @@ int slod_create(const slod_params *par, slod_ctx **out) {
     ctx->smem_solve = smem_solve_small;
   }
   DenseLayout &dl = ctx->dl;
-  dl.threads = big ? 512 : 128;
+  // the SIMT dense stage keeps kGEPT = 32 Gram entries per thread: 2-D patches with more than 64 coarse dofs need the
+  // 512-thread CTA that 3-D always uses
+  dl.threads = (big || (size_t)P.NcdMax * P.NcdMax > (size_t)32 * 128) ? 512 : 128;
   dl.ncd_max = P.NcdMax; dl.nb_max = nb_max; dl.coef_doubles = coef_doubles; dl.ldx = sl.ldx;
   dl.x_stride = sl.x_stride;
   dl.m_stride = (long long)P.NcdMax * P.NcdMax;
@@ -1269,6 +1271,23 @@ int slod_set_coefficient(slod_ctx *ctx, int field, int eta_refinement, const dou
 int slod_patch_count(const slod_ctx *ctx, int64_t *n) {
   if (!ctx || !n) return SLOD_ERR_INVALID;
   *n = ctx->n_patches;
+  return SLOD_OK;
+}
+
+int slod_get_plan(const slod_ctx *ctx, int32_t out[8]) {
+  if (!ctx || !out) return SLOD_ERR_INVALID;
+  // the rule of prepare_coefficients: one value per Gauss point once any table is finer than the sub-cells
+  int gauss = 0;
+  for (int f = 0; f < ctx->n_fields; ++f)
+    if (ctx->coef_set[f] && (1 << ctx->coef_r[f]) > ctx->P.nsub) gauss = 1;
+  out[0] = ctx->mma_variant;
+  out[1] = ctx->split_solver ? 1 : 0;
+  out[2] = ctx->dense_ntile;
+  out[3] = ctx->sl.gmem_window;
+  out[4] = ctx->dense_coef_gmem ? 1 : 0;
+  out[5] = ctx->coarse_nu > 0 ? 1 : 0;
+  out[6] = ctx->sp.use_ql;
+  out[7] = gauss;
   return SLOD_OK;
 }
 

@@ -16,7 +16,7 @@ import scipy.sparse.linalg as spla
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 from heat_oracle import coarse_mass, heat_solve_coarse, heat_solve_fine  # noqa: E402
-from parity_common import build_pair, pkg  # noqa: E402
+from parity_common import build_pair, case_id, pkg  # noqa: E402
 from test_online_gpu import _forcing, _host_C  # noqa: E402
 
 pytestmark = pytest.mark.gpu
@@ -28,8 +28,13 @@ CASES = [
     dict(dim=2, s=2, ref=3, n=2, ell=2),
     dict(dim=3, s=1, ref=2, n=2, ell=1),
     dict(dim=3, s=1, ref=2, n=2, ell=2),
+    # wide ELL rows (361 and 450 slots: k_ell_residual and the CG kernels over several 128-entry passes plus a tail) and
+    # one coefficient per Gauss point
+    dict(dim=2, s=1, ref=4, n=2, ell=4, plan=dict(mma_variant=0, dense_ntile=16)),
+    dict(dim=2, s=2, ref=3, n=2, ell=3, plan=dict(mma_variant=0, dense_ntile=16)),
+    dict(dim=2, s=1, ref=3, n=2, ell=1, r=5, plan=dict(gauss_coef=1)),
 ]
-IDS = ["-".join(f"{k}{v}" for k, v in c.items()) for c in CASES]
+IDS = [case_id(c) for c in CASES]
 CG = dict(max_steps=5000, tolerance=0.0, reduction=1e-13)
 DP = C.POINTER(C.c_double)
 

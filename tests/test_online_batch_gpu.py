@@ -13,7 +13,7 @@ import scipy.sparse.linalg as spla
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
-from parity_common import build_pair, pkg  # noqa: E402
+from parity_common import build_pair, case_id, pkg  # noqa: E402
 from test_online_gpu import END_TO_END, OPERATOR_CASES, _forcing, _host_C  # noqa: E402
 
 pytestmark = pytest.mark.gpu
@@ -46,22 +46,24 @@ def _block(rng, k, n, zero=1, repeat=(3, 0)):
     return F
 
 
-@pytest.mark.parametrize("case", OPERATOR_CASES, ids=lambda c: "-".join(f"{k}{v}" for k, v in c.items()))
+@pytest.mark.parametrize("case", OPERATOR_CASES, ids=case_id)
 def test_batch_operators(case):
-    """k = 5 with a zero and a repeated column: C^T F and C U at rounding level, the solve against scipy's direct solve
-    on the GPU's own K, the true residual, and each column against the single-vector calls."""
+    """k = 5 with a zero and a repeated column (k = 17, two groups with the last one partial, on the cases added for a
+    kernel plan): C^T F and C U at rounding level, the solve against scipy's direct solve on the GPU's own K, the true
+    residual, and each column against the single-vector calls."""
     ctx, _ = _ready(case)
     Cm = _host_C(ctx, case["n"], case["s"], case["ref"])
     K = _K(ctx)
     rng = np.random.default_rng(11)
-    F = _block(rng, 5, ctx.n_fine)
+    k = 17 if "plan" in case else 5
+    F = _block(rng, k, ctx.n_fine)
     B = ctx.coarse_rhs_batch(F)
-    assert B.shape == (5, Cm.shape[1])
+    assert B.shape == (k, Cm.shape[1])
     U, steps, res = ctx.coarse_solve_batch(B, **CG)
-    Ur = _block(rng, 5, Cm.shape[1])
+    Ur = _block(rng, k, Cm.shape[1])
     Uf = ctx.prolongate_batch(Ur)
     solve = spla.factorized(K.tocsc())
-    for j in range(5):
+    for j in range(k):
         b_ref = Cm.T @ F[j]
         uf_ref = Cm @ Ur[j]
         if j == 1:   # the zero column

@@ -18,7 +18,7 @@ import pytest
 import scipy.sparse as sp
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tools"))
-from parity_common import build_pair, pkg  # noqa: E402
+from parity_common import build_pair, case_id, pkg  # noqa: E402
 from oracle.slod_oracle import GlibcRand, reference_random_table  # noqa: E402
 
 pytestmark = pytest.mark.gpu
@@ -67,10 +67,15 @@ OPERATOR_CASES = [
     dict(dim=2, s=1, ref=3, n=2, ell=0),
     dict(dim=3, s=1, ref=2, n=2, ell=1),
     dict(dim=3, s=1, ref=3, n=2, ell=2, kind="uniform1e4", seed=3001),
+    # wide ELL rows: (2w + 1)^2 = 361 slots (ell 4) and 2 * 225 = 450 (elasticity, ell 3), several 128-entry passes of
+    # k_cg_spmv / k_cg_spmm / k_ell_residual plus a tail; one coefficient per Gauss point
+    dict(dim=2, s=1, ref=4, n=2, ell=4, plan=dict(mma_variant=0, dense_ntile=16)),
+    dict(dim=2, s=2, ref=3, n=2, ell=3, plan=dict(mma_variant=0, dense_ntile=16)),
+    dict(dim=2, s=1, ref=3, n=2, ell=1, r=5, plan=dict(gauss_coef=1)),
 ]
 
 
-@pytest.mark.parametrize("case", OPERATOR_CASES, ids=lambda c: "-".join(f"{k}{v}" for k, v in c.items()))
+@pytest.mark.parametrize("case", OPERATOR_CASES, ids=case_id)
 def test_online_operators(case):
     ctx, orc = build_pair(**case)
     n, s = case["n"], case["s"]
@@ -78,6 +83,15 @@ def test_online_operators(case):
     ctx.assemble_coarse()
     C = _host_C(ctx, n, s, case["ref"])
     assert ctx.n_fine == C.shape[0]
+    # K = C^T A_h C on the GPU's own phi: k_patch_finish (A phi) and the coarse kernel at rounding level, whatever the
+    # conditioning of the selection.  phi vanishes on the domain boundary, so the Dirichlet rows of A_h do not enter.
+    rowptr, col, val = ctx.coarse_csr()
+    _, A_h = orc.fem_solve(np.zeros(ctx.n_fine))
+    ones = C.copy()
+    ones.data[:] = 1.0
+    K_h = orc.galerkin_product(C, (A_h @ C).tocsc(), ones)
+    assert np.array_equal(rowptr, K_h.indptr) and np.array_equal(col, K_h.indices)     # bit-exact pattern
+    assert np.abs(val - K_h.data).max() <= 1e-12 * np.abs(K_h.data).max()
     rng = np.random.default_rng(7)
     # b = C^T f
     f = orc.fem_rhs(_forcing(s))
@@ -92,7 +106,6 @@ def test_online_operators(case):
     uh = ctx.prolongate(u)
     assert np.abs(uh - C @ u).max() <= 1e-12 * np.abs(C @ u).max()
     # K u = b against a direct solve with the matrix the GPU assembled
-    rowptr, col, val = ctx.coarse_csr()
     K = sp.csr_matrix((val.copy(), col.copy(), rowptr.copy()), shape=(C.shape[1],) * 2)
     x, steps, res = ctx.coarse_solve(b, max_steps=5000, tolerance=0.0, reduction=1e-13)
     x_ref, _ = orc.solve_coarse(K, b, direct=True)

@@ -34,8 +34,21 @@ def make_tables(dim, s, r, kind, seed):
     return out
 
 
+def case_id(case):
+    """Test id of a case dict; the expected plan is not part of it."""
+    return "-".join(f"{k}{v}" for k, v in case.items() if k != "plan")
+
+
+def check_plan(ctx, want):
+    """The kernels slod_create chose (slod_get_plan) include ``want`` ({PLAN_KEYS entry: value})."""
+    got = ctx.plan()
+    assert {k: got[k] for k in want} == want, got
+
+
 def build_pair(dim=2, s=1, ref=3, n=2, ell=1, stabilize=True, r=None, kind="uniform100", seed=1234, quirk=False,
-               tables=None):
+               tables=None, plan=None):
+    """GPU handle and oracle of one configuration.  ``plan``: the kernel variants the configuration exists to run,
+    asserted through slod_get_plan once the coefficients are set."""
     r = min(ref + int(np.log2(n)), 8 if dim == 2 else 6) if r is None else r
     tables = make_tables(dim, s, r, kind, seed) if tables is None else tables
     problem = "diffusion" if s == 1 else "elasticity"
@@ -43,6 +56,8 @@ def build_pair(dim=2, s=1, ref=3, n=2, ell=1, stabilize=True, r=None, kind="unif
                           stabilize=stabilize, problem=0 if s == 1 else 1, quirk_presaved=quirk)
     for f, t in enumerate(tables):
         ctx.set_coefficient(f, r, t)
+    if plan is not None:
+        check_plan(ctx, plan)
     prob = SlodProblem(dim=dim, spacedim=s, n_global_refinements=ref, n_subdivisions=n, oversampling=ell,
                        stabilize=stabilize, problem=problem, quirk_presaved=quirk,
                        coefficients=[CoefficientTable(dim, r, t) for t in tables])
