@@ -31,7 +31,7 @@ EXPORTS = [
     "slod_comm_unique_id", "slod_comm_init", "slod_offline_distributed", "slod_save_state", "slod_load_state",
     "slod_fine_norms_reference", "slod_set_host_outputs", "slod_coarse_rhs_batch", "slod_coarse_solve_batch",
     "slod_prolongate_batch", "slod_assemble_coarse_mass", "slod_get_coarse_mass_csr", "slod_l2_project_batch",
-    "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan",
+    "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan", "slod_debug_select",
 ]
 # slod_get_plan entries, in order
 PLAN_KEYS = ["mma_variant", "split_solver", "dense_ntile", "gmem_window", "dense_coef_gmem", "coarse_blocked", "use_ql",
@@ -103,6 +103,7 @@ def load_library(path=None):
     lib.slod_get_coarse_csr.argtypes = [vp, P(i64), P(i64), P(dbl), P(i64), P(i64)]
     lib.slod_get_patch_diagnostics.argtypes = [vp, i64, C.c_int, P(dbl)]
     lib.slod_debug_patch_stages.argtypes = [vp, i64, P(dbl), P(dbl), P(dbl)]
+    lib.slod_debug_select.argtypes = [vp, i64, P(i64), P(dbl), P(dbl), P(dbl), P(dbl)]
     lib.slod_get_timings.argtypes = [vp, P(dbl), C.c_int]
     lib.slod_compute_basis_device.argtypes = [vp, i64, i64, vp, vp, vp]
     lib.slod_assemble_coarse_device.argtypes = [vp, i64, i64, vp, vp, vp, vp]
@@ -494,6 +495,10 @@ class SlodContext:
         return l2.value, li.value, h1.value
 
     def diagnostics(self, patch, comp=0):
+        """8 doubles (slod_get_patch_diagnostics): [0] ||d||_inf before truncation, [1] truncation steps, [5] path
+        (0 LOD, 1 Cholesky fast path, 2 Jacobi, 3 QL), [6] QL iterations / Jacobi sweeps, [7] status bits.  [2], [3] by
+        path: 0 -> zeros; 1 -> largest diagonal entry of G_o and smallest LDL^T pivot (bounds: sigma_0 / n <= [2] <=
+        sigma_0, lambda_min <= [3] <= [2]); 2, 3 -> sigma_0 and the smallest sigma still used."""
         out = np.empty(8)
         self._ck(self.lib.slod_get_patch_diagnostics(self.h, patch, comp, _dp(out)))
         return out
@@ -506,6 +511,26 @@ class SlodContext:
         G = np.empty((ncd, ncd)) if want_G else None
         self._ck(self.lib.slod_debug_patch_stages(self.h, patch, _dp(X), _dp(Minv), _dp(G) if want_G else None))
         return X, Minv, G
+
+    def debug_select(self, patches, G, Minv):
+        """The selection stage on caller matrices (slod_debug_select).  patches: distinct ids; G, Minv: one
+        (n_coarse, n_coarse) array per patch, reference column order.  Returns (c, diag): c a list of (spacedim, n_coarse)
+        arrays, diag (len(patches), spacedim, 8) in the layout of diagnostics()."""
+        ids = np.ascontiguousarray(patches, dtype=np.int64).ravel()
+        if len(G) != ids.size or len(Minv) != ids.size:
+            raise ValueError("one G and one Minv per patch")
+        ncd = [self.patch_info(int(p))["n_coarse"] for p in ids]
+        for k, (g, m) in enumerate(zip(G, Minv)):
+            if np.shape(g) != (ncd[k], ncd[k]) or np.shape(m) != (ncd[k], ncd[k]):
+                raise ValueError(f"patch {ids[k]}: G and Minv must be {ncd[k]} x {ncd[k]}")
+        g = np.concatenate([np.asarray(x, dtype=np.float64).ravel() for x in G]) if ids.size else np.zeros(1)
+        m = np.concatenate([np.asarray(x, dtype=np.float64).ravel() for x in Minv]) if ids.size else np.zeros(1)
+        c = np.empty(max(1, self.s * sum(ncd)))
+        diag = np.empty((ids.size, self.s, 8))
+        self._ck(self.lib.slod_debug_select(self.h, ids.size, ids.ctypes.data_as(C.POINTER(C.c_int64)), _dp(g), _dp(m),
+                                            _dp(c), _dp(diag)))
+        off = np.concatenate([[0], np.cumsum([self.s * k for k in ncd])]).astype(int)
+        return [c[off[i]:off[i + 1]].reshape(self.s, ncd[i]) for i in range(ids.size)], diag
 
     def timings(self):
         out = np.zeros(8)

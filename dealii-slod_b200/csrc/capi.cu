@@ -493,6 +493,8 @@ void free_workspace(slod_ctx *c) {
 // call with a larger range reallocates.  ctx->chunk is committed only after every allocation has succeeded: a failed
 // allocation leaves the handle without a workspace (chunk == 0) instead of with dangling null pointers.
 // SLOD_CHUNK (environment) forces a small chunk: the multi-chunk loop is exercised by tests/test_parity_gpu.py.
+// SLOD_EIG_CAP forces few eigen items per round of the selection pipeline: the round loop is exercised by
+// tests/test_select_gpu.py.
 int ensure_workspace(slod_ctx *ctx, int64_t n_range) {
   const Params &P = ctx->P;
   n_range = std::max<int64_t>(1, std::min<int64_t>(n_range, ctx->n_patches));
@@ -543,6 +545,7 @@ int ensure_workspace(slod_ctx *ctx, int64_t n_range) {
       const size_t per_item = sizeof(double) * ((size_t)sp.eig.h_stride + sp.eig.v_stride) +
                               (size_t)sp.eig.log_cap * (sizeof(double2) + sizeof(unsigned short)) + 2 * sizeof(int);
       size_t cap = std::max<size_t>(64, ((size_t)4 << 30) / per_item);
+      if (const char *env = getenv("SLOD_EIG_CAP")) cap = (size_t)std::max(1, atoi(env));
       cap = std::min(cap, items);
       sp.eig.cap_items = (int)cap;
       CK(cudaMalloc(&sb.H, sizeof(double) * (size_t)sp.eig.h_stride * cap));
@@ -2683,6 +2686,107 @@ int slod_debug_patch_stages(slod_ctx *ctx, int64_t patch, double *X, double *Min
       }
   }
   return SLOD_OK;
+}
+
+int slod_debug_select(slod_ctx *ctx, int64_t n, const int64_t *patches, const double *G, const double *Minv, double *c,
+                      double *diag) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  if (n < 0 || (n > 0 && (!patches || !G || !Minv || !c || !diag))) return fail(ctx, SLOD_ERR_INVALID, "bad argument");
+  const Params &P = ctx->P;
+  const int s = P.s;
+  // host checks first: nothing is launched on an invalid list
+  std::vector<int64_t> moff((size_t)n + 1, 0), coff((size_t)n + 1, 0);   // offsets of the packed matrices / c blocks
+  std::vector<char> seen((size_t)ctx->n_patches, 0);
+  for (int64_t i = 0; i < n; ++i) {
+    const int64_t p = patches[i];
+    if (p < 0 || p >= ctx->n_patches) return fail(ctx, SLOD_ERR_INVALID, "patch id out of range");
+    if (seen[(size_t)p]) return fail(ctx, SLOD_ERR_INVALID, "repeated patch id " + std::to_string(p));
+    seen[(size_t)p] = 1;
+    const int ncd = make_geom(P, (int)p).Ncd;
+    moff[i + 1] = moff[i] + (int64_t)ncd * ncd;
+    coff[i + 1] = coff[i] + (int64_t)s * ncd;
+  }
+  for (int64_t k = 0; k < moff[n]; ++k)
+    if (!std::isfinite(G[k]) || !std::isfinite(Minv[k]))
+      return fail(ctx, SLOD_ERR_INVALID, "non-finite entry in G or Minv");
+  NEED_DEVICE();
+  if (n == 0) return SLOD_OK;
+  CK(cudaSetDevice(ctx->device));
+  int rc = wait_basis(ctx);   // the workspace of an enqueued range is about to be reused
+  if (rc) return rc;
+  rc = ensure_workspace(ctx, n);
+  if (rc) return rc;
+  BIND_PARAMS((cudaStream_t)0);
+  ctx->ids_p0 = ctx->ids_p1 = -1;   // the device work list is overwritten below
+  // the kernels write diagnostics at patch id * s + d and status bits at the patch id: scratch copies of both keep the
+  // handle's own arrays untouched
+  const size_t n_diag = (size_t)8 * s * ctx->n_patches;
+  double *d_dg = nullptr;
+  int *d_st = nullptr;
+  auto body = [&]() -> int {
+    CK(cudaMalloc(&d_dg, sizeof(double) * n_diag));
+    CK(cudaMalloc(&d_st, sizeof(int) * (size_t)ctx->n_patches));
+    CK(cudaMemset(d_dg, 0, sizeof(double) * n_diag));
+    CK(cudaMemset(d_st, 0, sizeof(int) * (size_t)ctx->n_patches));
+    const int64_t ms = ctx->dl.m_stride, ldc = P.NcdMax;
+    std::vector<double> hG, hM, hc;
+    std::vector<int> ids, zpos;
+    for (int64_t i0 = 0; i0 < n; i0 += ctx->chunk) {
+      const int nc = (int)std::min<int64_t>(ctx->chunk, n - i0);
+      ids.assign(patches + i0, patches + i0 + nc);
+      hG.assign((size_t)nc * ms, 0.0);
+      hM.assign((size_t)nc * ms, 0.0);
+      for (int w = 0; w < nc; ++w) {
+        const Geom g = make_geom(P, ids[w]);
+        const int ncd = g.Ncd;
+        const double *Gi = G + moff[i0 + w], *Mi = Minv + moff[i0 + w];
+        zpos.resize((size_t)ncd);
+        for (int col = 0; col < ncd; ++col) {   // reference column -> internal column (identity but on the split solver)
+          int k[3];
+          col_to_cell(P, g, col, k);
+          zpos[col] = ctx->split_solver ? zcell_to_col(g, k) : col;
+        }
+        for (int r = 0; r < ncd; ++r)
+          for (int col = 0; col < ncd; ++col) {
+            hG[(size_t)w * ms + (size_t)zpos[r] * ncd + zpos[col]] = Gi[(size_t)r * ncd + col];
+            hM[(size_t)w * ms + (size_t)zpos[r] * ncd + zpos[col]] = Mi[(size_t)r * ncd + col];
+          }
+      }
+      CK(cudaMemcpy(ctx->d_ids, ids.data(), sizeof(int) * nc, cudaMemcpyHostToDevice));
+      CK(cudaMemcpy(ctx->d_G, hG.data(), sizeof(double) * hG.size(), cudaMemcpyHostToDevice));
+      CK(cudaMemcpy(ctx->d_Minv, hM.data(), sizeof(double) * hM.size(), cudaMemcpyHostToDevice));
+      int nl = 0;
+      CK(launch_select_pipeline(ctx->sp, 0, ctx->d_ids, nc, ctx->d_Minv, ctx->d_G, ctx->d_cvec, d_dg, d_st, ctx->sb, &nl));
+      ctx->launches += nl;
+      hc.resize((size_t)nc * s * ldc);
+      CK(cudaMemcpy(hc.data(), ctx->d_cvec, sizeof(double) * hc.size(), cudaMemcpyDeviceToHost));
+      for (int w = 0; w < nc; ++w) {
+        const Geom g = make_geom(P, ids[w]);
+        const int ncd = g.Ncd;
+        for (int col = 0; col < ncd; ++col) {
+          int k[3];
+          col_to_cell(P, g, col, k);
+          const int zc = ctx->split_solver ? zcell_to_col(g, k) : col;
+          for (int d = 0; d < s; ++d) c[coff[i0 + w] + (int64_t)d * ncd + col] = hc[((size_t)w * s + d) * ldc + zc];
+        }
+      }
+    }
+    std::vector<double> hdg(n_diag);
+    std::vector<int> hst((size_t)ctx->n_patches);
+    CK(cudaMemcpy(hdg.data(), d_dg, sizeof(double) * n_diag, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(hst.data(), d_st, sizeof(int) * hst.size(), cudaMemcpyDeviceToHost));
+    for (int64_t i = 0; i < n; ++i)
+      for (int d = 0; d < s; ++d) {
+        double *out = diag + ((size_t)i * s + d) * 8;
+        std::memcpy(out, hdg.data() + ((size_t)patches[i] * s + d) * 8, sizeof(double) * 8);
+        out[7] = hst[(size_t)patches[i]];
+      }
+    return SLOD_OK;
+  };
+  rc = body();
+  if (d_dg) cudaFree(d_dg);
+  if (d_st) cudaFree(d_st);
+  return rc;
 }
 
 int slod_measure_fp64_peak(slod_ctx *ctx, double *dfma_tflops, double *dmma_tflops) {

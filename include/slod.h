@@ -252,13 +252,29 @@ int slod_alloc_host(size_t bytes, void **out);
 int slod_free_host(void *p);
 
 /* diagnostics: per patch and component 8 doubles:
- *   [0] ||d||_inf before truncation  [1] truncation steps  [2] sigma_0  [3] smallest kept sigma
+ *   [0] ||d||_inf before truncation  [1] truncation steps  [2], [3] see below
  *   [4] reserved  [5] selection path (0 LOD branch, 1 Cholesky fast path, 2 Jacobi fallback, 3 tridiagonal QL)
- *   [6] QL iterations / Jacobi sweeps [7] status bits */
+ *   [6] QL iterations / Jacobi sweeps (0 on paths 0 and 1)  [7] status bits
+ * [2] and [3] depend on the path.  G_o is the Gram matrix without row and column d, of size n = n_coarse - 1:
+ *   path 0: both 0 (no selection).
+ *   path 1: [2] the largest diagonal entry of G_o, [3] the smallest pivot of its LDL^T factorisation.  Bounds, not
+ *           eigenvalues: sigma_0 / n <= [2] <= sigma_0 and lambda_min(G_o) <= [3] <= [2].  The path is only taken when
+ *           [3] > 1e-12 [2], no pivot is <= 0 and ||d||_inf < 0.49 (then [1] = 0: the truncation loop does not fire).
+ *   paths 2, 3: [2] sigma_0 (largest |eigenvalue| of G_o), [3] the smallest sigma still used after the 1e-15 sigma_0
+ *           threshold and the [1] truncation steps (sigma_0 when none is left). */
 int slod_get_patch_diagnostics(const slod_ctx *ctx, int64_t patch, int comp, double out[8]);
 /* stage intermediates of one patch for staged parity tests (recomputed on demand for that patch):
  * X = A_ii^{-1} P_i  (n_internal x n_coarse, row-major), Minv (n_coarse^2), BD^T BD (n_coarse^2). Any may be NULL. */
 int slod_debug_patch_stages(slod_ctx *ctx, int64_t patch, double *X, double *Minv, double *G);
+/* the selection stage (source/LOD.cc:637-743) run exactly as slod_compute_basis runs it (same kernels, same plan:
+ * SLOD_NO_FAST_SELECT, SLOD_FORCE_JACOBI and SLOD_EIG_CAP apply), on caller matrices, for selection tests.
+ *   patches: n distinct patch ids (the patch fixes n_coarse and the LOD / SLOD branch);
+ *   G, Minv: packed per patch, n_coarse^2 each, row-major, reference column order;
+ *   c: packed per patch, [spacedim][n_coarse];  diag: [n][spacedim][8] in the layout of slod_get_patch_diagnostics.
+ * The handle's basis, coarse matrices, diagnostics and status words are left unchanged.  Repeated or out-of-range patch
+ * ids and non-finite entries: SLOD_ERR_INVALID, before anything runs. */
+int slod_debug_select(slod_ctx *ctx, int64_t n, const int64_t *patches, const double *G, const double *Minv, double *c,
+                      double *diag);
 
 /* FP64 throughput of the handle's device in TFLOP/s, measured now with two register-resident probe kernels: a DFMA chain
  * and an mma.sync.m8n8k4.f64 chain (the instruction of the tensor-core kernels).  The benchmark's roofline denominator. */
