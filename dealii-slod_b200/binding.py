@@ -32,6 +32,7 @@ EXPORTS = [
     "slod_fine_norms_reference", "slod_set_host_outputs", "slod_coarse_rhs_batch", "slod_coarse_solve_batch",
     "slod_prolongate_batch", "slod_assemble_coarse_mass", "slod_get_coarse_mass_csr", "slod_l2_project_batch",
     "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan", "slod_debug_select",
+    "slod_update_basis",
 ]
 # slod_get_plan entries, in order
 PLAN_KEYS = ["mma_variant", "split_solver", "dense_ntile", "gmem_window", "dense_coef_gmem", "coarse_blocked", "use_ql",
@@ -96,6 +97,7 @@ def load_library(path=None):
     lib.slod_get_patch_local_dofs.argtypes = [vp, i64, P(C.c_uint32), P(i32)]
     lib.slod_get_patch_dof_class.argtypes = [vp, i64, C.c_int, P(C.c_uint32), P(i32)]
     lib.slod_compute_basis.argtypes = [vp]
+    lib.slod_update_basis.argtypes = [vp, P(i64), P(i64)]
     lib.slod_get_basis.argtypes = [vp, i64, C.c_int, P(dbl), P(dbl)]
     lib.slod_basis_stride.argtypes = [vp, P(i64)]
     lib.slod_get_all_basis.argtypes = [vp, P(dbl), P(dbl)]
@@ -285,6 +287,13 @@ class SlodContext:
     # -- hot path, host buffers --------------------------------------------------------------------------
     def compute_basis(self):
         self._ck(self.lib.slod_compute_basis(self.h))
+
+    def update_basis(self):
+        """Recompute only the patches (and K row blocks) the coefficient change since the last compute_basis /
+        update_basis reaches (slod_update_basis).  Returns {"patches": n, "row_blocks": m}."""
+        n, m = C.c_int64(), C.c_int64()
+        self._ck(self.lib.slod_update_basis(self.h, C.byref(n), C.byref(m)))
+        return {"patches": n.value, "row_blocks": m.value}
 
     def basis(self, patch, comp=0):
         nf = self.patch_info(patch)["n_fine"]

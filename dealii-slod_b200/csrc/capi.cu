@@ -121,6 +121,16 @@ struct slod_ctx {
   double *h_out_phi = nullptr, *h_out_aphi = nullptr, *h_out_K = nullptr;   // slod_set_host_outputs
   cudaEvent_t ev_out[2]{};       // basis rows ready | coarse rows ready
   bool out_pending = false;
+  // slod_update_basis: the device coefficient array the handle's basis was computed from (its baseline), and whether
+  // d_Kell holds the coarse matrix of that basis
+  double *d_coef_base = nullptr;
+  size_t base_elems = 0;
+  int base_gauss = 0;
+  bool have_base = false, base_coarse = false;
+  unsigned char *d_cell_changed = nullptr;   // [n_patches]: one flag per coarse cell
+  int *d_rows = nullptr;                     // coarse rows (patches or Morton groups) to recompute
+  size_t rows_cap = 0;
+  std::vector<int> update_ids, update_rows;
 };
 
 namespace {
@@ -417,6 +427,7 @@ void free_dev(slod_ctx *c) {
   F(c->d_coef); F(c->d_phi); F(c->d_aphi); F(c->d_Kell); F(c->d_diag); F(c->d_status);
   F(c->d_perm); F(c->d_val); F(c->d_online); F(c->d_batch);
   F(c->d_Mell); F(c->d_Mval); F(c->d_Sell); F(c->d_heat);
+  F(c->d_coef_base); F(c->d_cell_changed); F(c->d_rows);
   free_workspace(c);
 }
 
@@ -573,19 +584,24 @@ int ensure_workspace(slod_ctx *ctx, int64_t n_range) {
 // Enqueues stages assembly .. premultiply for the patches [p0, p1) on `st` and returns without waiting: the work list
 // of the whole range is uploaded once, every chunk has its own timing events, the status words of the range are cleared
 // in front of the kernels and copied to page-locked host memory behind them.  wait_basis() is the synchronisation point.
-int run_basis(slod_ctx *ctx, int64_t p0, int64_t p1, double *d_phi, double *d_aphi, cudaStream_t st) {
+// `list` (ascending patch ids): only these patches are computed, in the same cost order as in a range; the status words
+// of [p0, p1) are still cleared and read back, so the caller passes a range that covers the list.
+int run_basis(slod_ctx *ctx, int64_t p0, int64_t p1, double *d_phi, double *d_aphi, cudaStream_t st,
+              const std::vector<int> *list = nullptr) {
   const Params &P = ctx->P;
   if (p0 < 0 || p1 > ctx->n_patches || p0 > p1) return fail(ctx, SLOD_ERR_INVALID, "bad patch range");
-  if (p0 == p1) return SLOD_OK;
+  const int64_t n_work = list ? (int64_t)list->size() : p1 - p0;
+  if (n_work == 0) return SLOD_OK;
   int rc = prepare_coefficients(ctx);
   if (rc) return rc;
-  rc = ensure_workspace(ctx, p1 - p0);
+  rc = ensure_workspace(ctx, n_work);
   if (rc) return rc;
   BIND_PARAMS(st);
-  // work order: largest patches first (integer geometry: cached per range, on the host and on the device)
-  if (ctx->ids_p0 != p0 || ctx->ids_p1 != p1) {
-    std::vector<int> order((size_t)(p1 - p0));
-    std::iota(order.begin(), order.end(), (int)p0);
+  // work order: largest patches first (integer geometry: cached per range, on the host and on the device; a list is not
+  // cached, and the next range uploads its own)
+  if (list || ctx->ids_p0 != p0 || ctx->ids_p1 != p1) {
+    std::vector<int> order = list ? *list : std::vector<int>((size_t)(p1 - p0));
+    if (!list) std::iota(order.begin(), order.end(), (int)p0);
     std::vector<long long> cost(order.size());
     for (size_t i = 0; i < order.size(); ++i) {
       const Geom g = make_geom(P, order[i]);
@@ -598,8 +614,8 @@ int run_basis(slod_ctx *ctx, int64_t p0, int64_t p1, double *d_phi, double *d_ap
     for (size_t i = 0; i < perm.size(); ++i) ctx->ids[i] = order[perm[i]];
     CK(cudaMemcpyAsync(ctx->d_ids, ctx->ids.data(), sizeof(int) * ctx->ids.size(), cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));   // pageable source: the vector may be rebuilt by the next call
-    ctx->ids_p0 = p0;
-    ctx->ids_p1 = p1;
+    ctx->ids_p0 = list ? -1 : p0;
+    ctx->ids_p1 = list ? -1 : p1;
   }
   const size_t n_ids = ctx->ids.size();
   if (!ctx->h_status) CK(cudaHostAlloc(&ctx->h_status, sizeof(int) * (size_t)ctx->n_patches, cudaHostAllocDefault));
@@ -695,6 +711,20 @@ int wait_basis(slod_ctx *ctx) {
   return SLOD_OK;
 }
 
+// Enqueues the copy of the device coefficient array that the basis just enqueued on stream 0 reads: the baseline of
+// slod_update_basis once the basis has succeeded (a few MB, device to device).
+int snapshot_coefficients(slod_ctx *ctx) {
+  if (ctx->d_coef_base && ctx->base_elems != ctx->d_coef_elems) {
+    CK(cudaFree(ctx->d_coef_base));
+    ctx->d_coef_base = nullptr;
+  }
+  if (!ctx->d_coef_base) CK(cudaMalloc(&ctx->d_coef_base, sizeof(double) * ctx->d_coef_elems));
+  ctx->base_elems = ctx->d_coef_elems;
+  ctx->base_gauss = ctx->P.gauss_coef;
+  CK(cudaMemcpyAsync(ctx->d_coef_base, ctx->d_coef, sizeof(double) * ctx->d_coef_elems, cudaMemcpyDeviceToDevice, 0));
+  return SLOD_OK;
+}
+
 int finish_coarse_timing(slod_ctx *ctx) {
   if (!ctx->coarse_timing_pending) return SLOD_OK;
   ctx->coarse_timing_pending = false;
@@ -705,15 +735,20 @@ int finish_coarse_timing(slod_ctx *ctx) {
   return SLOD_OK;
 }
 
+// Rows of the coarse matrix for the patches [p0, p1), or, with d_list, for the n_list entries of that device list:
+// Morton groups (patch id >> dim) on the blocked kernel, patches otherwise; [p0, p1) is then the whole matrix.
 int run_coarse(slod_ctx *ctx, int64_t p0, int64_t p1, const double *d_phi, const double *d_aphi, double *d_K,
-               cudaStream_t st, bool wait = true) {
+               cudaStream_t st, bool wait = true, const int *d_list = nullptr, int n_list = 0) {
   if (p0 < 0 || p1 > ctx->n_patches || p0 > p1) return fail(ctx, SLOD_ERR_INVALID, "bad patch range");
-  if (p0 == p1) return SLOD_OK;
+  if (p0 == p1 || (d_list && n_list == 0)) return SLOD_OK;
   BIND_PARAMS(st);
   CK(cudaEventRecord(ctx->ev[5], st));
   if (ctx->coarse_nu > 0)
     CK(launch_coarse_blocked(ctx->P.dim, ctx->P.s, ctx->n_sm, ctx->smem_coarse_blk, st, (int)p0, (int)p1, d_phi, d_aphi,
-                             d_K, ctx->fl, ctx->coarse_nu));
+                             d_K, ctx->fl, ctx->coarse_nu, d_list, n_list));
+  else if (d_list)
+    CK(launch_coarse(std::min(n_list, ctx->grid_coarse), ctx->smem_coarse, st, 0, n_list, d_phi, d_aphi, d_K, ctx->fl,
+                     d_list));
   else
     CK(launch_coarse((int)std::min<int64_t>(p1 - p0, ctx->grid_coarse), ctx->smem_coarse, st, (int)p0, (int)p1, d_phi,
                      d_aphi, d_K, ctx->fl));
@@ -1427,6 +1462,7 @@ int slod_compute_basis_device(slod_ctx *ctx, int64_t p0, int64_t p1, double *d_p
   NEED_DEVICE();
   if (!ctx->subs.empty()) return fail(ctx, SLOD_ERR_UNSUPPORTED, "device-buffer entry points need a single-device handle (n_gpus <= 1)");
   CK(cudaSetDevice(ctx->device));
+  ctx->have_base = ctx->base_coarse = false;   // the handle's diagnostics and status words now describe this run
   return run_basis(ctx, p0, p1, d_phi, d_aphi, (cudaStream_t)stream);
 }
 
@@ -1449,13 +1485,16 @@ int slod_compute_basis(slod_ctx *ctx) {
     CK(cudaMalloc(&ctx->d_aphi, sizeof(double) * n));
   }
   ctx->basis_done = ctx->coarse_done = false;
+  ctx->have_base = ctx->base_coarse = false;
   invalidate_mass(ctx);
   if (!ctx->subs.empty()) return multi_basis(ctx);
   int rc = run_basis(ctx, 0, ctx->n_patches, ctx->d_phi, ctx->d_aphi, 0);
   if (rc) return rc;
+  rc = snapshot_coefficients(ctx);
+  if (rc) return rc;
   rc = wait_basis(ctx);
   if (rc) return rc;
-  ctx->basis_done = true;
+  ctx->basis_done = ctx->have_base = true;
   return SLOD_OK;
 }
 
@@ -1504,6 +1543,7 @@ int slod_offline_distributed(slod_ctx *ctx, double *d_phi, double *d_aphi, doubl
   if (!ctx->subs.empty()) return fail(ctx, SLOD_ERR_UNSUPPORTED, "use slod_compute_basis / slod_assemble_coarse on an n_gpus > 1 handle");
   if (ctx->comm_world > 1 && !ctx->comm) return fail(ctx, SLOD_ERR_STATE, "slod_comm_init has not run");
   CK(cudaSetDevice(ctx->device));
+  ctx->have_base = ctx->base_coarse = false;   // the handle's diagnostics and status words now describe this run
   cudaStream_t st = (cudaStream_t)stream;
   int64_t b, e;
   owned_range(ctx->n_patches, ctx->comm_rank, ctx->comm_world, &b, &e);
@@ -1647,6 +1687,108 @@ int slod_assemble_coarse(slod_ctx *ctx) {
   CK(launch_gather(0, ctx->d_Kell, ctx->d_perm, ctx->d_val, ctx->csr_nnz));   // compact block-ELL -> CSR values
   ctx->launches += 1;
   ctx->coarse_done = true;
+  ctx->base_coarse = ctx->have_base;
+  return SLOD_OK;
+}
+
+// A patch reads the coefficient window of the coarse cells [clo, clo + m) (load_coef, kernels.cu): it is recomputed iff
+// one of those cells holds a value that differs bitwise from the baseline.  A row block of K depends on phi of its patch
+// and on A phi of the column patches of its CSR row; the pattern is symmetric, so the rows to recompute are the CSR
+// columns of the recomputed patches' rows.
+int slod_update_basis(slod_ctx *ctx, int64_t *n_patches_recomputed, int64_t *n_row_blocks_recomputed) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  if (n_patches_recomputed) *n_patches_recomputed = 0;
+  if (n_row_blocks_recomputed) *n_row_blocks_recomputed = 0;
+  NEED_DEVICE();
+  if (!ctx->subs.empty())
+    return fail(ctx, SLOD_ERR_UNSUPPORTED, "slod_update_basis needs a single-device handle: an n_gpus > 1 handle splits "
+                "the patches into fixed ranges per device, and a changed region falls into some of them only");
+  if (!ctx->have_base)
+    return fail(ctx, SLOD_ERR_STATE, "no baseline to update: slod_compute_basis has not succeeded on this handle since "
+                "it was created, restored by slod_load_state or used by a device-buffer entry point");
+  CK(cudaSetDevice(ctx->device));
+  int rc = finish_coarse_timing(ctx);   // the times of an earlier slod_assemble_coarse are collected now, not later
+  if (rc) return rc;
+  rc = prepare_coefficients(ctx);
+  if (rc) return rc;
+  BIND_PARAMS((cudaStream_t)0);
+  const Params &P = ctx->P;
+  const int64_t np = ctx->n_patches;   // = N^dim coarse cells
+  std::vector<unsigned char> changed((size_t)np, 1);
+  if (ctx->base_elems == ctx->d_coef_elems && ctx->base_gauss == P.gauss_coef) {   // else the layout changed: all cells
+    if (!ctx->d_cell_changed) CK(cudaMalloc(&ctx->d_cell_changed, (size_t)np));
+    CK(launch_coef_diff(0, ctx->d_coef_base, ctx->d_coef, (long long)ctx->d_coef_elems, P.dim, P.N, P.n,
+                        P.gauss_coef ? 1 << P.dim : 1, ctx->d_cell_changed));
+    ctx->launches += 1;
+    CK(cudaMemcpyAsync(changed.data(), ctx->d_cell_changed, (size_t)np, cudaMemcpyDeviceToHost, 0));
+    CK(cudaStreamSynchronize(0));
+  }
+  // box sums of the flags: S(x, y, z) = changed cells below (x, y, z) on every axis
+  const int N = P.N, Nz = (P.dim == 3) ? N : 1;
+  std::vector<int> S((size_t)(N + 1) * (N + 1) * (Nz + 1), 0);
+  auto at = [&](int x, int y, int z) -> int & { return S[((size_t)z * (N + 1) + y) * (N + 1) + x]; };
+  for (int z = 0; z < Nz; ++z)
+    for (int y = 0; y < N; ++y)
+      for (int x = 0; x < N; ++x)
+        at(x + 1, y + 1, z + 1) = changed[((size_t)z * N + y) * N + x] + at(x, y + 1, z + 1) + at(x + 1, y, z + 1) +
+                                  at(x + 1, y + 1, z) - at(x, y, z + 1) - at(x, y + 1, z) - at(x + 1, y, z) + at(x, y, z);
+  std::vector<int> &ids = ctx->update_ids;
+  ids.clear();
+  for (int64_t pid = 0; pid < np; ++pid) {
+    const Geom g = make_geom(P, (int)pid);
+    const int x0 = g.clo[0], y0 = g.clo[1], z0 = g.clo[2], x1 = x0 + g.m[0], y1 = y0 + g.m[1], z1 = z0 + g.m[2];
+    const int n_changed = at(x1, y1, z1) - at(x0, y1, z1) - at(x1, y0, z1) - at(x1, y1, z0) + at(x0, y0, z1) +
+                          at(x0, y1, z0) + at(x1, y0, z0) - at(x0, y0, z0);
+    if (n_changed > 0) ids.push_back((int)pid);
+  }
+  if (n_patches_recomputed) *n_patches_recomputed = (int64_t)ids.size();
+  for (int k = 0; k < 6; ++k) ctx->tm.ms[k] = 0.0;
+  if (ids.empty()) {   // the basis (and K, if it was assembled) are those of the current coefficient already
+    ctx->basis_done = true;
+    ctx->coarse_done = ctx->base_coarse;
+    return SLOD_OK;
+  }
+  ctx->basis_done = ctx->coarse_done = false;
+  ctx->have_base = false;
+  invalidate_mass(ctx);
+  // the status words of every patch are cleared and read back: outside the list they are zero after the basis that
+  // set the baseline, so the first nonzero word belongs to the first failing patch of the list, as in slod_compute_basis
+  rc = run_basis(ctx, 0, np, ctx->d_phi, ctx->d_aphi, 0, &ids);
+  if (rc) return rc;
+  rc = snapshot_coefficients(ctx);
+  if (rc) return rc;
+  rc = wait_basis(ctx);
+  if (rc) {
+    ctx->base_coarse = false;
+    return rc;
+  }
+  ctx->basis_done = ctx->have_base = true;
+  if (!ctx->base_coarse) return SLOD_OK;
+  std::vector<unsigned char> row((size_t)np, 0);
+  const int s = P.s;
+  for (int q : ids)
+    for (int64_t k = ctx->csr_rowptr[(size_t)q * s]; k < ctx->csr_rowptr[(size_t)q * s + 1]; k += s)
+      row[(size_t)(ctx->csr_col[k] / s)] = 1;
+  std::vector<int> &rows = ctx->update_rows;   // Morton groups on the blocked kernel, patches otherwise
+  rows.clear();
+  const int gsz = (ctx->coarse_nu > 0) ? 1 << P.dim : 1;
+  for (int64_t g = 0; g < np / gsz; ++g)
+    if (std::any_of(row.begin() + g * gsz, row.begin() + (g + 1) * gsz, [](unsigned char v) { return v != 0; }))
+      rows.push_back((int)g);
+  if (rows.size() > ctx->rows_cap) {
+    if (ctx->d_rows) CK(cudaFree(ctx->d_rows));
+    ctx->d_rows = nullptr;
+    ctx->rows_cap = 0;
+    CK(cudaMalloc(&ctx->d_rows, sizeof(int) * rows.size()));
+    ctx->rows_cap = rows.size();
+  }
+  CK(cudaMemcpyAsync(ctx->d_rows, rows.data(), sizeof(int) * rows.size(), cudaMemcpyHostToDevice, 0));
+  rc = run_coarse(ctx, 0, np, ctx->d_phi, ctx->d_aphi, ctx->d_Kell, 0, false, ctx->d_rows, (int)rows.size());
+  if (rc) return rc;
+  CK(launch_gather(0, ctx->d_Kell, ctx->d_perm, ctx->d_val, ctx->csr_nnz));
+  ctx->launches += 1;
+  ctx->coarse_done = true;
+  if (n_row_blocks_recomputed) *n_row_blocks_recomputed = (int64_t)rows.size() * gsz;
   return SLOD_OK;
 }
 
@@ -2570,6 +2712,7 @@ int slod_load_state(slod_ctx *ctx, const char *path) {
   }
   ctx->basis_done = ok;
   ctx->coarse_done = false;
+  ctx->have_base = ctx->base_coarse = false;   // the checkpoint holds no coefficient
   invalidate_mass(ctx);
   if (ok && h.has_coarse) {
     if (!ctx->d_Kell) CK(cudaMalloc(&ctx->d_Kell, sizeof(double) * nk));

@@ -744,17 +744,19 @@ k_patch_finish(const int *__restrict__ patch_ids, int n_work, const double *__re
 }
 
 // ------------------------------------------------------------------------------------------------
-// k_coarse : K rows of one patch in block-ELL form
+// k_coarse : K rows of one patch in block-ELL form.  patch_list == nullptr: the patches [patch_begin, patch_end);
+// else the patches patch_list[patch_begin .. patch_end)
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
-k_coarse(int patch_begin, int patch_end, const double *__restrict__ phi, const double *__restrict__ aphi,
-         double *__restrict__ Kell, FinishLayout lay) {
+k_coarse(int patch_begin, int patch_end, const int *__restrict__ patch_list, const double *__restrict__ phi,
+         const double *__restrict__ aphi, double *__restrict__ Kell, FinishLayout lay) {
   extern __shared__ double smem[];
   double *sPhi = smem;  // [s][Nf]
   const int tid = threadIdx.x, NT = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarp = NT >> 5;
   const int s = cP.s, n = cP.n, w = cP.w, ww = 2 * w + 1;
   const int nslots = (cP.dim == 3) ? ww * ww * ww : ww * ww;
-  for (int pid = patch_begin + blockIdx.x; pid < patch_end; pid += gridDim.x) {
+  for (int it = patch_begin + blockIdx.x; it < patch_end; it += gridDim.x) {
+    const int pid = patch_list ? patch_list[it] : it;
     const Geom g = make_geom(cP, pid);
     __syncthreads();
     for (int i = tid; i < s * lay.nf_max; i += NT) sPhi[i] = phi[(size_t)pid * s * lay.nf_max + i];
@@ -812,12 +814,16 @@ k_coarse(int patch_begin, int patch_end, const double *__restrict__ phi, const d
 // The basis functions of the group are staged in shared memory on the group's common node box (zero outside
 // each member's own box), so every A*phi value of a neighbour is loaded once per group and multiplied with all
 // members' phi at the same shared-memory offset: no per-pair index arithmetic, 2^dim times less L2 traffic.
+// LIST = false: the groups that meet [patch_begin, patch_end); true: the n_groups groups of group_list (every member's
+// rows are written, [patch_begin, patch_end) must then cover all patches).  Two instantiations keep the code of the
+// range path as it was.
 // ------------------------------------------------------------------------------------------------
 constexpr int kCoarseThreads = 512;
-template <int DIM, int S>
+template <int DIM, int S, bool LIST>
 __global__ void __launch_bounds__(kCoarseThreads, 1)
-k_coarse_blocked(int patch_begin, int patch_end, const double *__restrict__ phi, const double *__restrict__ aphi,
-                 double *__restrict__ Kell, FinishLayout lay, int NU) {
+k_coarse_blocked(int patch_begin, int patch_end, const int *__restrict__ group_list, int n_groups,
+                 const double *__restrict__ phi, const double *__restrict__ aphi, double *__restrict__ Kell,
+                 FinishLayout lay, int NU) {
   constexpr int NG = 1 << DIM;   // patches per group
   constexpr int NA = NG * S;     // accumulators per lane and neighbour: (member, component d)
   constexpr int NQ = 4;          // neighbours (adjacent in x) per warp pass (3: no spills but 8.3 instead of 7.7 ms)
@@ -828,8 +834,9 @@ k_coarse_blocked(int patch_begin, int patch_end, const double *__restrict__ phi,
   __shared__ int sUlo[3], sUhi[3];
   const int tid = threadIdx.x, NT = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarp = NT >> 5;
   const int n = cP.n, w = cP.w, ww = 2 * w + 1;
-  const int g0 = patch_begin >> DIM, g1 = ((patch_end - 1) >> DIM) + 1;
-  for (int grp = g0 + blockIdx.x; grp < g1; grp += gridDim.x) {
+  const int g0 = LIST ? 0 : patch_begin >> DIM, g1 = LIST ? n_groups : ((patch_end - 1) >> DIM) + 1;
+  for (int it = g0 + blockIdx.x; it < g1; it += gridDim.x) {
+    const int grp = LIST ? group_list[it] : it;
     __syncthreads();
     if (tid < NG) {
       const int pid = grp * NG + tid;
@@ -978,13 +985,21 @@ k_coarse_blocked(int patch_begin, int patch_end, const double *__restrict__ phi,
 }
 template <int DIM, int S>
 static cudaError_t launch_coarse_blocked_t(int grid, size_t smem, cudaStream_t st, int p0, int p1, const double *phi,
-                                           const double *aphi, double *Kell, const FinishLayout &lay, int NU) {
-  cudaError_t e = cudaFuncSetAttribute(k_coarse_blocked<DIM, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                                           const double *aphi, double *Kell, const FinishLayout &lay, int NU,
+                                           const int *groups, int n_groups) {
+  // a group list rewrites rows of a matrix that was assembled before: the slots the kernel never visits (neighbours
+  // outside the domain) are zero already, they depend on the geometry alone.  A range clears its rows first.
+  if (groups) {
+    cudaError_t e = cudaFuncSetAttribute(k_coarse_blocked<DIM, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    k_coarse_blocked<DIM, S, true><<<grid, kCoarseThreads, smem, st>>>(p0, p1, groups, n_groups, phi, aphi, Kell, lay, NU);
+    return cudaGetLastError();
+  }
+  cudaError_t e = cudaFuncSetAttribute(k_coarse_blocked<DIM, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  // slots of neighbours outside the domain are never visited: clear the rows first
   e = cudaMemsetAsync(Kell + (size_t)p0 * S * (lay.ell_width), 0, sizeof(double) * (size_t)(p1 - p0) * S * lay.ell_width, st);
   if (e != cudaSuccess) return e;
-  k_coarse_blocked<DIM, S><<<grid, kCoarseThreads, smem, st>>>(p0, p1, phi, aphi, Kell, lay, NU);
+  k_coarse_blocked<DIM, S, false><<<grid, kCoarseThreads, smem, st>>>(p0, p1, nullptr, 0, phi, aphi, Kell, lay, NU);
   return cudaGetLastError();
 }
 size_t coarse_blocked_smem(int dim, int s, int NU) {
@@ -992,10 +1007,11 @@ size_t coarse_blocked_smem(int dim, int s, int NU) {
   return sizeof(double) * ((size_t)(1 << dim) * s * nuv * s);
 }
 cudaError_t launch_coarse_blocked(int dim, int s, int grid, size_t smem, cudaStream_t st, int p0, int p1,
-                                  const double *phi, const double *aphi, double *Kell, const FinishLayout &lay, int NU) {
-  if (dim == 3 && s == 1) return launch_coarse_blocked_t<3, 1>(grid, smem, st, p0, p1, phi, aphi, Kell, lay, NU);
-  if (dim == 2 && s == 1) return launch_coarse_blocked_t<2, 1>(grid, smem, st, p0, p1, phi, aphi, Kell, lay, NU);
-  if (dim == 2 && s == 2) return launch_coarse_blocked_t<2, 2>(grid, smem, st, p0, p1, phi, aphi, Kell, lay, NU);
+                                  const double *phi, const double *aphi, double *Kell, const FinishLayout &lay, int NU,
+                                  const int *groups, int n_groups) {
+  if (dim == 3 && s == 1) return launch_coarse_blocked_t<3, 1>(grid, smem, st, p0, p1, phi, aphi, Kell, lay, NU, groups, n_groups);
+  if (dim == 2 && s == 1) return launch_coarse_blocked_t<2, 1>(grid, smem, st, p0, p1, phi, aphi, Kell, lay, NU, groups, n_groups);
+  if (dim == 2 && s == 2) return launch_coarse_blocked_t<2, 2>(grid, smem, st, p0, p1, phi, aphi, Kell, lay, NU, groups, n_groups);
   return cudaErrorInvalidValue;
 }
 
@@ -1202,6 +1218,8 @@ cudaError_t launch_gather(cudaStream_t st, const double *src, const long long *p
   k_gather<<<148 * 8, 256, 0, st>>>(src, perm, dst, n);
   return cudaGetLastError();
 }
+
+#include "update.cuh"
 }  // namespace slod
 #include "online.cuh"
 #include "online_batch.cuh"
@@ -1449,10 +1467,10 @@ cudaError_t launch_fine_norms_reference(cudaStream_t st, long long n_cells, int 
 }
 
 cudaError_t launch_coarse(int grid, size_t smem, cudaStream_t st, int p0, int p1, const double *phi, const double *aphi,
-                          double *Kell, const FinishLayout &lay) {
+                          double *Kell, const FinishLayout &lay, const int *patches) {
   cudaError_t e = cudaFuncSetAttribute(k_coarse, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  k_coarse<<<grid, 256, smem, st>>>(p0, p1, phi, aphi, Kell, lay);
+  k_coarse<<<grid, 256, smem, st>>>(p0, p1, patches, phi, aphi, Kell, lay);
   return cudaGetLastError();
 }
 

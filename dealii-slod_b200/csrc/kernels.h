@@ -122,11 +122,18 @@ cudaError_t launch_select_pipeline(const SelectPlan &pl, cudaStream_t st, const 
 cudaError_t launch_patch_finish(int grid, size_t smem, cudaStream_t st, const int *ids, int n_work, const double *coef,
                                 const double *X, const double *cvec, double *phi, double *aphi,
                                 const FinishLayout &lay);
-// blocked coarse-matrix kernel: one CTA per Morton-aligned group of 2^dim patches, NU = nodes per axis of the common box
+// blocked coarse-matrix kernel: one CTA per Morton-aligned group of 2^dim patches, NU = nodes per axis of the common box.
+// groups != nullptr: only the n_groups groups listed (group = patch id >> dim), every row of each; [p0, p1) must then be
+// all patches.  The rows of an assembled matrix are rewritten in place.
 size_t coarse_blocked_smem(int dim, int s, int NU);
 cudaError_t launch_coarse_blocked(int dim, int s, int grid, size_t smem, cudaStream_t st, int p0, int p1,
-                                  const double *phi, const double *aphi, double *Kell, const FinishLayout &lay, int NU);
+                                  const double *phi, const double *aphi, double *Kell, const FinishLayout &lay, int NU,
+                                  const int *groups = nullptr, int n_groups = 0);
 cudaError_t launch_gather(cudaStream_t st, const double *src, const long long *perm, double *dst, long long n);
+// incremental update (update.cuh): cell_changed[N^dim] = 1 where a value of the coarse cell's sub-cells differs bitwise
+// between the two device coefficient arrays (n doubles each, nq values per sub-cell, n_sub sub-cells per cell and axis)
+cudaError_t launch_coef_diff(cudaStream_t st, const double *base, const double *cur, long long n, int dim, int N,
+                             int n_sub, int nq, unsigned char *cell_changed);
 // online phase (online.cuh): b = C^T f, CG on the block-ELL coarse matrix, u_h = C u
 cudaError_t launch_coarse_rhs(cudaStream_t st, int n_patches, int s, const double *phi, const double *f, double *b,
                               int nf_max);
@@ -182,7 +189,8 @@ cudaError_t launch_fine_quadratic_form(cudaStream_t st, int op, long long n_node
 cudaError_t launch_fine_norms_reference(cudaStream_t st, long long n_cells, int nq, const double *gauss_x,
                                         const double *gauss_w, const double *v, double *partial, int *n_blocks);
 cudaError_t run_fp64_probe(int n_sm, double *dfma_tflops, double *dmma_tflops);
+// patches != nullptr: the patches patches[p0 .. p1) instead of the range [p0, p1)
 cudaError_t launch_coarse(int grid, size_t smem, cudaStream_t st, int p0, int p1, const double *phi, const double *aphi,
-                          double *Kell, const FinishLayout &lay);
+                          double *Kell, const FinishLayout &lay, const int *patches = nullptr);
 
 }  // namespace slod

@@ -146,6 +146,31 @@ int slod_assemble_coarse(slod_ctx *ctx);
  * the sparse product are kept).  Call with rowptr == NULL to query n_rows and nnz. */
 int slod_get_coarse_csr(const slod_ctx *ctx, int64_t *rowptr, int64_t *col, double *val, int64_t *n_rows,
                         int64_t *nnz);
+/* Bring the basis (and the coarse matrix, if it was assembled) up to date with the coefficient tables set since the
+ * last successful slod_compute_basis / slod_update_basis, recomputing only what the change reaches (an extension: the
+ * reference recomputes everything).
+ * Baseline: the device coefficient array (the tables expanded onto the sub-cells or Gauss points) that the last
+ * successful slod_compute_basis or slod_update_basis of this single-device handle read.  Calls that only use the
+ * coefficient (slod_fem_solve, slod_fine_norms*, slod_fem_heat_solve) leave it alone.
+ * A patch is recomputed iff a value of its coefficient window (the coarse cells of its box; under quirk_presaved, the
+ * donor's box for a full-size patch) differs bitwise from the baseline -- any field, sub-cell or Gauss point; 0.0 ->
+ * -0.0 counts, a table cell no Gauss point samples does not.  If the array's layout changed (its length, or one value
+ * per Gauss point instead of per sub-cell or back), every patch is recomputed.
+ * If slod_assemble_coarse ran on the basis being updated, the block-ELL rows of every patch whose own or a structural
+ * neighbour's basis changed are recomputed (on the blocked kernel: whole Morton groups of 2^dim patches) and the CSR
+ * values refreshed; like slod_assemble_coarse the call may return with those kernels enqueued only.  Otherwise K stays
+ * unassembled.
+ * Afterwards slod_get_all_basis, slod_get_patch_diagnostics and slod_get_coarse_csr (and the block-ELL rows) are
+ * bit-identical to what a fresh handle computes from the same tables with slod_compute_basis (+ slod_assemble_coarse).
+ * slod_get_timings [0]..[4] report the update's stages (0 where nothing ran).  If nothing differs, only the comparison
+ * kernel runs and both counts are 0.  If any patch is recomputed, M_H is stale as after slod_compute_basis.
+ * n_patches_recomputed / n_row_blocks_recomputed (may be NULL): patches and K row blocks (spacedim rows each) recomputed.
+ * Errors: no baseline (no basis yet, a basis restored by slod_load_state or computed through the device-buffer
+ * entry points, the last compute failed) -> SLOD_ERR_STATE; an n_gpus > 1 handle -> SLOD_ERR_UNSUPPORTED; a recomputed
+ * patch with a numerical status -> SLOD_ERR_NUMERIC naming the first one, as slod_compute_basis would, and the handle
+ * has no basis and no baseline until the next successful slod_compute_basis. */
+int slod_update_basis(slod_ctx *ctx, int64_t *n_patches_recomputed /* may be NULL */,
+                      int64_t *n_row_blocks_recomputed /* may be NULL */);
 
 /* ---- online phase on the handle's basis and coarse matrix (SURVEY 8f row 1; replaces LOD::solve(),
  * source/LOD.cc:975-1001, and the prolongation in LOD::compare_lod_with_fem(), source/LOD.cc:1251).
