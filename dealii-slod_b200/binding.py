@@ -32,7 +32,7 @@ EXPORTS = [
     "slod_fine_norms_reference", "slod_set_host_outputs", "slod_coarse_rhs_batch", "slod_coarse_solve_batch",
     "slod_prolongate_batch", "slod_assemble_coarse_mass", "slod_get_coarse_mass_csr", "slod_l2_project_batch",
     "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan", "slod_debug_select",
-    "slod_update_basis",
+    "slod_update_basis", "slod_heat_theta_solve", "slod_heat_theta_solve_batch", "slod_fem_heat_theta_solve",
 ]
 # slod_get_plan entries, in order
 PLAN_KEYS = ["mma_variant", "split_solver", "dense_ntile", "gmem_window", "dense_coef_gmem", "coarse_blocked", "use_ql",
@@ -90,6 +90,10 @@ def load_library(path=None):
     lib.slod_heat_solve.argtypes = [vp, P(dbl), P(dbl), dbl, i32, i32, P(dbl), i32, dbl, dbl, P(i32)]
     lib.slod_heat_solve_batch.argtypes = [vp, i32, P(dbl), P(dbl), dbl, i32, i32, P(dbl), i32, dbl, dbl, P(i32)]
     lib.slod_fem_heat_solve.argtypes = [vp, P(dbl), P(dbl), dbl, i32, i32, P(dbl), i32, dbl, dbl, P(i32)]
+    theta = [dbl, dbl, i32, i32, i32, i32, P(dbl), P(dbl), P(dbl), P(dbl), i32, dbl, dbl, P(i32)]
+    lib.slod_heat_theta_solve.argtypes = [vp] + theta
+    lib.slod_heat_theta_solve_batch.argtypes = [vp, i32] + theta
+    lib.slod_fem_heat_theta_solve.argtypes = [vp] + theta
     lib.slod_fine_norms.argtypes = [vp, P(dbl), P(dbl), P(dbl), P(dbl)]
     lib.slod_get_patch_info.argtypes = [vp, i64] + [P(i32)] * 6 + [P(i32), P(i32)]
     lib.slod_get_patch_cells.argtypes = [vp, i64, P(C.c_uint32), P(i32)]
@@ -471,6 +475,69 @@ class SlodContext:
         self._ck(self.lib.slod_fem_heat_solve(self.h, None if f is None else _dp(f), None if u0 is None else _dp(u0),
                                               dt, n_steps, out_every, _dp(out), max_steps, tolerance, reduction,
                                               steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out, steps
+
+    # -- theta scheme with forcing sum_q g_q(t) f_q(x) (slod_heat_theta_solve / _batch, slod_fem_heat_theta_solve) --
+    def _fields(self, F, G, n_steps, lead, n):
+        """F (*lead, n_fields, n) or None, G (*lead, n_steps + 1, n_fields) or None -> (F, G, n_fields) as C arrays."""
+        if F is None:
+            return None, None, 1
+        F = np.ascontiguousarray(F, dtype=np.float64)
+        if F.ndim != len(lead) + 2 or F.shape[:len(lead)] != lead or F.shape[-1] != n or F.shape[-2] < 1:
+            raise ValueError(f"fields must have shape {lead + ('n_fields', n)}, got {F.shape}")
+        nq = F.shape[-2]
+        if G is not None:
+            G = np.ascontiguousarray(G, dtype=np.float64)
+            if G.shape != lead + (n_steps + 1, nq):
+                raise ValueError(f"g must have shape {lead + (n_steps + 1, nq)}, got {G.shape}")
+        return F, G, nq
+
+    def heat_theta_solve(self, f_fields, g, u0_coarse, theta, dt, n_steps, out_every=1, n_startup=0, max_steps=10000,
+                         tolerance=0.0, reduction=1e-12):
+        """The theta scheme on the SLOD space: f_fields (n_fields, n_fine) or None, g (n_steps + 1, n_fields) or None
+        (g = 1), u0_coarse or None.  Returns (U (n_steps // out_every, n_coarse), cg_steps int32[n_steps])."""
+        nc = self.n_patches * self.s
+        f, gg, nq = self._fields(f_fields, g, n_steps, (), self.n_fine)
+        u0 = self._vec_or_none(u0_coarse, nc, "coarse vector")
+        out = np.empty((max(n_steps // max(out_every, 1), 1), nc))
+        steps = np.zeros(max(n_steps, 1), dtype=np.int32)
+        self._ck(self.lib.slod_heat_theta_solve(self.h, theta, dt, n_steps, out_every, n_startup, nq,
+                                                None if f is None else _dp(f), None if gg is None else _dp(gg),
+                                                None if u0 is None else _dp(u0), _dp(out), max_steps, tolerance,
+                                                reduction, steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out, steps
+
+    def heat_theta_solve_batch(self, F, G, U0, theta, dt, n_steps, out_every=1, n_startup=0, max_steps=10000,
+                               tolerance=0.0, reduction=1e-12):
+        """k trajectories at once: F (k, n_fields, n_fine), G (k, n_steps + 1, n_fields), U0 (k, n_coarse) (each may be
+        None).  Returns (U (n_steps // out_every, k, n_coarse), cg_steps int32 (n_steps, k))."""
+        nc = self.n_patches * self.s
+        if F is None and U0 is None:
+            raise ValueError("give F or U0 (the number of trajectories)")
+        k = np.shape(F)[0] if F is not None else np.shape(U0)[0]
+        f, gg, nq = self._fields(F, G, n_steps, (k,), self.n_fine)
+        u0 = None if U0 is None else self._block(U0, nc, "coarse block")
+        if u0 is not None and u0.shape[0] != k:
+            raise ValueError("F and U0 must have the same number of rows")
+        out = np.empty((max(n_steps // max(out_every, 1), 1), k, nc))
+        steps = np.zeros((max(n_steps, 1), k), dtype=np.int32)
+        self._ck(self.lib.slod_heat_theta_solve_batch(self.h, k, theta, dt, n_steps, out_every, n_startup, nq,
+                                                      None if f is None else _dp(f), None if gg is None else _dp(gg),
+                                                      None if u0 is None else _dp(u0), _dp(out), max_steps, tolerance,
+                                                      reduction, steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out, steps
+
+    def fem_heat_theta_solve(self, f_fields, g, u0_fine, theta, dt, n_steps, out_every=1, n_startup=0,
+                             max_steps=200000, tolerance=0.0, reduction=1e-12):
+        """The fine-scale reference of heat_theta_solve.  Returns (U (n_steps // out_every, n_fine), cg_steps)."""
+        f, gg, nq = self._fields(f_fields, g, n_steps, (), self.n_fine)
+        u0 = self._vec_or_none(u0_fine, self.n_fine, "fine vector")
+        out = np.empty((max(n_steps // max(out_every, 1), 1), self.n_fine))
+        steps = np.zeros(max(n_steps, 1), dtype=np.int32)
+        self._ck(self.lib.slod_fem_heat_theta_solve(self.h, theta, dt, n_steps, out_every, n_startup, nq,
+                                                    None if f is None else _dp(f), None if gg is None else _dp(gg),
+                                                    None if u0 is None else _dp(u0), _dp(out), max_steps, tolerance,
+                                                    reduction, steps.ctypes.data_as(C.POINTER(C.c_int32))))
         return out, steps
 
     # -- fine-scale reference problem (assemble_and_solve_fem_problem, source/LOD.cc:1004-1094) and norms (:1252) --

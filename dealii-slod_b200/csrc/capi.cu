@@ -107,11 +107,11 @@ struct slod_ctx {
   size_t batch_doubles = 0;
   double *d_val = nullptr;
   int64_t csr_nnz = 0;
-  // heat equation on the SLOD space: M_H in block-ELL form and its CSR values, S = M_H + dt K for the dt of the last
-  // time-stepping call (s_dt == 0: not formed), and the scratch of the time steppers
+  // heat equation on the SLOD space: M_H in block-ELL form and its CSR values, S = M_H + c K for the coefficient c of K
+  // last formed (s_coef == 0: not formed), and the scratch of the time steppers
   double *d_Mell = nullptr, *d_Mval = nullptr, *d_Sell = nullptr;
   bool mass_done = false;
-  double s_dt = 0.0;
+  double s_coef = 0.0;
   double *d_heat = nullptr;
   size_t heat_doubles = 0;
   // multi-GPU: (a) n_gpus > 1: this handle is rank 0 and owns one sub-handle per further device; (b) slod_comm_init
@@ -409,7 +409,7 @@ void patch_cells_rel(const Params &P, const Geom &g, std::vector<std::array<int,
 // M_H and S are derived from the basis and from K: a new basis, a restored checkpoint or a new K make them stale
 void invalidate_mass(slod_ctx *c) {
   c->mass_done = false;
-  c->s_dt = 0.0;
+  c->s_coef = 0.0;
 }
 
 int check_patch(const slod_ctx *ctx, int64_t patch) {
@@ -2324,7 +2324,7 @@ static int heat_scratch(slod_ctx *ctx, size_t doubles, double **out) {
   return SLOD_OK;
 }
 
-// the common preconditions of the two coarse time steppers, and S = M_H + dt K (kept until dt changes)
+// the common preconditions of the two coarse time steppers
 static int heat_prepare(slod_ctx *ctx, double dt, int32_t n_steps, int32_t out_every, const double *u_out,
                         int32_t max_steps, double tolerance, double reduction) {
   if (!ctx->coarse_done) return fail(ctx, SLOD_ERR_STATE, "slod_assemble_coarse has not run");
@@ -2332,26 +2332,73 @@ static int heat_prepare(slod_ctx *ctx, double dt, int32_t n_steps, int32_t out_e
   if (!u_out) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
   int rc = check_time_steps(ctx, dt, n_steps, out_every);
   if (rc) return rc;
-  rc = check_solver_control(ctx, max_steps, tolerance, reduction);
-  if (rc) return rc;
-  if (ctx->s_dt == dt) return SLOD_OK;
+  return check_solver_control(ctx, max_steps, tolerance, reduction);
+}
+
+// S = M_H + coef K, kept until the coefficient of K changes (or M_H / K become stale)
+static cudaError_t heat_form_S(slod_ctx *ctx, double coef, long long *launches) {
+  if (ctx->s_coef == coef) return cudaSuccess;
   const size_t nk = (size_t)ctx->n_patches * ctx->P.s * ctx->P.ell_width;
-  if (!ctx->d_Sell) CK(cudaMalloc(&ctx->d_Sell, sizeof(double) * nk));
-  CK(launch_lincomb(0, (long long)nk, 1.0, ctx->d_Mell, dt, ctx->d_Kell, ctx->d_Sell));
-  ctx->launches += 1;
-  ctx->s_dt = dt;
+  cudaError_t e = ctx->d_Sell ? cudaSuccess : cudaMalloc(&ctx->d_Sell, sizeof(double) * nk);
+  if (e == cudaSuccess) e = launch_lincomb(0, (long long)nk, 1.0, ctx->d_Mell, coef, ctx->d_Kell, ctx->d_Sell);
+  *launches += 1;
+  ctx->s_coef = e == cudaSuccess ? coef : 0.0;
+  return e;
+}
+
+// The theta-scheme arguments (slod.h); g_count: the entries of g.  g is read only when fields are given.
+static int check_theta(slod_ctx *ctx, double theta, int32_t n_steps, int32_t n_startup, int32_t n_fields,
+                       const double *f, const double *g, size_t g_count) {
+  if (!(theta >= 0.5 && theta <= 1.0)) return fail(ctx, SLOD_ERR_INVALID, "theta must be in [1/2, 1]");
+  if (n_startup < 0 || n_startup > n_steps) return fail(ctx, SLOD_ERR_INVALID, "n_startup must be in [0, n_steps]");
+  if (f && n_fields < 1) return fail(ctx, SLOD_ERR_INVALID, "n_fields must be at least 1");
+  if (f && g)
+    for (size_t i = 0; i < g_count; ++i)
+      if (!std::isfinite(g[i])) return fail(ctx, SLOD_ERR_INVALID, "g has a non-finite entry");
   return SLOD_OK;
 }
 
-static int heat_cg_failure(slod_ctx *ctx, int step, int column, int flag, int steps, double res) {
-  char buf[240];
+// One solve of the time loop: S = M_H + coef K, r = tau (sum_q w_q b_q - K u), S delta = r, u += delta.  A full step k
+// of the theta scheme is one stage (coef = theta dt, tau = dt, w_q = theta g_q(t_k) + (1 - theta) g_q(t_{k-1})); a
+// Rannacher start-up step is two backward-Euler stages of dt / 2 (w_q = (g_q(t_{k-1}) + g_q(t_k)) / 2, then g_q(t_k)).
+// At theta = 1 without start-up coef = tau = dt and w_q = g_q(t_k) exactly: the backward-Euler entry points.
+struct ThetaStage {
+  int step;         // the time step k = 1 .. n_steps the stage belongs to
+  bool ends_step;   // u is u^k after this stage
+  double tau, coef;
+};
+static std::vector<ThetaStage> theta_stages(double theta, double dt, int n_steps, int n_startup) {
+  std::vector<ThetaStage> st;
+  for (int k = 1; k <= n_steps; ++k) {
+    if (k <= n_startup) {
+      st.push_back({k, false, 0.5 * dt, 0.5 * dt});
+      st.push_back({k, true, 0.5 * dt, 0.5 * dt});
+    } else {
+      st.push_back({k, true, dt, theta * dt});
+    }
+  }
+  return st;
+}
+// the weights of every stage of one column, w[stage][nf]; g [n_steps + 1][nf] or NULL (g = 1)
+static void theta_weights(double theta, int n_steps, int n_startup, int nf, const double *g, double *w) {
+  auto G = [&](int k, int q) { return g ? g[(size_t)k * nf + q] : 1.0; };
+  for (int k = 1; k <= n_steps; ++k)
+    for (int half = (k <= n_startup ? 0 : 1); half < 2; ++half, w += nf)
+      for (int q = 0; q < nf; ++q)
+        w[q] = k <= n_startup ? (half ? G(k, q) : 0.5 * (G(k - 1, q) + G(k, q)))
+                              : theta * G(k, q) + (1.0 - theta) * G(k - 1, q);
+}
+
+// coef: the coefficient c of K in the matrix M_H + c K of the failing solve (theta dt, or dt / 2 in a start-up step)
+static int heat_cg_failure(slod_ctx *ctx, int step, int column, double coef, int flag, int steps, double res) {
+  char buf[260];
   const std::string col = column >= 0 ? " column " + std::to_string(column) : std::string();
   if (flag == 2)
-    std::snprintf(buf, sizeof buf, "time step %d%s: CG on M_H + dt K broke down after %d steps (residual %.3e): the "
-                  "matrix is not positive definite", step, col.c_str(), steps, res);
+    std::snprintf(buf, sizeof buf, "time step %d%s: CG on M_H + c K (c = %.6g) broke down after %d steps (residual "
+                  "%.3e): the matrix is not positive definite", step, col.c_str(), coef, steps, res);
   else
-    std::snprintf(buf, sizeof buf, "time step %d%s: CG on M_H + dt K did not converge: %d steps, residual %.3e", step,
-                  col.c_str(), steps, res);
+    std::snprintf(buf, sizeof buf, "time step %d%s: CG on M_H + c K (c = %.6g) did not converge: %d steps, residual "
+                  "%.3e", step, col.c_str(), coef, steps, res);
   return fail(ctx, SLOD_ERR_NUMERIC, buf);
 }
 
@@ -2414,11 +2461,11 @@ int slod_l2_project_batch(slod_ctx *ctx, int32_t n_rhs, const double *v_fine, do
   return SLOD_OK;
 }
 
-int slod_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_coarse, double dt, int32_t n_steps,
-                    int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
-                    int32_t *cg_steps) {
-  if (!ctx) return SLOD_ERR_INVALID;
-  NEED_DEVICE();
+// the single-trajectory theta scheme: slod_heat_theta_solve after its argument checks, and slod_heat_solve (theta = 1)
+static int heat_theta_single(slod_ctx *ctx, const char *name, double theta, double dt, int32_t n_steps,
+                             int32_t out_every, int32_t n_startup, int32_t n_fields, const double *f_fine,
+                             const double *g, const double *u0_coarse, double *u_out, int32_t max_steps,
+                             double tolerance, double reduction, int32_t *cg_steps) {
   CK(cudaSetDevice(ctx->device));
   BIND_PARAMS((cudaStream_t)0);
   int rc = heat_prepare(ctx, dt, n_steps, out_every, u_out, max_steps, tolerance, reduction);
@@ -2426,55 +2473,70 @@ int slod_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_coarse
   int64_t n_fine = 0;
   slod_fine_size(ctx, &n_fine);
   const int nrows = (int)(ctx->n_patches * ctx->P.s);
+  const int nf = f_fine ? n_fields : 1;   // no forcing: one zero load
+  const std::vector<ThetaStage> stages = theta_stages(theta, dt, n_steps, n_startup);
+  std::vector<double> w(stages.size() * nf);
+  theta_weights(theta, n_steps, n_startup, nf, f_fine ? g : nullptr, w.data());
   double *d_f = nullptr, *d_r = nullptr, *d_delta = nullptr, *d_work = nullptr, *d_u = nullptr;
   rc = online_scratch(ctx, &d_f, nullptr, &d_r, &d_delta, &d_work);
   if (rc) return rc;
-  rc = heat_scratch(ctx, 2 * (size_t)nrows, &d_u);
+  rc = heat_scratch(ctx, (1 + (size_t)nf) * nrows + w.size(), &d_u);   // u | b_0 .. b_{nf-1} | weights
   if (rc) return rc;
-  double *d_b = d_u + nrows;
-  cudaError_t e = cudaSuccess;
+  double *d_b = d_u + nrows, *d_w = d_b + (size_t)nf * nrows;
+  cudaError_t e = cudaMemcpyAsync(d_w, w.data(), sizeof(double) * w.size(), cudaMemcpyHostToDevice, 0);
   if (f_fine) {
-    e = cudaMemcpyAsync(d_f, f_fine, sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
-    if (e == cudaSuccess) e = launch_coarse_rhs(0, (int)ctx->n_patches, ctx->P.s, ctx->d_phi, d_f, d_b, ctx->P.NfMax);
-    ctx->launches += 1;
-  } else {
+    for (int q = 0; q < nf && e == cudaSuccess; ++q) {   // C^T f_q, one field at a time through the fine scratch
+      e = cudaMemcpyAsync(d_f, f_fine + (size_t)q * n_fine, sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+      if (e == cudaSuccess)
+        e = launch_coarse_rhs(0, (int)ctx->n_patches, ctx->P.s, ctx->d_phi, d_f, d_b + (size_t)q * nrows,
+                              ctx->P.NfMax);
+      ctx->launches += 1;
+    }
+  } else if (e == cudaSuccess) {
     e = cudaMemsetAsync(d_b, 0, sizeof(double) * nrows, 0);
   }
   if (e == cudaSuccess)
     e = u0_coarse ? cudaMemcpyAsync(d_u, u0_coarse, sizeof(double) * nrows, cudaMemcpyHostToDevice, 0)
                   : cudaMemsetAsync(d_u, 0, sizeof(double) * nrows, 0);
-  const CgOperator S{ctx->d_Sell, nullptr, 0};
   long long n_launch = 0;
-  int failed_step = 0, flag = 0, st_steps = 0;
-  double res = 0.0;
-  for (int k = 1; k <= n_steps && e == cudaSuccess; ++k) {
-    e = launch_ell_residual(0, nrows, 1, ctx->d_Kell, d_u, d_b, dt, d_r);
+  int failed_step = 0, flag = 0, st_steps = 0, step_cg = 0;
+  double res = 0.0, failed_coef = 0.0;
+  for (size_t i = 0; i < stages.size() && e == cudaSuccess; ++i) {
+    const ThetaStage &sg = stages[i];
+    const int k = sg.step;
+    e = heat_form_S(ctx, sg.coef, &n_launch);
+    if (e == cudaSuccess)
+      e = launch_ell_residual(0, nrows, 1, ctx->d_Kell, d_u, nf, d_b, nrows, d_w + i * nf, sg.tau, d_r);
+    const CgOperator S{ctx->d_Sell, nullptr, 0};   // after heat_form_S: the first call allocates d_Sell
     if (e == cudaSuccess)
       e = run_cg(0, nrows, S, d_r, d_delta, d_work, max_steps, tolerance, reduction, &st_steps, &res, &flag, &n_launch);
     if (e != cudaSuccess) break;
-    if (cg_steps) cg_steps[k - 1] = st_steps;
+    step_cg = (i > 0 && stages[i - 1].step == k ? step_cg : 0) + st_steps;
+    if (cg_steps) cg_steps[k - 1] = step_cg;
     if (flag != 1) {
       failed_step = k;
+      failed_coef = sg.coef;
       break;
     }
     e = launch_lincomb(0, nrows, 1.0, d_u, 1.0, d_delta, d_u);
-    if (e == cudaSuccess && k % out_every == 0)
+    if (e == cudaSuccess && sg.ends_step && k % out_every == 0)
       e = cudaMemcpyAsync(u_out + (size_t)(k / out_every - 1) * nrows, d_u, sizeof(double) * nrows,
                           cudaMemcpyDeviceToHost, 0);
     n_launch += 2;
   }
   if (e == cudaSuccess) e = cudaStreamSynchronize(0);
   ctx->launches += n_launch;
-  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_heat_solve: ") + cudaGetErrorString(e));
-  if (failed_step) return heat_cg_failure(ctx, failed_step, -1, flag, st_steps, res);
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string(name) + ": " + cudaGetErrorString(e));
+  if (failed_step) return heat_cg_failure(ctx, failed_step, -1, failed_coef, flag, st_steps, res);
   return SLOD_OK;
 }
 
-int slod_heat_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, const double *u0_coarse, double dt,
-                          int32_t n_steps, int32_t out_every, double *u_out, int32_t max_steps, double tolerance,
-                          double reduction, int32_t *cg_steps) {
-  if (!ctx) return SLOD_ERR_INVALID;
-  NEED_DEVICE();
+// n_rhs trajectories in groups of kBatch interleaved columns: slod_heat_theta_solve_batch after its argument checks,
+// and slod_heat_solve_batch (theta = 1)
+static int heat_theta_batch(slod_ctx *ctx, const char *name, int32_t n_rhs, double theta, double dt, int32_t n_steps,
+                            int32_t out_every, int32_t n_startup, int32_t n_fields, const double *f_fine,
+                            const double *g, const double *u0_coarse, double *u_out, int32_t max_steps,
+                            double tolerance, double reduction, int32_t *cg_steps) {
   if (n_rhs < 1) return fail(ctx, SLOD_ERR_INVALID, "n_rhs must be at least 1");
   CK(cudaSetDevice(ctx->device));
   BIND_PARAMS((cudaStream_t)0);
@@ -2485,84 +2547,110 @@ int slod_heat_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, co
   const int nrows = (int)(ctx->n_patches * ctx->P.s);
   const int n_groups = (n_rhs + kBatch - 1) / kBatch;
   const size_t gsz = (size_t)kBatch * nrows;   // one interleaved group
-  BatchScratch w{};
-  rc = batch_scratch(ctx, &w);
+  const int nf = f_fine ? n_fields : 1;        // no forcing: one zero load
+  const std::vector<ThetaStage> stages = theta_stages(theta, dt, n_steps, n_startup);
+  const size_t ns = stages.size(), wg = ns * nf * kBatch;   // weights of one group: [stage][q][kb]
+  std::vector<double> w((size_t)n_groups * wg, 0.0), wj(ns * nf);
+  for (int j = 0; j < n_rhs; ++j) {
+    const double *gj = f_fine && g ? g + (size_t)j * ((size_t)n_steps + 1) * nf : nullptr;
+    theta_weights(theta, n_steps, n_startup, nf, gj, wj.data());
+    const int grp = j / kBatch, jj = j % kBatch, kb = std::min(kBatch, n_rhs - grp * kBatch);
+    for (size_t i = 0; i < ns * nf; ++i) w[grp * wg + i * kb + jj] = wj[i];
+  }
+  BatchScratch ws{};
+  rc = batch_scratch(ctx, &ws);
   if (rc) return rc;
-  double *d_U = nullptr;   // [group][nrows][kb] states, then the right-hand sides C^T f in the same layout
-  rc = heat_scratch(ctx, 2 * (size_t)n_groups * gsz, &d_U);
+  double *d_U = nullptr;   // [group][nrows][kb] states | loads C^T f_q, [q][group][nrows][kb] | weights [group][wg]
+  rc = heat_scratch(ctx, (1 + (size_t)nf) * n_groups * gsz + w.size(), &d_U);
   if (rc) return rc;
-  double *d_B = d_U + (size_t)n_groups * gsz;
-  cudaError_t e = cudaSuccess;
+  const size_t b_stride = (size_t)n_groups * gsz;
+  double *d_B = d_U + b_stride, *d_W = d_B + nf * b_stride;
+  cudaError_t e = cudaMemcpyAsync(d_W, w.data(), sizeof(double) * w.size(), cudaMemcpyHostToDevice, 0);
   long long n_launch = 0;
-  for (int g = 0; g < n_groups && e == cudaSuccess; ++g) {
-    const int j0 = g * kBatch, kb = std::min(kBatch, n_rhs - j0);
-    double *U = d_U + g * gsz, *B = d_B + g * gsz;
+  for (int grp = 0; grp < n_groups && e == cudaSuccess; ++grp) {
+    const int j0 = grp * kBatch, kb = std::min(kBatch, n_rhs - j0);
+    double *U = d_U + grp * gsz, *B = d_B + grp * gsz;
     if (f_fine) {
-      e = cudaMemcpyAsync(w.fine_stage, f_fine + (size_t)j0 * n_fine, sizeof(double) * kb * (size_t)n_fine,
-                          cudaMemcpyHostToDevice, 0);
-      if (e == cudaSuccess) e = launch_interleave(0, n_fine, kb, w.fine_stage, w.fine, true);
-      if (e == cudaSuccess)
-        e = launch_coarse_rhs_multi(0, (int)ctx->n_patches, ctx->P.s, kb, ctx->d_phi, w.fine, B, ctx->P.NfMax);
-      n_launch += 2;
-    } else {
+      for (int q = 0; q < nf && e == cudaSuccess; ++q) {
+        // field q of the group's columns, one copy per column: the host rows are nf n_fine doubles apart, which can
+        // exceed the largest pitch of a 2-D copy
+        for (int c = 0; c < kb && e == cudaSuccess; ++c)
+          e = cudaMemcpyAsync(ws.fine_stage + (size_t)c * n_fine, f_fine + ((size_t)(j0 + c) * nf + q) * n_fine,
+                              sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+        if (e == cudaSuccess) e = launch_interleave(0, n_fine, kb, ws.fine_stage, ws.fine, true);
+        if (e == cudaSuccess)
+          e = launch_coarse_rhs_multi(0, (int)ctx->n_patches, ctx->P.s, kb, ctx->d_phi, ws.fine, B + q * b_stride,
+                                      ctx->P.NfMax);
+        n_launch += 2;
+      }
+    } else if (e == cudaSuccess) {
       e = cudaMemsetAsync(B, 0, sizeof(double) * kb * (size_t)nrows, 0);
     }
     if (e == cudaSuccess && u0_coarse) {
-      e = cudaMemcpyAsync(w.coarse_stage, u0_coarse + (size_t)j0 * nrows, sizeof(double) * kb * (size_t)nrows,
+      e = cudaMemcpyAsync(ws.coarse_stage, u0_coarse + (size_t)j0 * nrows, sizeof(double) * kb * (size_t)nrows,
                           cudaMemcpyHostToDevice, 0);
-      if (e == cudaSuccess) e = launch_interleave(0, nrows, kb, w.coarse_stage, U, true);
+      if (e == cudaSuccess) e = launch_interleave(0, nrows, kb, ws.coarse_stage, U, true);
       n_launch += 1;
     } else if (e == cudaSuccess) {
       e = cudaMemsetAsync(U, 0, sizeof(double) * kb * (size_t)nrows, 0);
     }
   }
-  std::vector<int> st_steps(n_rhs, 0), flag(n_rhs, 0);
+  std::vector<int> st_steps(n_rhs, 0), flag(n_rhs, 0), step_cg(n_rhs, 0);
   std::vector<double> res(n_rhs, 0.0);
   int failed_step = 0, failed_col = -1;
-  for (int k = 1; k <= n_steps && e == cudaSuccess && !failed_step; ++k) {
-    for (int g = 0; g < n_groups && e == cudaSuccess; ++g) {
-      const int j0 = g * kBatch, kb = std::min(kBatch, n_rhs - j0);
-      double *U = d_U + g * gsz, *B = d_B + g * gsz;
-      e = launch_ell_residual(0, nrows, kb, ctx->d_Kell, U, B, dt, w.coarse_a);
+  double failed_coef = 0.0;
+  for (size_t i = 0; i < ns && e == cudaSuccess && !failed_step; ++i) {
+    const ThetaStage &sg = stages[i];
+    const int k = sg.step;
+    const bool first = i == 0 || stages[i - 1].step != k;
+    e = heat_form_S(ctx, sg.coef, &n_launch);
+    for (int grp = 0; grp < n_groups && e == cudaSuccess; ++grp) {
+      const int j0 = grp * kBatch, kb = std::min(kBatch, n_rhs - j0);
+      double *U = d_U + grp * gsz, *B = d_B + grp * gsz;
+      e = launch_ell_residual(0, nrows, kb, ctx->d_Kell, U, nf, B, (long long)b_stride, d_W + grp * wg + i * nf * kb,
+                              sg.tau, ws.coarse_a);
       if (e == cudaSuccess)
-        e = run_cg_multi(0, nrows, ctx->d_Sell, kb, w.coarse_a, w.coarse_b, w.work, max_steps, tolerance, reduction,
+        e = run_cg_multi(0, nrows, ctx->d_Sell, kb, ws.coarse_a, ws.coarse_b, ws.work, max_steps, tolerance, reduction,
                          &st_steps[j0], &res[j0], &flag[j0], &n_launch);
       if (e != cudaSuccess) break;
-      for (int j = 0; j < kb; ++j) {
-        if (cg_steps) cg_steps[(size_t)(k - 1) * n_rhs + j0 + j] = st_steps[j0 + j];
-        if (flag[j0 + j] != 1 && !failed_step) {
+      for (int j = j0; j < j0 + kb; ++j) {
+        step_cg[j] = (first ? 0 : step_cg[j]) + st_steps[j];
+        if (cg_steps) cg_steps[(size_t)(k - 1) * n_rhs + j] = step_cg[j];
+        if (flag[j] != 1 && !failed_step) {
           failed_step = k;
-          failed_col = j0 + j;
+          failed_col = j;
+          failed_coef = sg.coef;
         }
       }
       if (failed_step) break;
-      e = launch_lincomb(0, (long long)kb * nrows, 1.0, U, 1.0, w.coarse_b, U);
+      e = launch_lincomb(0, (long long)kb * nrows, 1.0, U, 1.0, ws.coarse_b, U);
       n_launch += 2;
     }
-    if (e != cudaSuccess || failed_step || k % out_every != 0) continue;
-    for (int g = 0; g < n_groups && e == cudaSuccess; ++g) {
-      const int j0 = g * kBatch, kb = std::min(kBatch, n_rhs - j0);
-      e = launch_interleave(0, nrows, kb, d_U + g * gsz, w.coarse_stage, false);
+    if (e != cudaSuccess || failed_step || !sg.ends_step || k % out_every != 0) continue;
+    for (int grp = 0; grp < n_groups && e == cudaSuccess; ++grp) {
+      const int j0 = grp * kBatch, kb = std::min(kBatch, n_rhs - j0);
+      e = launch_interleave(0, nrows, kb, d_U + grp * gsz, ws.coarse_stage, false);
       if (e == cudaSuccess)
-        e = cudaMemcpyAsync(u_out + ((size_t)(k / out_every - 1) * n_rhs + j0) * nrows, w.coarse_stage,
+        e = cudaMemcpyAsync(u_out + ((size_t)(k / out_every - 1) * n_rhs + j0) * nrows, ws.coarse_stage,
                             sizeof(double) * kb * (size_t)nrows, cudaMemcpyDeviceToHost, 0);
       n_launch += 1;
     }
   }
   if (e == cudaSuccess) e = cudaStreamSynchronize(0);
   ctx->launches += n_launch;
-  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_heat_solve_batch: ") + cudaGetErrorString(e));
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string(name) + ": " + cudaGetErrorString(e));
   if (failed_step)
-    return heat_cg_failure(ctx, failed_step, failed_col, flag[failed_col], st_steps[failed_col], res[failed_col]);
+    return heat_cg_failure(ctx, failed_step, failed_col, failed_coef, flag[failed_col], st_steps[failed_col],
+                           res[failed_col]);
   return SLOD_OK;
 }
 
-// the fine-scale reference trajectory: the same scheme with M_h + dt A_h on the global grid (homogeneous Dirichlet rows)
-int slod_fem_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_fine, double dt, int32_t n_steps,
-                        int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
-                        int32_t *cg_steps) {
-  if (!ctx) return SLOD_ERR_INVALID;
-  NEED_DEVICE();
+// the fine-scale reference trajectory: the same scheme with M_h + coef A_h on the global grid (homogeneous Dirichlet
+// rows); slod_fem_heat_theta_solve after its argument checks, and slod_fem_heat_solve (theta = 1)
+static int fem_heat_theta(slod_ctx *ctx, const char *name, double theta, double dt, int32_t n_steps, int32_t out_every,
+                          int32_t n_startup, int32_t n_fields, const double *f_fine, const double *g,
+                          const double *u0_fine, double *u_out, int32_t max_steps, double tolerance, double reduction,
+                          int32_t *cg_steps) {
   if (!u_out) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
   int rc = check_time_steps(ctx, dt, n_steps, out_every);
   if (rc) return rc;
@@ -2576,9 +2664,13 @@ int slod_fem_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_fi
   int64_t n_fine = 0;
   slod_fine_size(ctx, &n_fine);
   const long long n_nodes = n_fine / P.s;
-  // homogeneous Dirichlet conditions: the boundary rows of f and u0 are zero
-  std::vector<double> f(n_fine, 0.0), u0(n_fine, 0.0);
-  if (f_fine) std::copy(f_fine, f_fine + n_fine, f.begin());
+  const int nf = f_fine ? n_fields : 1;   // no forcing: one zero field
+  const std::vector<ThetaStage> stages = theta_stages(theta, dt, n_steps, n_startup);
+  std::vector<double> w(stages.size() * nf);
+  theta_weights(theta, n_steps, n_startup, nf, f_fine ? g : nullptr, w.data());
+  // homogeneous Dirichlet conditions: the boundary rows of the fields and of u0 are zero
+  std::vector<double> f((size_t)nf * n_fine, 0.0), u0(n_fine, 0.0);
+  if (f_fine) std::copy(f_fine, f_fine + (size_t)nf * n_fine, f.begin());
   if (u0_fine) std::copy(u0_fine, u0_fine + n_fine, u0.begin());
   const long long G = P.nsub + 1;
   for (long long node = 0; node < n_nodes; ++node) {
@@ -2590,50 +2682,140 @@ int slod_fem_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_fi
       bd = bd || i == 0 || i == G - 1;
     }
     if (bd)
-      for (int c = 0; c < P.s; ++c) f[node * P.s + c] = u0[node * P.s + c] = 0.0;
+      for (int c = 0; c < P.s; ++c) {
+        u0[node * P.s + c] = 0.0;
+        for (int q = 0; q < nf; ++q) f[(size_t)q * n_fine + node * P.s + c] = 0.0;
+      }
   }
-  double *d_r = nullptr, *d_delta = nullptr, *d_work = nullptr, *d_f = nullptr;
+  double *d_r = nullptr, *d_delta = nullptr, *d_work = nullptr, *d_F = nullptr;
   rc = online_scratch(ctx, &d_r, &d_delta, nullptr, nullptr, &d_work);
   if (rc) return rc;
-  rc = heat_scratch(ctx, 3 * (size_t)n_fine, &d_f);
+  rc = heat_scratch(ctx, (3 + (size_t)nf) * n_fine + w.size(), &d_F);   // fields | u | A u | load | weights
   if (rc) return rc;
-  double *d_u = d_f + n_fine, *d_q = d_u + n_fine;
+  double *d_u = d_F + (size_t)nf * n_fine, *d_q = d_u + n_fine, *d_load = d_q + n_fine, *d_w = d_load + n_fine;
   CgOperator A{nullptr, ctx->d_coef, n_nodes};
   A.op = kFineHeatDirichlet;
-  A.tau = dt;
-  cudaError_t e = cudaMemcpyAsync(d_f, f.data(), sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+  cudaError_t e = cudaMemcpyAsync(d_F, f.data(), sizeof(double) * f.size(), cudaMemcpyHostToDevice, 0);
   if (e == cudaSuccess) e = cudaMemcpyAsync(d_u, u0.data(), sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_w, w.data(), sizeof(double) * w.size(), cudaMemcpyHostToDevice, 0);
   long long n_launch = 0;
-  int failed_step = 0, flag = 0, st_steps = 0;
-  double res = 0.0;
-  for (int k = 1; k <= n_steps && e == cudaSuccess; ++k) {
+  int failed_step = 0, flag = 0, st_steps = 0, step_cg = 0;
+  double res = 0.0, failed_coef = 0.0;
+  for (size_t i = 0; i < stages.size() && e == cudaSuccess; ++i) {
+    const ThetaStage &sg = stages[i];
+    const int k = sg.step;
+    A.tau = sg.coef;
     e = launch_fine_apply(0, kFineStiffDirichlet, 0.0, n_nodes, ctx->d_coef, d_u, d_q);
-    if (e == cudaSuccess) e = launch_lincomb(0, n_fine, dt, d_f, -dt, d_q, d_r);   // dt (f - A u), zero boundary rows
+    if (e == cudaSuccess) e = launch_weighted_sum(0, n_fine, nf, d_w + i * nf, d_F, d_load);
+    if (e == cudaSuccess) e = launch_lincomb(0, n_fine, sg.tau, d_load, -sg.tau, d_q, d_r);   // tau (load - A u)
     if (e == cudaSuccess)
       e = run_cg(0, (int)n_fine, A, d_r, d_delta, d_work, max_steps, tolerance, reduction, &st_steps, &res, &flag,
                  &n_launch);
     if (e != cudaSuccess) break;
-    if (cg_steps) cg_steps[k - 1] = st_steps;
+    step_cg = (i > 0 && stages[i - 1].step == k ? step_cg : 0) + st_steps;
+    if (cg_steps) cg_steps[k - 1] = step_cg;
     if (flag != 1) {
       failed_step = k;
+      failed_coef = sg.coef;
       break;
     }
     e = launch_lincomb(0, n_fine, 1.0, d_u, 1.0, d_delta, d_u);
-    if (e == cudaSuccess && k % out_every == 0)
+    if (e == cudaSuccess && sg.ends_step && k % out_every == 0)
       e = cudaMemcpyAsync(u_out + (size_t)(k / out_every - 1) * n_fine, d_u, sizeof(double) * (size_t)n_fine,
                           cudaMemcpyDeviceToHost, 0);
-    n_launch += 3;
+    n_launch += 4;
   }
   if (e == cudaSuccess) e = cudaStreamSynchronize(0);
   ctx->launches += n_launch;
-  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string("slod_fem_heat_solve: ") + cudaGetErrorString(e));
+  if (e != cudaSuccess) return fail(ctx, SLOD_ERR_CUDA, std::string(name) + ": " + cudaGetErrorString(e));
   if (failed_step) {
     char buf[200];
-    std::snprintf(buf, sizeof buf, "time step %d: fine CG on M_h + dt A_h %s: %d steps, residual %.3e", failed_step,
-                  flag == 2 ? "broke down" : "did not converge", st_steps, res);
+    std::snprintf(buf, sizeof buf, "time step %d: fine CG on M_h + c A_h (c = %.6g) %s: %d steps, residual %.3e",
+                  failed_step, failed_coef, flag == 2 ? "broke down" : "did not converge", st_steps, res);
     return fail(ctx, SLOD_ERR_NUMERIC, buf);
   }
   return SLOD_OK;
+}
+
+int slod_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_coarse, double dt, int32_t n_steps,
+                    int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
+                    int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  return heat_theta_single(ctx, "slod_heat_solve", 1.0, dt, n_steps, out_every, 0, 1, f_fine, nullptr, u0_coarse,
+                           u_out, max_steps, tolerance, reduction, cg_steps);
+}
+
+int slod_heat_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, const double *u0_coarse, double dt,
+                          int32_t n_steps, int32_t out_every, double *u_out, int32_t max_steps, double tolerance,
+                          double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  return heat_theta_batch(ctx, "slod_heat_solve_batch", n_rhs, 1.0, dt, n_steps, out_every, 0, 1, f_fine, nullptr,
+                          u0_coarse, u_out, max_steps, tolerance, reduction, cg_steps);
+}
+
+int slod_fem_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_fine, double dt, int32_t n_steps,
+                        int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
+                        int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  NEED_DEVICE();
+  return fem_heat_theta(ctx, "slod_fem_heat_solve", 1.0, dt, n_steps, out_every, 0, 1, f_fine, nullptr, u0_fine, u_out,
+                        max_steps, tolerance, reduction, cg_steps);
+}
+
+// The theta-scheme entry points check every argument before the device and the call order, so that a maps-only handle
+// reports an invalid argument as such.
+static int check_theta_call(slod_ctx *ctx, double theta, double dt, int32_t n_steps, int32_t out_every,
+                            int32_t n_startup, int32_t n_fields, const double *f_fine, const double *g, size_t g_rows,
+                            const double *u_out, int32_t max_steps, double tolerance, double reduction) {
+  if (!u_out) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  int rc = check_time_steps(ctx, dt, n_steps, out_every);
+  if (rc) return rc;
+  rc = check_solver_control(ctx, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  return check_theta(ctx, theta, n_steps, n_startup, n_fields, f_fine, g,
+                     n_fields > 0 ? g_rows * ((size_t)n_steps + 1) * n_fields : 0);
+}
+
+int slod_heat_theta_solve(slod_ctx *ctx, double theta, double dt, int32_t n_steps, int32_t out_every,
+                          int32_t n_startup, int32_t n_fields, const double *f_fine, const double *g,
+                          const double *u0_coarse, double *u_out, int32_t max_steps, double tolerance,
+                          double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  int rc = check_theta_call(ctx, theta, dt, n_steps, out_every, n_startup, n_fields, f_fine, g, 1, u_out, max_steps,
+                            tolerance, reduction);
+  if (rc) return rc;
+  NEED_DEVICE();
+  return heat_theta_single(ctx, "slod_heat_theta_solve", theta, dt, n_steps, out_every, n_startup, n_fields, f_fine, g,
+                           u0_coarse, u_out, max_steps, tolerance, reduction, cg_steps);
+}
+
+int slod_heat_theta_solve_batch(slod_ctx *ctx, int32_t n_rhs, double theta, double dt, int32_t n_steps,
+                                int32_t out_every, int32_t n_startup, int32_t n_fields, const double *f_fine,
+                                const double *g, const double *u0_coarse, double *u_out, int32_t max_steps,
+                                double tolerance, double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  if (n_rhs < 1) return fail(ctx, SLOD_ERR_INVALID, "n_rhs must be at least 1");
+  int rc = check_theta_call(ctx, theta, dt, n_steps, out_every, n_startup, n_fields, f_fine, g, (size_t)n_rhs, u_out,
+                            max_steps, tolerance, reduction);
+  if (rc) return rc;
+  NEED_DEVICE();
+  return heat_theta_batch(ctx, "slod_heat_theta_solve_batch", n_rhs, theta, dt, n_steps, out_every, n_startup,
+                          n_fields, f_fine, g, u0_coarse, u_out, max_steps, tolerance, reduction, cg_steps);
+}
+
+int slod_fem_heat_theta_solve(slod_ctx *ctx, double theta, double dt, int32_t n_steps, int32_t out_every,
+                              int32_t n_startup, int32_t n_fields, const double *f_fine, const double *g,
+                              const double *u0_fine, double *u_out, int32_t max_steps, double tolerance,
+                              double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  int rc = check_theta_call(ctx, theta, dt, n_steps, out_every, n_startup, n_fields, f_fine, g, 1, u_out, max_steps,
+                            tolerance, reduction);
+  if (rc) return rc;
+  NEED_DEVICE();
+  return fem_heat_theta(ctx, "slod_fem_heat_theta_solve", theta, dt, n_steps, out_every, n_startup, n_fields, f_fine,
+                        g, u0_fine, u_out, max_steps, tolerance, reduction, cg_steps);
 }
 
 // ---- checkpoint: parameters + phi + A*phi (+ block-ELL coarse matrix) --------------------------------------------

@@ -1,10 +1,11 @@
-// The coarse mass matrix and backward Euler on the SLOD space.
+// The coarse mass matrix and theta-scheme time stepping on the SLOD space.
 //
 //   k_mass_apply     M_h phi       the exact Q1 mass matrix of the sub-cell grid applied to every basis function on its
 //                                  own node box; k_coarse_blocked / k_coarse then form M_H = C^T (M_h C) exactly as
 //                                  they form K = C^T (A C)
-//   k_ell_residual   tau (B - K U) the right-hand side of one backward-Euler step in increment form
-//   k_lincomb        a x + b y     S = M_H + tau K on the block-ELL arrays, u += delta
+//   k_ell_residual   tau (sum_q W_q B_q - K U)   the right-hand side of one theta-scheme step in increment form
+//   k_weighted_sum   sum_q w_q F_q                the load of one step of the fine reference
+//   k_lincomb        a x + b y                    S = M_H + c K on the block-ELL arrays, u += delta
 //
 // On the uniform grid M_h is the tensor product of the 1-D matrices h (1/6, 2/3, 1/6), block diagonal in the
 // components.  phi vanishes on the boundary of its node box and outside it, so applying M_h box by box is exact on every
@@ -54,12 +55,16 @@ k_mass_apply(int n_patches, const double *__restrict__ phi, double *__restrict__
   }
 }
 
-// R = tau (B - K U) for kb <= kBatch interleaved columns ([n][kb]; kb = 1: plain vectors).  One warp per row
-// (grid-stride as k_cg_spmv); lane l adds the entries t = l, l + 32, ... for every column, then one warp sum per column:
-// a column's arithmetic depends neither on kb nor on the other columns.
+// R = tau (sum_q W[q][j] B_q - K U) for kb <= kBatch interleaved columns ([n][kb]; kb = 1: plain vectors) and nf >= 1
+// loads B_q = B + q * b_stride, with per-column weights W[nf][kb].  One warp per row (grid-stride as k_cg_spmv); lane l
+// adds the entries t = l, l + 32, ... for every column, then one warp sum per column; lane j then sums the nf loads of
+// column j.  A column's arithmetic depends neither on kb nor on the other columns.  The load sum starts from its first
+// term, so nf = 1 with weight 1.0 gives tau (B - K U) exactly.  Each row reads nf loads per column: with per-step
+// forcing (nf = n_steps + 1) a trajectory reads O(n_steps^2) coarse values.
 __global__ void __launch_bounds__(kCgThreads)
-k_ell_residual(int nrows, int kb, const double *__restrict__ Kell, const double *__restrict__ U,
-               const double *__restrict__ B, double tau, double *__restrict__ R) {
+k_ell_residual(int nrows, int kb, const double *__restrict__ Kell, const double *__restrict__ U, int nf,
+               const double *__restrict__ B, long long b_stride, const double *__restrict__ W, double tau,
+               double *__restrict__ R) {
   __shared__ int sTab[kCgThreads / 32][3][kCgTab];
   const int s = cP.s, w = cP.w, ww = 2 * w + 1, dim = cP.dim;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -81,12 +86,29 @@ k_ell_residual(int nrows, int kb, const double *__restrict__ Kell, const double 
       for (int j = 0; j < kBatch; ++j)
         if (j < kb) acc[j] += kv * u[j];
     }
+    double v = 0.0;   // lane j: the K U entry of column j (warp_sum leaves the same bits in every lane)
 #pragma unroll
     for (int j = 0; j < kBatch; ++j) {
       if (j >= kb) break;   // kb is uniform
-      const double v = warp_sum(acc[j]);
-      if (lane == 0) R[(size_t)row * kb + j] = tau * (B[(size_t)row * kb + j] - v);
+      const double sj = warp_sum(acc[j]);
+      if (lane == j) v = sj;
     }
+    if (lane < kb) {   // lane j forms the load of column j, in field order: the columns' sums run side by side
+      const size_t i = (size_t)row * kb + lane;
+      double load = W[lane] * B[i];
+      for (int q = 1; q < nf; ++q) load += W[(size_t)q * kb + lane] * B[q * b_stride + i];
+      R[i] = tau * (load - v);
+    }
+  }
+}
+
+// out = sum_q w[q] F_q for nf >= 1 fields F_q = F + q n, summed from the first term in field order
+__global__ void __launch_bounds__(256)
+k_weighted_sum(long long n, int nf, const double *__restrict__ w, const double *__restrict__ F, double *__restrict__ out) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    double acc = w[0] * F[i];
+    for (int q = 1; q < nf; ++q) acc += w[q] * F[q * n + i];
+    out[i] = acc;
   }
 }
 

@@ -1377,9 +1377,14 @@ cudaError_t launch_mass_apply(cudaStream_t st, int n_patches, int s, const doubl
   k_mass_apply<<<rows < 148 * 16 ? rows : 148 * 16, 256, 0, st>>>(n_patches, phi, mphi, nf_max);
   return cudaGetLastError();
 }
-cudaError_t launch_ell_residual(cudaStream_t st, int nrows, int kb, const double *Kell, const double *U, const double *B,
-                                double tau, double *R) {
-  k_ell_residual<<<cg_multi_apply_blocks(nrows), kCgThreads, 0, st>>>(nrows, kb, Kell, U, B, tau, R);
+cudaError_t launch_ell_residual(cudaStream_t st, int nrows, int kb, const double *Kell, const double *U, int nf,
+                                const double *B, long long b_stride, const double *W, double tau, double *R) {
+  k_ell_residual<<<cg_multi_apply_blocks(nrows), kCgThreads, 0, st>>>(nrows, kb, Kell, U, nf, B, b_stride, W, tau, R);
+  return cudaGetLastError();
+}
+cudaError_t launch_weighted_sum(cudaStream_t st, long long n, int nf, const double *w, const double *F, double *out) {
+  const long long blocks = (n + 255) / 256;
+  k_weighted_sum<<<(int)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, st>>>(n, nf, w, F, out);
   return cudaGetLastError();
 }
 cudaError_t launch_lincomb(cudaStream_t st, long long n, double a, const double *x, double b, const double *y, double *z) {

@@ -145,14 +145,14 @@ enum FineOp {
   kFineEnergy = 1,          // the same without the boundary treatment: x.y = energy norm^2
   kFineMass = 2,            // mass matrix: x.y = L2 norm^2
   kFineLaplace = 3,         // component-wise unweighted Laplace: x.y = H1 seminorm^2
-  kFineHeatDirichlet = 4    // mass + tau * stiffness (backward Euler), with the boundary treatment of op 0
+  kFineHeatDirichlet = 4    // mass + tau * stiffness (theta-scheme step), with the boundary treatment of op 0
 };
 struct CgOperator {
   const double *Kell;     // block-ELL coarse matrix, or nullptr for a fine Dirichlet operator
   const double *d_coef;   // fine operator: sub-cell coefficients
   long long n_nodes;      // fine operator: nodes of the global grid
   int op = kFineStiffDirichlet;   // fine operator: kFineStiffDirichlet or kFineHeatDirichlet
-  double tau = 0.0;               // fine operator kFineHeatDirichlet: the time step
+  double tau = 0.0;               // fine operator kFineHeatDirichlet: the coefficient of the stiffness
 };
 size_t cg_workspace_doubles(const CgOperator &A, int nrows);
 cudaError_t run_cg(cudaStream_t st, int nrows, const CgOperator &A, const double *b, double *x, double *work,
@@ -176,9 +176,12 @@ cudaError_t run_cg_multi(cudaStream_t st, int nrows, const double *Kell, int kb,
 // heat equation on the SLOD space (heat.cuh)
 // M_h phi of every patch on its own node box, the [n_patches][s][nf_max] layout of A phi
 cudaError_t launch_mass_apply(cudaStream_t st, int n_patches, int s, const double *phi, double *mphi, int nf_max);
-// R = tau (B - K U) on the block-ELL matrix for kb <= kBatch interleaved columns (kb = 1: plain vectors)
-cudaError_t launch_ell_residual(cudaStream_t st, int nrows, int kb, const double *Kell, const double *U, const double *B,
-                                double tau, double *R);
+// R = tau (sum_q W[q][j] B_q - K U) on the block-ELL matrix for kb <= kBatch interleaved columns (kb = 1: plain
+// vectors) and nf >= 1 loads B_q = B + q b_stride in the layout of U; W: nf x kb device weights
+cudaError_t launch_ell_residual(cudaStream_t st, int nrows, int kb, const double *Kell, const double *U, int nf,
+                                const double *B, long long b_stride, const double *W, double tau, double *R);
+// out = sum_q w[q] F[q n .. q n + n) for nf >= 1 (w: nf device doubles)
+cudaError_t launch_weighted_sum(cudaStream_t st, long long n, int nf, const double *w, const double *F, double *out);
 // z = a x + b y (z may alias x or y)
 cudaError_t launch_lincomb(cudaStream_t st, long long n, double a, const double *x, double b, const double *y, double *z);
 // y = Op x for a FineOp (tau: kFineHeatDirichlet), no reduction

@@ -262,6 +262,38 @@ int slod_heat_solve_batch(slod_ctx *ctx, int32_t n_rhs, const double *f_fine, co
 int slod_fem_heat_solve(slod_ctx *ctx, const double *f_fine, const double *u0_fine, double dt, int32_t n_steps,
                         int32_t out_every, double *u_out, int32_t max_steps, double tolerance, double reduction,
                         int32_t *cg_steps);
+/* The theta scheme for M_H u' + K u = C^T f(t), theta in [1/2, 1] (1/2: Crank-Nicolson, 1: backward Euler), in the
+ * increment form above: (M_H + theta dt K) delta = dt (theta b(t_k) + (1 - theta) b(t_{k-1}) - K u^{k-1}).
+ * Forcing: f(x, t) = sum_q g_q(t) f_q(x), q = 0 .. n_fields - 1.  f_fine holds the fields [n_fields][n_fine] (NULL: zero
+ * forcing; n_fields and g are then ignored); g holds g_q(t_k) at t_k = k dt as [n_steps + 1][n_fields] (NULL: g = 1).
+ * Arbitrary per-step loads are n_fields = n_steps + 1 with g the identity.  C^T f_q is formed once per field and kept
+ * on the device (n_fields coarse vectors per trajectory); every step's residual reads all n_fields of them, so the
+ * per-step form costs O(n_steps) per step.
+ * Rannacher start-up: each of the first n_startup steps is two backward-Euler steps of dt / 2 with the loads
+ * (g(t_{k-1}) + g(t_k)) / 2 and g(t_k); cg_steps of such a step is the sum of its two solves.  Crank-Nicolson leaves
+ * the stiff modes (dt lambda >> 1) of a non-smooth u0 undamped, with amplification near -1: one or two start-up steps
+ * damp them.  M_H + c K is kept for the last coefficient c of K formed (theta dt, or dt / 2 during start-up).
+ * At theta = 1, n_fields = 1, g = NULL, n_startup = 0 these are slod_heat_solve / _batch / slod_fem_heat_solve, bit
+ * for bit.  Every argument is checked before the device and the call order: theta outside [1/2, 1], n_startup < 0 or
+ * > n_steps, n_fields < 1 with fields given, a non-finite entry of g (read only with fields given) and the checks of
+ * slod_heat_solve -> SLOD_ERR_INVALID.  Then SLOD_ERR_CUDA (maps-only handle), SLOD_ERR_STATE and SLOD_ERR_NUMERIC as
+ * there.
+ * slod_heat_theta_solve_batch: f_fine [n_rhs][n_fields][n_fine], g [n_rhs][n_steps + 1][n_fields], u0 [n_rhs][n_coarse],
+ * u_out [n_out][n_rhs][n_coarse], cg_steps [n_steps][n_rhs]; columns are independent as in slod_heat_solve_batch.
+ * slod_fem_heat_theta_solve: the fine-scale reference of the same scheme (M_h + theta dt A_h, as slod_fem_heat_solve),
+ * fine u0 and u_out [n_out][n_fine]. */
+int slod_heat_theta_solve(slod_ctx *ctx, double theta, double dt, int32_t n_steps, int32_t out_every,
+                          int32_t n_startup, int32_t n_fields, const double *f_fine, const double *g,
+                          const double *u0_coarse, double *u_out, int32_t max_steps, double tolerance,
+                          double reduction, int32_t *cg_steps);
+int slod_heat_theta_solve_batch(slod_ctx *ctx, int32_t n_rhs, double theta, double dt, int32_t n_steps,
+                                int32_t out_every, int32_t n_startup, int32_t n_fields, const double *f_fine,
+                                const double *g, const double *u0_coarse, double *u_out, int32_t max_steps,
+                                double tolerance, double reduction, int32_t *cg_steps);
+int slod_fem_heat_theta_solve(slod_ctx *ctx, double theta, double dt, int32_t n_steps, int32_t out_every,
+                              int32_t n_startup, int32_t n_fields, const double *f_fine, const double *g,
+                              const double *u0_fine, double *u_out, int32_t max_steps, double tolerance,
+                              double reduction, int32_t *cg_steps);
 
 /* ---- checkpoint of the offline phase (SURVEY 8f row 4; the reference has none: it recomputes every run) ----------
  * slod_save_state writes the parameters, the basis (phi, A*phi) and, if assembled, the coarse matrix to one binary

@@ -1,4 +1,4 @@
-"""Coarse mass matrix and backward Euler on the SLOD space at the headline workload.
+"""Coarse mass matrix and theta-scheme time stepping on the SLOD space at the headline workload.
 
     python tools/heat_bench.py [--out profiles/heat_bench.json] [--workload NAME] [--steps 20] [--k 16] [--dt 1e-3]
                                [--reps 3]
@@ -9,7 +9,13 @@ once, then times, after one warm-up call of each, the median over --reps repetit
     (M_h phi and the product C^T (M_h C), slod_get_timings [6] / [7]);
   * slod_heat_solve: --steps backward-Euler steps for the forcing f = 1 from u0 = 0, host clock, CG steps per time step;
   * slod_heat_solve_batch with --k seeded random forcings, the same steps: host clock, CG steps per time step (the
-    largest over the columns, which sets the group's step count).
+    largest over the columns, which sets the group's step count);
+  * slod_heat_theta_solve at theta = 1/2 (Crank-Nicolson) for the same forcing with g = sin(pi t / T), T = steps dt,
+    without and with two Rannacher start-up steps, and with 8 fields (f = 1 and 7 seeded ones, seeded g);
+  * slod_heat_theta_solve_batch at theta = 1/2 for the --k forcings (one field each, g as above) and with 8 fields per
+    column (seeded);
+  * both at theta = 1/2 with per-step forcing: steps + 1 seeded fields and g the identity (every step reads all
+    steps + 1 coarse loads, so this time grows with the number of steps).
 All CG solves stop at a reduction of 1e-10.  Host-buffer copies are included in the host times.  The device name and
 power limit are read in the same run.  Writes one JSON line to --out and prints it.
 """
@@ -89,6 +95,32 @@ def main():
     F = rng.standard_normal((args.k, nf)) * h ** w["dim"]
     batch_ms, (_, stk) = _median_ms(lambda: ctx.heat_solve_batch(F, None, args.dt, args.steps, args.steps, **CG),
                                     args.reps)
+    T = args.dt * args.steps
+    g1 = np.sin(np.pi * np.arange(args.steps + 1) * args.dt / T)[:, None]
+    nq = 8
+    F8 = np.concatenate([f1[None], rng.standard_normal((nq - 1, nf)) * h ** w["dim"]])
+    G8 = rng.standard_normal((args.steps + 1, nq))
+    theta = {}
+    FP = rng.standard_normal((args.steps + 1, nf)) * h ** w["dim"]
+    GP = np.eye(args.steps + 1)
+    for key, fields, g, ns in (("cn", f1[None], g1, 0), ("cn_startup2", f1[None], g1, 2), ("cn_fields8", F8, G8, 0),
+                               ("cn_per_step", FP, GP, 0)):
+        ms, (_, st) = _median_ms(lambda: ctx.heat_theta_solve(fields, g, None, 0.5, args.dt, args.steps, args.steps,
+                                                              n_startup=ns, **CG), args.reps)
+        theta[key] = {"n_fields": fields.shape[0], "n_startup": ns, "ms": ms, "ms_per_step": ms / args.steps,
+                      "cg_steps": st.tolist(), "ms_per_cg_step": ms / max(int(st.sum()), 1)}
+    Gk = np.broadcast_to(g1, (args.k,) + g1.shape)
+    FK8 = rng.standard_normal((args.k, nq, nf)) * h ** w["dim"]
+    GK8 = rng.standard_normal((args.k, args.steps + 1, nq))
+    FKP = np.broadcast_to(FP, (args.k,) + FP.shape)
+    GKP = np.broadcast_to(GP, (args.k,) + GP.shape)
+    for key, fields, g in (("cn_batch", F[:, None], Gk), ("cn_batch_fields8", FK8, GK8),
+                           ("cn_batch_per_step", FKP, GKP)):
+        ms, (_, st) = _median_ms(lambda: ctx.heat_theta_solve_batch(fields, g, None, 0.5, args.dt, args.steps,
+                                                                    args.steps, **CG), args.reps)
+        theta[key] = {"k": args.k, "n_fields": fields.shape[1], "ms": ms, "ms_per_step": ms / args.steps,
+                      "ms_per_step_per_rhs": ms / args.steps / args.k, "cg_steps_max": st.max(axis=1).tolist(),
+                      "ms_per_cg_step": ms / max(int(st.max(axis=1).sum()), 1)}
     name, power = _device()
     row = {
         "metric": "heat", "workload": args.workload, "device": name, "power_limit": power,
@@ -104,6 +136,7 @@ def main():
                              "ms_per_step_per_rhs": batch_ms / args.steps / args.k,
                              "cg_steps_max": stk.max(axis=1).tolist(),
                              "ms_per_cg_step": batch_ms / max(int(stk.max(axis=1).sum()), 1)},
+        "heat_theta_solve": theta,
     }
     line = json.dumps(row)
     print(line)
