@@ -33,6 +33,7 @@ EXPORTS = [
     "slod_prolongate_batch", "slod_assemble_coarse_mass", "slod_get_coarse_mass_csr", "slod_l2_project_batch",
     "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan", "slod_debug_select",
     "slod_update_basis", "slod_heat_theta_solve", "slod_heat_theta_solve_batch", "slod_fem_heat_theta_solve",
+    "slod_wave_solve", "slod_wave_solve_batch", "slod_fem_wave_solve",
 ]
 # slod_get_plan entries, in order
 PLAN_KEYS = ["mma_variant", "split_solver", "dense_ntile", "gmem_window", "dense_coef_gmem", "coarse_blocked", "use_ql",
@@ -94,6 +95,10 @@ def load_library(path=None):
     lib.slod_heat_theta_solve.argtypes = [vp] + theta
     lib.slod_heat_theta_solve_batch.argtypes = [vp, i32] + theta
     lib.slod_fem_heat_theta_solve.argtypes = [vp] + theta
+    wave = [dbl, dbl, i32, i32, i32, P(dbl), P(dbl), P(dbl), P(dbl), P(dbl), P(dbl), P(dbl), i32, dbl, dbl, P(i32)]
+    lib.slod_wave_solve.argtypes = [vp] + wave
+    lib.slod_wave_solve_batch.argtypes = [vp, i32] + wave
+    lib.slod_fem_wave_solve.argtypes = [vp] + wave
     lib.slod_fine_norms.argtypes = [vp, P(dbl), P(dbl), P(dbl), P(dbl)]
     lib.slod_get_patch_info.argtypes = [vp, i64] + [P(i32)] * 6 + [P(i32), P(i32)]
     lib.slod_get_patch_cells.argtypes = [vp, i64, P(C.c_uint32), P(i32)]
@@ -539,6 +544,67 @@ class SlodContext:
                                                     None if u0 is None else _dp(u0), _dp(out), max_steps, tolerance,
                                                     reduction, steps.ctypes.data_as(C.POINTER(C.c_int32))))
         return out, steps
+
+    # -- wave equation M_H u'' + K u = sum_q g_q(t) C^T f_q, Newmark with gamma = 1/2 (slod_wave_solve / _batch,
+    #    slod_fem_wave_solve) --
+    def wave_solve(self, f_fields, g, u0_coarse, v0_coarse, beta, dt, n_steps, out_every=1, max_steps=10000,
+                   tolerance=0.0, reduction=1e-12):
+        """Newmark on the SLOD space: f_fields (n_fields, n_fine) or None, g (n_steps + 1, n_fields) or None (g = 1),
+        u0_coarse / v0_coarse or None.  Returns (U, V (n_steps // out_every, n_coarse), energy[n_out + 1],
+        cg_steps int32[n_steps + 1])."""
+        nc = self.n_patches * self.s
+        f, gg, nq = self._fields(f_fields, g, n_steps, (), self.n_fine)
+        u0 = self._vec_or_none(u0_coarse, nc, "coarse vector")
+        v0 = self._vec_or_none(v0_coarse, nc, "coarse vector")
+        n_out = max(n_steps // max(out_every, 1), 1)
+        u, v, en = np.empty((n_out, nc)), np.empty((n_out, nc)), np.empty(n_out + 1)
+        steps = np.zeros(max(n_steps + 1, 1), dtype=np.int32)
+        self._ck(self.lib.slod_wave_solve(self.h, beta, dt, n_steps, out_every, nq, None if f is None else _dp(f),
+                                          None if gg is None else _dp(gg), None if u0 is None else _dp(u0),
+                                          None if v0 is None else _dp(v0), _dp(u), _dp(v), _dp(en), max_steps,
+                                          tolerance, reduction, steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return u, v, en, steps
+
+    def wave_solve_batch(self, F, G, U0, V0, beta, dt, n_steps, out_every=1, max_steps=10000, tolerance=0.0,
+                         reduction=1e-12):
+        """k trajectories at once: F (k, n_fields, n_fine), G (k, n_steps + 1, n_fields), U0 / V0 (k, n_coarse) (each may
+        be None).  Returns (U, V (n_steps // out_every, k, n_coarse), energy (n_out + 1, k), cg_steps int32
+        (n_steps + 1, k))."""
+        nc = self.n_patches * self.s
+        given = [a for a in (F, U0, V0) if a is not None]
+        if not given:
+            raise ValueError("give F, U0 or V0 (the number of trajectories)")
+        k = np.shape(given[0])[0]
+        f, gg, nq = self._fields(F, G, n_steps, (k,), self.n_fine)
+        u0 = None if U0 is None else self._block(U0, nc, "coarse block")
+        v0 = None if V0 is None else self._block(V0, nc, "coarse block")
+        if any(a is not None and a.shape[0] != k for a in (u0, v0)):
+            raise ValueError("F, U0 and V0 must have the same number of rows")
+        n_out = max(n_steps // max(out_every, 1), 1)
+        u, v, en = np.empty((n_out, k, nc)), np.empty((n_out, k, nc)), np.empty((n_out + 1, k))
+        steps = np.zeros((max(n_steps + 1, 1), k), dtype=np.int32)
+        self._ck(self.lib.slod_wave_solve_batch(self.h, k, beta, dt, n_steps, out_every, nq,
+                                                None if f is None else _dp(f), None if gg is None else _dp(gg),
+                                                None if u0 is None else _dp(u0), None if v0 is None else _dp(v0),
+                                                _dp(u), _dp(v), _dp(en), max_steps, tolerance, reduction,
+                                                steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return u, v, en, steps
+
+    def fem_wave_solve(self, f_fields, g, u0_fine, v0_fine, beta, dt, n_steps, out_every=1, max_steps=200000,
+                       tolerance=0.0, reduction=1e-12):
+        """The fine-scale reference of wave_solve.  Returns (U, V (n_steps // out_every, n_fine), energy[n_out + 1],
+        cg_steps int32[n_steps + 1])."""
+        f, gg, nq = self._fields(f_fields, g, n_steps, (), self.n_fine)
+        u0 = self._vec_or_none(u0_fine, self.n_fine, "fine vector")
+        v0 = self._vec_or_none(v0_fine, self.n_fine, "fine vector")
+        n_out = max(n_steps // max(out_every, 1), 1)
+        u, v, en = np.empty((n_out, self.n_fine)), np.empty((n_out, self.n_fine)), np.empty(n_out + 1)
+        steps = np.zeros(max(n_steps + 1, 1), dtype=np.int32)
+        self._ck(self.lib.slod_fem_wave_solve(self.h, beta, dt, n_steps, out_every, nq, None if f is None else _dp(f),
+                                              None if gg is None else _dp(gg), None if u0 is None else _dp(u0),
+                                              None if v0 is None else _dp(v0), _dp(u), _dp(v), _dp(en), max_steps,
+                                              tolerance, reduction, steps.ctypes.data_as(C.POINTER(C.c_int32))))
+        return u, v, en, steps
 
     # -- fine-scale reference problem (assemble_and_solve_fem_problem, source/LOD.cc:1004-1094) and norms (:1252) --
     def fem_solve(self, f_fine, max_steps=200000, tolerance=1e-12, reduction=1e-10):

@@ -2768,6 +2768,309 @@ int slod_fem_heat_theta_solve(slod_ctx *ctx, double theta, double dt, int32_t n_
                         g, u0_fine, u_out, max_steps, tolerance, reduction, cg_steps);
 }
 
+// ---- wave equation on the SLOD space: Newmark time stepping (gamma = 1/2) ----
+// M_H u'' + K u = b(t), b(t) = sum_q g_q(t) C^T f_q.  Each step solves for the acceleration with S = M_H + beta dt^2 K
+// (wave.cuh): the right-hand side b(t_{k+1}) - K ut is k_ell_residual with U = ut and tau = 1, and the CG drivers start
+// from zero.  beta = 0 solves with M_H itself: heat_form_S treats a coefficient of 0 as "not formed".
+static int check_wave_call(slod_ctx *ctx, double beta, double dt, int32_t n_steps, int32_t out_every, int32_t n_fields,
+                           const double *f_fine, const double *g, size_t g_rows, const double *u_out, int32_t max_steps,
+                           double tolerance, double reduction) {
+  if (!u_out) return fail(ctx, SLOD_ERR_INVALID, "null buffer");
+  int rc = check_time_steps(ctx, dt, n_steps, out_every);
+  if (rc) return rc;
+  rc = check_solver_control(ctx, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  if (!(beta >= 0.0 && beta <= 0.5)) return fail(ctx, SLOD_ERR_INVALID, "beta must be in [0, 1/2]");
+  if (f_fine && n_fields < 1) return fail(ctx, SLOD_ERR_INVALID, "n_fields must be at least 1");
+  if (f_fine && g)
+    for (size_t i = 0, n = g_rows * ((size_t)n_steps + 1) * n_fields; i < n; ++i)
+      if (!std::isfinite(g[i])) return fail(ctx, SLOD_ERR_INVALID, "g has a non-finite entry");
+  return SLOD_OK;
+}
+
+// the weights g_q(t_k) of one column, w[k][nf] for k = 0 .. n_steps; g [n_steps + 1][nf] or NULL (g = 1)
+static void wave_weights(int n_steps, int nf, const double *g, double *w) {
+  for (size_t i = 0; i < ((size_t)n_steps + 1) * nf; ++i) w[i] = g ? g[i] : 1.0;
+}
+
+// The failure of an acceleration solve: step 0 is the start solve M a_0 = b(t_0) - K u_0.
+static int wave_outcome(slod_ctx *ctx, bool fine, int step, int column, double c, int flag, int steps, double res) {
+  const char *label = step == 0 ? (fine ? "start solve (step 0): fine CG on M_h" : "start solve (step 0): CG on M_H")
+                      : c > 0 ? (fine ? "fine CG on M_h + c A_h" : "CG on M_H + c K")
+                              : (fine ? "fine CG on M_h" : "CG on M_H");
+  return cg_outcome(ctx, step, column, label, step == 0 ? 0.0 : c, flag, steps, res);
+}
+
+// n_rhs trajectories of the coarse scheme in groups of kBatch interleaved columns; batch = false: one trajectory with
+// the single-vector kernels (run_cg), which agrees with a one-column batch to the solver tolerance.
+static int wave_coarse(slod_ctx *ctx, const char *name, bool batch, int32_t n_rhs, double beta, double dt,
+                       int32_t n_steps, int32_t out_every, int32_t n_fields, const double *f_fine, const double *g,
+                       const double *u0_coarse, const double *v0_coarse, double *u_out, double *v_out,
+                       double *energy_out, int32_t max_steps, double tolerance, double reduction, int32_t *cg_steps) {
+  CK(cudaSetDevice(ctx->device));
+  BIND_PARAMS((cudaStream_t)0);
+  int rc = heat_prepare(ctx, dt, n_steps, out_every, u_out, max_steps, tolerance, reduction);
+  if (rc) return rc;
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const int nrows = (int)(ctx->n_patches * ctx->P.s);
+  const int n_groups = batch ? (n_rhs + kBatch - 1) / kBatch : 1;
+  const int gmax = batch ? kBatch : 1;          // columns of a full group
+  const size_t gsz = (size_t)gmax * nrows;      // one interleaved group
+  const int nf = f_fine ? n_fields : 1;         // no forcing: one zero load
+  const size_t nk = (size_t)n_steps + 1, wg = nk * nf * gmax;   // weights of one group: [k][q][kb]
+  std::vector<double> w((size_t)n_groups * wg, 0.0), wj(nk * nf);
+  for (int j = 0; j < n_rhs; ++j) {
+    wave_weights(n_steps, nf, f_fine && g ? g + (size_t)j * nk * nf : nullptr, wj.data());
+    const int grp = j / gmax, jj = j % gmax, kb = std::min(gmax, n_rhs - grp * gmax);
+    for (size_t i = 0; i < nk * nf; ++i) w[grp * wg + i * kb + jj] = wj[i];
+  }
+  BatchScratch ws{};
+  double *d_f = nullptr, *d_r = nullptr, *d_anew = nullptr, *d_work = nullptr;
+  if (batch) {
+    rc = batch_scratch(ctx, &ws);
+    d_r = ws.coarse_a;
+    d_anew = ws.coarse_b;
+    d_work = ws.work;
+  } else {
+    rc = online_scratch(ctx, &d_f, nullptr, &d_r, &d_anew, &d_work);
+  }
+  if (rc) return rc;
+  // [group] u | v | a | ut, each [nrows][kb] | loads C^T f_q, [q][group][nrows][kb] | weights | energy partials | E
+  const size_t b_stride = (size_t)n_groups * gsz, n_part = wave_energy_workspace_doubles(nrows);
+  rc = grow(ctx, ctx->d_heat, ctx->heat_doubles, (4 + (size_t)nf) * b_stride + w.size() + n_part + kBatch);
+  if (rc) return rc;
+  double *d_state = ctx->d_heat, *d_B = d_state + 4 * b_stride, *d_W = d_B + nf * b_stride;
+  double *d_part = d_W + w.size(), *d_E = d_part + n_part;
+  auto U = [&](int grp, int which) { return d_state + (size_t)which * b_stride + grp * gsz; };   // 0 u, 1 v, 2 a, 3 ut
+  cudaError_t e = cudaMemcpyAsync(d_W, w.data(), sizeof(double) * w.size(), cudaMemcpyHostToDevice, 0);
+  long long n_launch = 0;
+  for (int grp = 0; grp < n_groups && e == cudaSuccess; ++grp) {
+    const int j0 = grp * gmax, kb = std::min(gmax, n_rhs - j0);
+    double *B = d_B + grp * gsz;
+    if (f_fine) {
+      for (int q = 0; q < nf && e == cudaSuccess; ++q) {
+        // field q of the group's columns, one copy per column (the host rows are nf n_fine doubles apart)
+        for (int c = 0; c < kb && e == cudaSuccess; ++c)
+          e = cudaMemcpyAsync((batch ? ws.fine_stage : d_f) + (size_t)c * n_fine, f_fine + ((size_t)(j0 + c) * nf + q) * n_fine,
+                              sizeof(double) * (size_t)n_fine, cudaMemcpyHostToDevice, 0);
+        if (e == cudaSuccess && batch) e = launch_interleave(0, n_fine, kb, ws.fine_stage, ws.fine, true);
+        if (e == cudaSuccess)
+          e = batch ? launch_coarse_rhs_multi(0, (int)ctx->n_patches, ctx->P.s, kb, ctx->d_phi, ws.fine,
+                                              B + q * b_stride, ctx->P.NfMax)
+                    : launch_coarse_rhs(0, (int)ctx->n_patches, ctx->P.s, ctx->d_phi, d_f, B + q * b_stride,
+                                        ctx->P.NfMax);
+        n_launch += batch ? 2 : 1;
+      }
+    } else if (e == cudaSuccess) {
+      e = cudaMemsetAsync(B, 0, sizeof(double) * kb * (size_t)nrows, 0);
+    }
+    const double *init[2] = {u0_coarse, v0_coarse};
+    for (int which = 0; which < 2 && e == cudaSuccess; ++which) {
+      if (!init[which]) {
+        e = cudaMemsetAsync(U(grp, which), 0, sizeof(double) * kb * (size_t)nrows, 0);
+      } else if (batch) {
+        e = upload_group(init[which] + (size_t)j0 * nrows, nrows, kb, ws.coarse_stage, U(grp, which));
+        n_launch += 1;
+      } else {
+        e = cudaMemcpyAsync(U(grp, which), init[which], sizeof(double) * nrows, cudaMemcpyHostToDevice, 0);
+      }
+    }
+  }
+  // S = M_H + beta dt^2 K for the steps; the start solve and beta = 0 use M_H
+  const double coef = beta * dt * dt;
+  if (e == cudaSuccess && coef > 0.0) e = heat_form_S(ctx, coef, &n_launch);
+  std::vector<int> st_steps(n_rhs, 0), flag(n_rhs, 0);
+  std::vector<double> res(n_rhs, 0.0);
+  int failed_step = -1, failed_col = -1;
+  for (int k = 0; k <= n_steps && e == cudaSuccess && failed_step < 0; ++k) {
+    const double *Sell = (k > 0 && coef > 0.0) ? ctx->d_Sell : ctx->d_Mell;
+    const bool out = k == 0 || k % out_every == 0;   // k = 0: only the energy at t_0
+    for (int grp = 0; grp < n_groups && e == cudaSuccess; ++grp) {
+      const int j0 = grp * gmax, kb = std::min(gmax, n_rhs - j0);
+      // k = 0: M a_0 = b(t_0) - K u_0; k > 0: S a_k = b(t_k) - K ut
+      e = launch_ell_residual(0, nrows, kb, ctx->d_Kell, U(grp, k == 0 ? 0 : 3), nf, d_B + grp * gsz,
+                              (long long)b_stride, d_W + grp * wg + (size_t)k * nf * kb, 1.0, d_r);
+      double *x = k == 0 ? U(grp, 2) : d_anew;
+      if (e == cudaSuccess) {
+        if (batch) {
+          e = run_cg_multi(0, nrows, Sell, kb, d_r, x, d_work, max_steps, tolerance, reduction, &st_steps[j0],
+                           &res[j0], &flag[j0], &n_launch);
+        } else {
+          const CgOperator S{Sell, nullptr, 0};
+          e = run_cg(0, nrows, S, d_r, x, d_work, max_steps, tolerance, reduction, &st_steps[0], &res[0], &flag[0],
+                     &n_launch);
+        }
+      }
+      if (e != cudaSuccess) break;
+      for (int j = j0; j < j0 + kb; ++j) {
+        if (cg_steps) cg_steps[(size_t)k * n_rhs + j] = st_steps[j];
+        if (flag[j] != 1 && failed_step < 0) {
+          failed_step = k;
+          failed_col = j;
+        }
+      }
+      if (failed_step >= 0) break;
+      e = launch_newmark_update(0, (long long)kb * nrows, k == 0, beta, dt, U(grp, 0), U(grp, 1), U(grp, 2), d_anew,
+                                U(grp, 3));
+      n_launch += 2;
+      if (e == cudaSuccess && out && energy_out) {
+        e = launch_wave_energy(0, nrows, kb, ctx->d_Kell, ctx->d_Mell, U(grp, 0), U(grp, 1), d_part, d_E);
+        if (e == cudaSuccess)
+          e = cudaMemcpyAsync(energy_out + (size_t)(k / out_every) * n_rhs + j0, d_E, sizeof(double) * kb,
+                              cudaMemcpyDeviceToHost, 0);
+        n_launch += 2;
+      }
+    }
+    if (e != cudaSuccess || failed_step >= 0 || k == 0 || k % out_every != 0) continue;
+    const int o = k / out_every - 1;
+    double *outs[2] = {u_out, v_out};
+    for (int which = 0; which < 2; ++which)
+      for (int grp = 0; grp < n_groups && e == cudaSuccess && outs[which]; ++grp) {
+        const int j0 = grp * gmax, kb = std::min(gmax, n_rhs - j0);
+        double *host = outs[which] + ((size_t)o * n_rhs + j0) * nrows;
+        if (batch) {
+          e = download_group(U(grp, which), nrows, kb, ws.coarse_stage, host);
+          n_launch += 1;
+        } else {
+          e = cudaMemcpyAsync(host, U(grp, which), sizeof(double) * nrows, cudaMemcpyDeviceToHost, 0);
+        }
+      }
+  }
+  rc = finish_call(ctx, name, e, n_launch);
+  if (rc || failed_step < 0) return rc;
+  return wave_outcome(ctx, false, failed_step, batch ? failed_col : -1, coef, flag[failed_col], st_steps[failed_col],
+                      res[failed_col]);
+}
+
+// the fine-scale reference trajectory: the same scheme with M_h + beta dt^2 A_h on the global grid (homogeneous
+// Dirichlet rows: kFineHeatDirichlet with tau = beta dt^2; tau = 0 is M_h with identity boundary rows).  The energy is
+// 1/2 v^T M_h v + 1/2 u^T A_h u from the quadratic forms of k_fine_apply, exact because u and v vanish on the boundary.
+static int fem_wave(slod_ctx *ctx, double beta, double dt, int32_t n_steps, int32_t out_every, int32_t n_fields,
+                    const double *f_fine, const double *g, const double *u0_fine, const double *v0_fine, double *u_out,
+                    double *v_out, double *energy_out, int32_t max_steps, double tolerance, double reduction,
+                    int32_t *cg_steps) {
+  const char *name = "slod_fem_wave_solve";
+  CK(cudaSetDevice(ctx->device));
+  int rc = prepare_coefficients(ctx);
+  if (rc) return rc;
+  BIND_PARAMS((cudaStream_t)0);
+  int64_t n_fine = 0;
+  slod_fine_size(ctx, &n_fine);
+  const long long n_nodes = n_fine / ctx->P.s;
+  const int nf = f_fine ? n_fields : 1;   // no forcing: one zero field
+  std::vector<double> w(((size_t)n_steps + 1) * nf);
+  wave_weights(n_steps, nf, f_fine ? g : nullptr, w.data());
+  std::vector<double> f((size_t)nf * n_fine, 0.0), x0(2 * (size_t)n_fine, 0.0);   // boundary rows zero
+  if (f_fine) std::copy(f_fine, f_fine + (size_t)nf * n_fine, f.begin());
+  if (u0_fine) std::copy(u0_fine, u0_fine + n_fine, x0.begin());
+  if (v0_fine) std::copy(v0_fine, v0_fine + n_fine, x0.begin() + n_fine);
+  zero_boundary_rows(ctx->P, f.data(), nf, n_fine);
+  zero_boundary_rows(ctx->P, x0.data(), 2, n_fine);
+  int nb = 0;
+  launch_fine_quadratic_form(0, kFineMass, n_nodes, nullptr, nullptr, nullptr, &nb);
+  double *d_r = nullptr, *d_anew = nullptr, *d_work = nullptr;
+  rc = online_scratch(ctx, &d_r, &d_anew, nullptr, nullptr, &d_work);
+  if (rc) return rc;
+  // fields | u | v | a | ut | A ut | load | weights | energy partials
+  rc = grow(ctx, ctx->d_heat, ctx->heat_doubles, (6 + (size_t)nf) * n_fine + w.size() + 2 * (size_t)nb);
+  if (rc) return rc;
+  double *d_F = ctx->d_heat, *d_u = d_F + (size_t)nf * n_fine, *d_v = d_u + n_fine, *d_a = d_v + n_fine;
+  double *d_ut = d_a + n_fine, *d_q = d_ut + n_fine, *d_load = d_q + n_fine, *d_w = d_load + n_fine;
+  double *d_part = d_w + w.size();
+  CgOperator A{nullptr, ctx->d_coef, n_nodes};
+  A.op = kFineHeatDirichlet;
+  cudaError_t e = cudaMemcpyAsync(d_F, f.data(), sizeof(double) * f.size(), cudaMemcpyHostToDevice, 0);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_u, x0.data(), sizeof(double) * x0.size(), cudaMemcpyHostToDevice, 0);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_w, w.data(), sizeof(double) * w.size(), cudaMemcpyHostToDevice, 0);
+  const double coef = beta * dt * dt;
+  std::vector<double> part(2 * (size_t)nb);
+  long long n_launch = 0;
+  int failed_step = -1, flag = 0, st_steps = 0;
+  double res = 0.0;
+  for (int k = 0; k <= n_steps && e == cudaSuccess; ++k) {
+    A.tau = k == 0 ? 0.0 : coef;
+    // k = 0: M a_0 = b(t_0) - A u_0; k > 0: (M + beta dt^2 A) a_k = b(t_k) - A ut
+    e = launch_fine_apply(0, kFineStiffDirichlet, 0.0, n_nodes, ctx->d_coef, k == 0 ? d_u : d_ut, d_q);
+    if (e == cudaSuccess) e = launch_weighted_sum(0, n_fine, nf, d_w + (size_t)k * nf, d_F, d_load);
+    if (e == cudaSuccess) e = launch_lincomb(0, n_fine, 1.0, d_load, -1.0, d_q, d_r);
+    if (e == cudaSuccess)
+      e = run_cg(0, (int)n_fine, A, d_r, k == 0 ? d_a : d_anew, d_work, max_steps, tolerance, reduction, &st_steps,
+                 &res, &flag, &n_launch);
+    if (e != cudaSuccess) break;
+    if (cg_steps) cg_steps[k] = st_steps;
+    if (flag != 1) {
+      failed_step = k;
+      break;
+    }
+    e = launch_newmark_update(0, n_fine, k == 0, beta, dt, d_u, d_v, d_a, d_anew, d_ut);
+    n_launch += 4;
+    if (e != cudaSuccess || (k > 0 && k % out_every != 0)) continue;
+    const size_t o = (size_t)(k / out_every);   // k = 0: only the energy at t_0
+    if (k > 0 && e == cudaSuccess)
+      e = cudaMemcpyAsync(u_out + (o - 1) * n_fine, d_u, sizeof(double) * (size_t)n_fine, cudaMemcpyDeviceToHost, 0);
+    if (k > 0 && e == cudaSuccess && v_out)
+      e = cudaMemcpyAsync(v_out + (o - 1) * n_fine, d_v, sizeof(double) * (size_t)n_fine, cudaMemcpyDeviceToHost, 0);
+    if (e == cudaSuccess && energy_out) {
+      e = launch_fine_quadratic_form(0, kFineMass, n_nodes, ctx->d_coef, d_v, d_part, &nb);
+      if (e == cudaSuccess) e = launch_fine_quadratic_form(0, kFineEnergy, n_nodes, ctx->d_coef, d_u, d_part + nb, &nb);
+      if (e == cudaSuccess)
+        e = cudaMemcpyAsync(part.data(), d_part, sizeof(double) * part.size(), cudaMemcpyDeviceToHost, 0);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+      n_launch += 2;
+      if (e != cudaSuccess) break;
+      double sum[2] = {0.0, 0.0};
+      for (int i = 0; i < 2; ++i)
+        for (int b = 0; b < nb; ++b) sum[i] += part[(size_t)i * nb + b];   // block order: reproducible
+      energy_out[o] = 0.5 * sum[0] + 0.5 * sum[1];
+    }
+  }
+  rc = finish_call(ctx, name, e, n_launch);
+  if (rc || failed_step < 0) return rc;
+  return wave_outcome(ctx, true, failed_step, -1, coef, flag, st_steps, res);
+}
+
+int slod_wave_solve(slod_ctx *ctx, double beta, double dt, int32_t n_steps, int32_t out_every, int32_t n_fields,
+                    const double *f_fine, const double *g, const double *u0_coarse, const double *v0_coarse,
+                    double *u_out, double *v_out, double *energy_out, int32_t max_steps, double tolerance,
+                    double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  int rc = check_wave_call(ctx, beta, dt, n_steps, out_every, n_fields, f_fine, g, 1, u_out, max_steps, tolerance,
+                           reduction);
+  if (rc) return rc;
+  NEED_DEVICE();
+  return wave_coarse(ctx, "slod_wave_solve", false, 1, beta, dt, n_steps, out_every, n_fields, f_fine, g, u0_coarse,
+                     v0_coarse, u_out, v_out, energy_out, max_steps, tolerance, reduction, cg_steps);
+}
+
+int slod_wave_solve_batch(slod_ctx *ctx, int32_t n_rhs, double beta, double dt, int32_t n_steps, int32_t out_every,
+                          int32_t n_fields, const double *f_fine, const double *g, const double *u0_coarse,
+                          const double *v0_coarse, double *u_out, double *v_out, double *energy_out,
+                          int32_t max_steps, double tolerance, double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  int rc = check_n_rhs(ctx, n_rhs);
+  if (rc) return rc;
+  rc = check_wave_call(ctx, beta, dt, n_steps, out_every, n_fields, f_fine, g, (size_t)n_rhs, u_out, max_steps,
+                       tolerance, reduction);
+  if (rc) return rc;
+  NEED_DEVICE();
+  return wave_coarse(ctx, "slod_wave_solve_batch", true, n_rhs, beta, dt, n_steps, out_every, n_fields, f_fine, g,
+                     u0_coarse, v0_coarse, u_out, v_out, energy_out, max_steps, tolerance, reduction, cg_steps);
+}
+
+int slod_fem_wave_solve(slod_ctx *ctx, double beta, double dt, int32_t n_steps, int32_t out_every, int32_t n_fields,
+                        const double *f_fine, const double *g, const double *u0_fine, const double *v0_fine,
+                        double *u_out, double *v_out, double *energy_out, int32_t max_steps, double tolerance,
+                        double reduction, int32_t *cg_steps) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  int rc = check_wave_call(ctx, beta, dt, n_steps, out_every, n_fields, f_fine, g, 1, u_out, max_steps, tolerance,
+                           reduction);
+  if (rc) return rc;
+  NEED_DEVICE();
+  return fem_wave(ctx, beta, dt, n_steps, out_every, n_fields, f_fine, g, u0_fine, v0_fine, u_out, v_out, energy_out,
+                  max_steps, tolerance, reduction, cg_steps);
+}
+
 // ---- checkpoint: parameters + phi + A*phi (+ block-ELL coarse matrix) --------------------------------------------
 namespace {
 struct StateHeader {

@@ -1224,6 +1224,7 @@ cudaError_t launch_gather(cudaStream_t st, const double *src, const long long *p
 #include "online.cuh"
 #include "online_batch.cuh"
 #include "heat.cuh"
+#include "wave.cuh"
 namespace slod {
 
 cudaError_t launch_coarse_rhs(cudaStream_t st, int n_patches, int s, const double *phi, const double *f, double *b,
@@ -1396,6 +1397,23 @@ cudaError_t launch_fine_apply(cudaStream_t st, int op, double tau, long long n_n
                               const double *x, double *y) {
   const int nb = (int)((n_nodes + kCgThreads - 1) / kCgThreads);
   k_fine_apply<<<nb, kCgThreads, 0, st>>>(op, tau, n_nodes, d_coef, x, y, nullptr, nullptr, nullptr);
+  return cudaGetLastError();
+}
+
+// ---- wave equation: Newmark time stepping (wave.cuh) ----
+cudaError_t launch_newmark_update(cudaStream_t st, long long n, bool first, double beta, double dt, double *u, double *v,
+                                  double *a, const double *a_new, double *ut) {
+  const long long blocks = (n + 255) / 256;
+  k_newmark_update<<<(int)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, st>>>(n, first ? 1 : 0, beta, dt, u, v, a,
+                                                                                 a_new, ut);
+  return cudaGetLastError();
+}
+size_t wave_energy_workspace_doubles(int nrows) { return (size_t)kBatch * cg_multi_apply_blocks(nrows); }
+cudaError_t launch_wave_energy(cudaStream_t st, int nrows, int kb, const double *Kell, const double *Mell,
+                               const double *U, const double *V, double *partial, double *E) {
+  const int nb = cg_multi_apply_blocks(nrows);
+  k_wave_energy<<<nb, kCgThreads, 0, st>>>(nrows, kb, Kell, Mell, U, V, partial);
+  k_wave_energy_sum<<<1, kCgThreads, 0, st>>>(kb, partial, nb, E);
   return cudaGetLastError();
 }
 

@@ -187,6 +187,16 @@ cudaError_t launch_lincomb(cudaStream_t st, long long n, double a, const double 
 // y = Op x for a FineOp (tau: kFineHeatDirichlet), no reduction
 cudaError_t launch_fine_apply(cudaStream_t st, int op, double tau, long long n_nodes, const double *d_coef,
                               const double *x, double *y);
+// wave equation on the SLOD space (wave.cuh)
+// Newmark corrector u = ut + beta dt^2 a_new, v += dt/2 (a + a_new), a = a_new, then the next predictor
+// ut = u + dt v + (1/2 - beta) dt^2 a, element-wise over n values (first: the predictor alone, a_new unread)
+cudaError_t launch_newmark_update(cudaStream_t st, long long n, bool first, double beta, double dt, double *u, double *v,
+                                  double *a, const double *a_new, double *ut);
+// E[j] = 1/2 (V_j^T M V_j + U_j^T K U_j) on the block-ELL matrices for kb <= kBatch interleaved columns (kb = 1: plain
+// vectors); partial: wave_energy_workspace_doubles(nrows) device doubles
+size_t wave_energy_workspace_doubles(int nrows);
+cudaError_t launch_wave_energy(cudaStream_t st, int nrows, int kb, const double *Kell, const double *Mell,
+                               const double *U, const double *V, double *partial, double *E);
 cudaError_t launch_fine_quadratic_form(cudaStream_t st, int op, long long n_nodes, const double *d_coef, const double *x,
                                        double *partial, int *n_partial);
 cudaError_t launch_fine_norms_reference(cudaStream_t st, long long n_cells, int nq, const double *gauss_x,

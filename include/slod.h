@@ -295,6 +295,43 @@ int slod_fem_heat_theta_solve(slod_ctx *ctx, double theta, double dt, int32_t n_
                               const double *u0_fine, double *u_out, int32_t max_steps, double tolerance,
                               double reduction, int32_t *cg_steps);
 
+/* The wave equation M_H u'' + K u = C^T f(t) on the SLOD space, Newmark time stepping with gamma = 1/2 and beta in
+ * [0, 1/2] (0: the explicit central-difference scheme, 1/4: average acceleration, unconditionally stable and energy
+ * conserving).  Time points t_k = k dt; the forcing f_fine, g, n_fields is that of slod_heat_theta_solve, step k uses
+ * g(t_k).  Each step solves for the acceleration, from zero, with the stopping rule of slod_coarse_solve:
+ *   start       M_H a_0 = b(t_0) - K u_0
+ *   step k      ut = u_{k-1} + dt v_{k-1} + (1/2 - beta) dt^2 a_{k-1},  (M_H + beta dt^2 K) a_k = b(t_k) - K ut,
+ *               u_k = ut + beta dt^2 a_k,  v_k = v_{k-1} + dt/2 (a_{k-1} + a_k)
+ * The explicit scheme is stable for dt^2 lambda_max(M_H^-1 K) <= 4 (for beta < 1/4: <= 4 / (1 - 4 beta)); the SLOD
+ * space holds no fine-scale modes, so that step is set by the coarse mesh, not by the fine one.
+ * u0_coarse, v0_coarse NULL: zero.  u_out [n_out][n_coarse] with n_out = n_steps / out_every, output o the state at step
+ * (o + 1) out_every; v_out (NULL: not written) the same for v; energy_out [n_out + 1] (NULL: not computed) the energy
+ * E = 1/2 v^T M_H v + 1/2 u^T K u at t_0 and at the outputs; cg_steps [n_steps + 1], entry 0 the start solve.
+ * M_H + beta dt^2 K is formed in the cache of the heat calls (beta = 0 solves with M_H itself).
+ * Every argument is checked before the device and the call order: beta outside [0, 1/2] or NaN, n_fields < 1 with fields
+ * given, a non-finite entry of g (read only with fields given) and the checks of slod_heat_solve -> SLOD_ERR_INVALID.
+ * Then SLOD_ERR_CUDA (maps-only handle), SLOD_ERR_STATE (slod_assemble_coarse / slod_assemble_coarse_mass have not run)
+ * and SLOD_ERR_NUMERIC when an acceleration solve fails, naming the step (0: the start solve) and the column; the outputs
+ * of the earlier steps are written.
+ * slod_wave_solve_batch: f_fine [n_rhs][n_fields][n_fine], g [n_rhs][n_steps + 1][n_fields], u0 / v0 [n_rhs][n_coarse],
+ * u_out / v_out [n_out][n_rhs][n_coarse], energy_out [n_out + 1][n_rhs], cg_steps [n_steps + 1][n_rhs]; a column is bit
+ * for bit the same whatever n_rhs, its position and its neighbours, and agrees with slod_wave_solve to the tolerance.
+ * slod_fem_wave_solve: the fine-scale reference of the same scheme (M_h + beta dt^2 A_h, homogeneous Dirichlet rows; the
+ * boundary rows of the fields, u0 and v0 are ignored), fine u0 / v0 / u_out / v_out, energy 1/2 v^T M_h v + 1/2 u^T A_h u.
+ * Needs only the coefficient. */
+int slod_wave_solve(slod_ctx *ctx, double beta, double dt, int32_t n_steps, int32_t out_every, int32_t n_fields,
+                    const double *f_fine, const double *g, const double *u0_coarse, const double *v0_coarse,
+                    double *u_out, double *v_out, double *energy_out, int32_t max_steps, double tolerance,
+                    double reduction, int32_t *cg_steps);
+int slod_wave_solve_batch(slod_ctx *ctx, int32_t n_rhs, double beta, double dt, int32_t n_steps, int32_t out_every,
+                          int32_t n_fields, const double *f_fine, const double *g, const double *u0_coarse,
+                          const double *v0_coarse, double *u_out, double *v_out, double *energy_out,
+                          int32_t max_steps, double tolerance, double reduction, int32_t *cg_steps);
+int slod_fem_wave_solve(slod_ctx *ctx, double beta, double dt, int32_t n_steps, int32_t out_every, int32_t n_fields,
+                        const double *f_fine, const double *g, const double *u0_fine, const double *v0_fine,
+                        double *u_out, double *v_out, double *energy_out, int32_t max_steps, double tolerance,
+                        double reduction, int32_t *cg_steps);
+
 /* ---- checkpoint of the offline phase (SURVEY 8f row 4; the reference has none: it recomputes every run) ----------
  * slod_save_state writes the parameters, the basis (phi, A*phi) and, if assembled, the coarse matrix to one binary
  * file; slod_load_state restores them into a handle created with the SAME parameters (else SLOD_ERR_INVALID), after
