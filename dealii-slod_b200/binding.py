@@ -33,7 +33,7 @@ EXPORTS = [
     "slod_prolongate_batch", "slod_assemble_coarse_mass", "slod_get_coarse_mass_csr", "slod_l2_project_batch",
     "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan", "slod_debug_select",
     "slod_update_basis", "slod_heat_theta_solve", "slod_heat_theta_solve_batch", "slod_fem_heat_theta_solve",
-    "slod_wave_solve", "slod_wave_solve_batch", "slod_fem_wave_solve",
+    "slod_wave_solve", "slod_wave_solve_batch", "slod_fem_wave_solve", "slod_debug_patch_stages_list",
 ]
 # slod_get_plan entries, in order
 PLAN_KEYS = ["mma_variant", "split_solver", "dense_ntile", "gmem_window", "dense_coef_gmem", "coarse_blocked", "use_ql",
@@ -114,6 +114,7 @@ def load_library(path=None):
     lib.slod_get_coarse_csr.argtypes = [vp, P(i64), P(i64), P(dbl), P(i64), P(i64)]
     lib.slod_get_patch_diagnostics.argtypes = [vp, i64, C.c_int, P(dbl)]
     lib.slod_debug_patch_stages.argtypes = [vp, i64, P(dbl), P(dbl), P(dbl)]
+    lib.slod_debug_patch_stages_list.argtypes = [vp, i64, P(i64), P(dbl), P(dbl), P(dbl)]
     lib.slod_debug_select.argtypes = [vp, i64, P(i64), P(dbl), P(dbl), P(dbl), P(dbl)]
     lib.slod_get_timings.argtypes = [vp, P(dbl), C.c_int]
     lib.slod_compute_basis_device.argtypes = [vp, i64, i64, vp, vp, vp]
@@ -653,6 +654,29 @@ class SlodContext:
         G = np.empty((ncd, ncd)) if want_G else None
         self._ck(self.lib.slod_debug_patch_stages(self.h, patch, _dp(X), _dp(Minv), _dp(G) if want_G else None))
         return X, Minv, G
+
+    def debug_stages_list(self, patches, want_G=True):
+        """debug_stages for a list of distinct patches in one work list (slod_debug_patch_stages_list).  Returns three
+        lists in the order of `patches`: X (n_internal, n_coarse), Minv and G (n_coarse, n_coarse); G holds None for
+        LOD-branch patches and everywhere when want_G is False."""
+        ids = np.ascontiguousarray(patches, dtype=np.int64).ravel()
+        info = [self.patch_info(int(p)) for p in ids]
+        ni = [i["n_internal"] for i in info]
+        ncd = [i["n_coarse"] for i in info]
+        xoff = np.concatenate([[0], np.cumsum([a * b for a, b in zip(ni, ncd)])]).astype(int)
+        moff = np.concatenate([[0], np.cumsum([k * k for k in ncd])]).astype(int)
+        X, Minv = np.empty(max(1, xoff[-1])), np.empty(max(1, moff[-1]))
+        G = np.empty(max(1, moff[-1])) if want_G else None
+        self._ck(self.lib.slod_debug_patch_stages_list(self.h, ids.size, ids.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                       _dp(X), _dp(Minv), _dp(G) if want_G else None))
+        Xs = [X[xoff[i]:xoff[i + 1]].reshape(ni[i], ncd[i]) for i in range(ids.size)]
+        Ms = [Minv[moff[i]:moff[i + 1]].reshape(ncd[i], ncd[i]) for i in range(ids.size)]
+        # the SLOD branch (source/LOD.cc:563-564): stabilised, oversampling > 0, the patch is not the whole domain
+        n_cells = (2 ** self.par.n_global_refinements) ** self.dim
+        slod = [want_G and bool(self.par.stabilize) and self.par.oversampling > 0 and i["n_cells"] != n_cells
+                for i in info]
+        Gs = [G[moff[i]:moff[i + 1]].reshape(ncd[i], ncd[i]) if slod[i] else None for i in range(ids.size)]
+        return Xs, Ms, Gs
 
     def debug_select(self, patches, G, Minv):
         """The selection stage on caller matrices (slod_debug_select).  patches: distinct ids; G, Minv: one

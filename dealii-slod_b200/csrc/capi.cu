@@ -595,37 +595,52 @@ int ensure_workspace(slod_ctx *ctx, int64_t n_range) {
 
 // The solve and dense stages of the n_work patches of the device list `ids`, with the kernels the plan chose: split
 // factor + triangular solve, tensor-core or SIMT solver; then flux + tensor-core dense, or SIMT dense.  wc: the work
-// counter of the persistent kernels (nullptr: static distribution).  Optional events: ev_factor behind the factor kernel
-// of the split solver, ev_solved between the two stages.
-int launch_patch_stages(slod_ctx *ctx, const int *ids, int nw, int *wc, cudaStream_t st, cudaEvent_t ev_factor,
-                        cudaEvent_t ev_solved) {
+// counter of the persistent kernels (nullptr: static distribution).  diag / status: the per-patch diagnostics and status
+// words the kernels write (indexed by patch id).  Optional events: ev_factor behind the factor kernel of the split
+// solver, ev_solved between the two stages.
+int launch_patch_stages(slod_ctx *ctx, const int *ids, int nw, int *wc, cudaStream_t st, double *diag, int *status,
+                        cudaEvent_t ev_factor, cudaEvent_t ev_solved) {
   if (ctx->split_solver) {
     static const int factor_grid_env = getenv("SLOD_FACTOR_GRID") ? atoi(getenv("SLOD_FACTOR_GRID")) : 0;   // experiments
     CK(launch_patch_factor(std::min(nw, factor_grid_env > 0 ? factor_grid_env : 2 * ctx->n_sm), ctx->smem_factor, st, ids, nw, ctx->d_coef, ctx->d_Lrec,
-                           ctx->d_stw, ctx->d_status, ctx->sl.coef_doubles, ctx->mma_nip, ctx->sl.ldx, ctx->sl.x_stride, wc));
+                           ctx->d_stw, status, ctx->sl.coef_doubles, ctx->mma_nip, ctx->sl.ldx, ctx->sl.x_stride, wc));
     if (ev_factor) CK(cudaEventRecord(ev_factor, st));
     CK(launch_patch_trisolve(std::min(nw, ctx->n_sm), ctx->smem_tri, st, ids, nw, ctx->d_Lrec, ctx->d_X,
                              ctx->sl.coef_doubles, ctx->mma_nip, ctx->sl.ldx, ctx->sl.x_stride, wc));
   } else if (ctx->mma_variant >= 0)
     CK(launch_patch_solve_mma(ctx->mma_variant, std::min(nw, ctx->grid_solve), ctx->smem_solve, st, ids, nw,
-                              ctx->d_coef, ctx->d_X, ctx->d_Lws, ctx->d_status, ctx->sl.coef_doubles, ctx->sl.ldx,
+                              ctx->d_coef, ctx->d_X, ctx->d_Lws, status, ctx->sl.coef_doubles, ctx->sl.ldx,
                               ctx->sl.x_stride, ctx->mma_lws_per_cta, ctx->mma_nip, ctx->mma_stw, wc));
   else
     CK(launch_patch_solve(std::min(nw, ctx->grid_solve), ctx->smem_solve, st, ids, nw, ctx->d_coef, ctx->d_X,
-                          ctx->d_Lws, ctx->d_status, ctx->sl));
+                          ctx->d_Lws, status, ctx->sl));
   if (ev_solved) CK(cudaEventRecord(ev_solved, st));
   if (ctx->dense_ntile) {
     CK(launch_patch_flux(std::min(nw, ctx->grid_flux), ctx->smem_flux, st, ids, nw, ctx->d_coef, ctx->d_X,
                          ctx->d_W, ctx->xl, wc));
     CK(launch_patch_dense_mma(ctx->dense_ntile, std::min(nw, ctx->grid_dense), ctx->smem_dense, st, ids, nw,
-                              ctx->d_coef, ctx->d_X, ctx->d_W, ctx->d_Minv, ctx->d_G, ctx->d_diag, ctx->d_status,
-                              ctx->dl, wc));
+                              ctx->d_coef, ctx->d_X, ctx->d_W, ctx->d_Minv, ctx->d_G, diag, status, ctx->dl, wc));
   }
   else
     CK(launch_patch_dense(std::min(nw, ctx->grid_dense), ctx->smem_dense, st, ids, nw, ctx->d_coef, ctx->d_X,
-                          ctx->d_Minv, ctx->d_G, ctx->d_diag, ctx->d_status, ctx->dl));
+                          ctx->d_Minv, ctx->d_G, diag, status, ctx->dl));
   ctx->launches += (ctx->split_solver ? 2 : 1) + (ctx->dense_ntile ? 2 : 1);
   return SLOD_OK;
+}
+
+// Work order of the patch kernels: largest patches first (stable, so equal costs keep the given order).
+std::vector<int> cost_order(const Params &P, const std::vector<int> &order) {
+  std::vector<long long> cost(order.size());
+  for (size_t i = 0; i < order.size(); ++i) {
+    const Geom g = make_geom(P, order[i]);
+    cost[i] = (long long)g.Ni * g.bw * (g.bw + 4LL * g.Ncd) + (long long)g.Ncd * g.Ncd * g.Ncd * 8;
+  }
+  std::vector<int> perm(order.size());
+  std::iota(perm.begin(), perm.end(), 0);
+  std::stable_sort(perm.begin(), perm.end(), [&](int a, int b) { return cost[a] > cost[b]; });
+  std::vector<int> out(order.size());
+  for (size_t i = 0; i < perm.size(); ++i) out[i] = order[perm[i]];
+  return out;
 }
 
 // Enqueues stages assembly .. premultiply for the patches [p0, p1) on `st` and returns without waiting: the work list
@@ -649,16 +664,7 @@ int run_basis(slod_ctx *ctx, int64_t p0, int64_t p1, double *d_phi, double *d_ap
   if (list || ctx->ids_p0 != p0 || ctx->ids_p1 != p1) {
     std::vector<int> order = list ? *list : std::vector<int>((size_t)(p1 - p0));
     if (!list) std::iota(order.begin(), order.end(), (int)p0);
-    std::vector<long long> cost(order.size());
-    for (size_t i = 0; i < order.size(); ++i) {
-      const Geom g = make_geom(P, order[i]);
-      cost[i] = (long long)g.Ni * g.bw * (g.bw + 4LL * g.Ncd) + (long long)g.Ncd * g.Ncd * g.Ncd * 8;
-    }
-    std::vector<int> perm(order.size());
-    std::iota(perm.begin(), perm.end(), 0);
-    std::stable_sort(perm.begin(), perm.end(), [&](int a, int b) { return cost[a] > cost[b]; });
-    ctx->ids.resize(order.size());
-    for (size_t i = 0; i < perm.size(); ++i) ctx->ids[i] = order[perm[i]];
+    ctx->ids = cost_order(P, order);
     CK(cudaMemcpyAsync(ctx->d_ids, ctx->ids.data(), sizeof(int) * ctx->ids.size(), cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));   // pageable source: the vector may be rebuilt by the next call
     ctx->ids_p0 = list ? -1 : p0;
@@ -682,7 +688,8 @@ int run_basis(slod_ctx *ctx, int64_t p0, int64_t p1, double *d_phi, double *d_ap
     const int *ids = ctx->d_ids + off;
     cudaEvent_t *ev = ctx->chunk_ev.data() + 5 * ci;
     CK(cudaEventRecord(ev[0], st));
-    rc = launch_patch_stages(ctx, ids, nw, wc, st, ci == 0 ? ctx->ev_split : nullptr, ev[1]);
+    rc = launch_patch_stages(ctx, ids, nw, wc, st, ctx->d_diag, ctx->d_status, ci == 0 ? ctx->ev_split : nullptr,
+                             ev[1]);
     if (rc) return rc;
     CK(cudaEventRecord(ev[2], st));
     int nl = 0;
@@ -3211,32 +3218,13 @@ static std::vector<int> internal_columns(const slod_ctx *ctx, const Geom &g) {
   return zpos;
 }
 
-int slod_debug_patch_stages(slod_ctx *ctx, int64_t patch, double *X, double *Minv, double *G) {
-  int rc = check_patch(ctx, patch);
-  if (rc) return rc;
-  NEED_DEVICE();
-  CK(cudaSetDevice(ctx->device));
-  rc = prepare_coefficients(ctx);
-  if (rc) return rc;
-  rc = wait_basis(ctx);   // the workspace of an enqueued range is about to be reused
-  if (rc) return rc;
-  rc = ensure_workspace(ctx, 1);
-  if (rc) return rc;
-  BIND_PARAMS((cudaStream_t)0);
-  ctx->ids_p0 = ctx->ids_p1 = -1;   // the device work list is overwritten below
-  const int id = (int)patch;
-  CK(cudaMemcpy(ctx->d_ids, &id, sizeof(int), cudaMemcpyHostToDevice));
-  rc = launch_patch_stages(ctx, ctx->d_ids, 1, nullptr, 0, nullptr, nullptr);
-  if (rc) return rc;
-  CK(cudaDeviceSynchronize());
-  const Geom g = make_geom(ctx->P, id);
-  if (X) CK(cudaMemcpy2D(X, sizeof(double) * g.Ncd, ctx->d_X, sizeof(double) * ctx->sl.ldx, sizeof(double) * g.Ncd, g.Ni,
-                         cudaMemcpyDeviceToHost));
-  if (Minv) CK(cudaMemcpy(Minv, ctx->d_Minv, sizeof(double) * g.Ncd * g.Ncd, cudaMemcpyDeviceToHost));
-  if (G) {
-    if (!g.slod) return fail(ctx, SLOD_ERR_STATE, "patch takes the LOD branch: no Gram matrix");
-    CK(cudaMemcpy(G, ctx->d_G, sizeof(double) * g.Ncd * g.Ncd, cudaMemcpyDeviceToHost));
-  }
+// X, Minv and G of the patch in workspace slot w to host memory (any may be NULL), in the reference column order
+static int copy_stages_out(slod_ctx *ctx, const Geom &g, int w, double *X, double *Minv, double *G) {
+  const size_t ms = ctx->dl.m_stride;
+  if (X) CK(cudaMemcpy2D(X, sizeof(double) * g.Ncd, ctx->d_X + (size_t)w * ctx->sl.x_stride, sizeof(double) * ctx->sl.ldx,
+                         sizeof(double) * g.Ncd, g.Ni, cudaMemcpyDeviceToHost));
+  if (Minv) CK(cudaMemcpy(Minv, ctx->d_Minv + w * ms, sizeof(double) * g.Ncd * g.Ncd, cudaMemcpyDeviceToHost));
+  if (G) CK(cudaMemcpy(G, ctx->d_G + w * ms, sizeof(double) * g.Ncd * g.Ncd, cudaMemcpyDeviceToHost));
   if (ctx->split_solver) {
     const std::vector<int> zpos = internal_columns(ctx, g);   // back to the reference order
     std::vector<double> tmp;
@@ -3253,6 +3241,98 @@ int slod_debug_patch_stages(slod_ctx *ctx, int64_t patch, double *X, double *Min
       }
   }
   return SLOD_OK;
+}
+
+int slod_debug_patch_stages(slod_ctx *ctx, int64_t patch, double *X, double *Minv, double *G) {
+  int rc = check_patch(ctx, patch);
+  if (rc) return rc;
+  NEED_DEVICE();
+  CK(cudaSetDevice(ctx->device));
+  rc = prepare_coefficients(ctx);
+  if (rc) return rc;
+  rc = wait_basis(ctx);   // the workspace of an enqueued range is about to be reused
+  if (rc) return rc;
+  rc = ensure_workspace(ctx, 1);
+  if (rc) return rc;
+  BIND_PARAMS((cudaStream_t)0);
+  ctx->ids_p0 = ctx->ids_p1 = -1;   // the device work list is overwritten below
+  const int id = (int)patch;
+  CK(cudaMemcpy(ctx->d_ids, &id, sizeof(int), cudaMemcpyHostToDevice));
+  rc = launch_patch_stages(ctx, ctx->d_ids, 1, nullptr, 0, ctx->d_diag, ctx->d_status, nullptr, nullptr);
+  if (rc) return rc;
+  CK(cudaDeviceSynchronize());
+  const Geom g = make_geom(ctx->P, id);
+  if (G && !g.slod) return fail(ctx, SLOD_ERR_STATE, "patch takes the LOD branch: no Gram matrix");
+  return copy_stages_out(ctx, g, 0, X, Minv, G);
+}
+
+int slod_debug_patch_stages_list(slod_ctx *ctx, int64_t n, const int64_t *patches, double *X, double *Minv, double *G) {
+  if (!ctx) return SLOD_ERR_INVALID;
+  if (n < 0 || (n > 0 && (!patches || !X || !Minv))) return fail(ctx, SLOD_ERR_INVALID, "bad argument");
+  const Params &P = ctx->P;
+  // host checks first: nothing is launched on an invalid list
+  std::vector<int64_t> xoff((size_t)n + 1, 0), moff((size_t)n + 1, 0);   // offsets of the packed X / square blocks
+  std::vector<int> slot_of((size_t)ctx->n_patches, -1);                   // position of a patch id in `patches`
+  for (int64_t i = 0; i < n; ++i) {
+    const int64_t p = patches[i];
+    if (p < 0 || p >= ctx->n_patches) return fail(ctx, SLOD_ERR_INVALID, "patch id out of range");
+    if (slot_of[(size_t)p] >= 0) return fail(ctx, SLOD_ERR_INVALID, "repeated patch id " + std::to_string(p));
+    slot_of[(size_t)p] = (int)i;
+    const Geom g = make_geom(P, (int)p);
+    xoff[i + 1] = xoff[i] + (int64_t)g.Ni * g.Ncd;
+    moff[i + 1] = moff[i] + (int64_t)g.Ncd * g.Ncd;
+  }
+  NEED_DEVICE();
+  if (n == 0) return SLOD_OK;
+  CK(cudaSetDevice(ctx->device));
+  int rc = prepare_coefficients(ctx);
+  if (rc) return rc;
+  rc = wait_basis(ctx);   // the workspace of an enqueued range is about to be reused
+  if (rc) return rc;
+  rc = ensure_workspace(ctx, n);
+  if (rc) return rc;
+  BIND_PARAMS((cudaStream_t)0);
+  ctx->ids_p0 = ctx->ids_p1 = -1;   // the device work list is overwritten below
+  const std::vector<int> order = cost_order(P, std::vector<int>(patches, patches + n));
+  // diagnostics and status words go to scratch copies (indexed by patch id): the handle's own arrays stay untouched
+  const size_t n_diag = (size_t)8 * P.s * ctx->n_patches;
+  double *d_dg = nullptr;
+  int *d_st = nullptr;
+  auto body = [&]() -> int {
+    CK(cudaMalloc(&d_dg, sizeof(double) * n_diag));
+    CK(cudaMalloc(&d_st, sizeof(int) * (size_t)ctx->n_patches));
+    CK(cudaMemset(d_st, 0, sizeof(int) * (size_t)ctx->n_patches));
+    CK(cudaMemcpy(ctx->d_ids, order.data(), sizeof(int) * order.size(), cudaMemcpyHostToDevice));
+    std::vector<int> st((size_t)ctx->n_patches);
+    for (int64_t i0 = 0; i0 < n; i0 += ctx->chunk) {
+      const int nc = (int)std::min<int64_t>(ctx->chunk, n - i0);
+      rc = launch_patch_stages(ctx, ctx->d_ids + i0, nc, ctx->d_work_counter, 0, d_dg, d_st, nullptr, nullptr);
+      if (rc) return rc;
+      CK(cudaDeviceSynchronize());
+      for (int w = 0; w < nc; ++w) {
+        const int id = order[(size_t)(i0 + w)];
+        const int64_t i = slot_of[(size_t)id];
+        const Geom g = make_geom(P, id);
+        double *Gi = G ? G + moff[i] : nullptr;
+        if (Gi && !g.slod) {   // LOD branch: no Gram matrix
+          std::fill(Gi, Gi + (size_t)g.Ncd * g.Ncd, 0.0);
+          Gi = nullptr;
+        }
+        rc = copy_stages_out(ctx, g, w, X + xoff[i], Minv + moff[i], Gi);
+        if (rc) return rc;
+      }
+    }
+    CK(cudaMemcpy(st.data(), d_st, sizeof(int) * st.size(), cudaMemcpyDeviceToHost));
+    for (int64_t i = 0; i < n; ++i)
+      if (st[(size_t)patches[i]])
+        return fail(ctx, SLOD_ERR_NUMERIC, "patch " + std::to_string(patches[i]) + ": numerical status bits " +
+                                               std::to_string(st[(size_t)patches[i]]));
+    return SLOD_OK;
+  };
+  rc = body();
+  if (d_dg) cudaFree(d_dg);
+  if (d_st) cudaFree(d_st);
+  return rc;
 }
 
 int slod_debug_select(slod_ctx *ctx, int64_t n, const int64_t *patches, const double *G, const double *Minv, double *c,

@@ -360,6 +360,14 @@ int slod_get_patch_diagnostics(const slod_ctx *ctx, int64_t patch, int comp, dou
 /* stage intermediates of one patch for staged parity tests (recomputed on demand for that patch):
  * X = A_ii^{-1} P_i  (n_internal x n_coarse, row-major), Minv (n_coarse^2), BD^T BD (n_coarse^2). Any may be NULL. */
 int slod_debug_patch_stages(slod_ctx *ctx, int64_t patch, double *X, double *Minv, double *G);
+/* the same stages for a list of patches, run as one work list in the cost order of slod_compute_basis (the persistent
+ * kernels go from one patch to the next as they do there); per patch the results equal slod_debug_patch_stages'.
+ *   patches: n distinct patch ids;
+ *   X: packed per patch, n_internal x n_coarse, row-major;  Minv, G: packed per patch, n_coarse^2 each, row-major;
+ *   reference column order.  G may be NULL; the blocks of LOD-branch patches (no Gram matrix) are set to 0.
+ * The handle's basis, coarse matrices, diagnostics and status words are left unchanged.  Repeated or out-of-range patch
+ * ids: SLOD_ERR_INVALID, before anything runs; a patch whose solve or dense stage sets status bits: SLOD_ERR_NUMERIC. */
+int slod_debug_patch_stages_list(slod_ctx *ctx, int64_t n, const int64_t *patches, double *X, double *Minv, double *G);
 /* the selection stage (source/LOD.cc:637-743) run exactly as slod_compute_basis runs it (same kernels, same plan:
  * SLOD_NO_FAST_SELECT, SLOD_FORCE_JACOBI and SLOD_EIG_CAP apply), on caller matrices, for selection tests.
  *   patches: n distinct patch ids (the patch fixes n_coarse and the LOD / SLOD branch);
