@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("SLOD_LIB") or os.path.join(_HERE, "libslod_b200.so") 
 SLOD_OK = 0
 ERRORS = {1: "SLOD_ERR_INVALID", 2: "SLOD_ERR_UNSUPPORTED", 3: "SLOD_ERR_CUDA", 4: "SLOD_ERR_STATE",
           5: "SLOD_ERR_NUMERIC"}
-PROBLEM_DIFFUSION, PROBLEM_ELASTICITY = 0, 1
+PROBLEM_DIFFUSION, PROBLEM_ELASTICITY, PROBLEM_DIFFUSION_TENSOR = 0, 1, 2
 
 # every symbol include/slod.h declares (tests check that the library exports all of them)
 EXPORTS = [
@@ -34,6 +34,7 @@ EXPORTS = [
     "slod_heat_solve", "slod_heat_solve_batch", "slod_fem_heat_solve", "slod_get_plan", "slod_debug_select",
     "slod_update_basis", "slod_heat_theta_solve", "slod_heat_theta_solve_batch", "slod_fem_heat_theta_solve",
     "slod_wave_solve", "slod_wave_solve_batch", "slod_fem_wave_solve", "slod_debug_patch_stages_list",
+    "slod_set_coefficient_tensor",
 ]
 # slod_get_plan entries, in order
 PLAN_KEYS = ["mma_variant", "split_solver", "dense_ntile", "gmem_window", "dense_coef_gmem", "coarse_blocked", "use_ql",
@@ -75,6 +76,7 @@ def load_library(path=None):
     lib.slod_last_error.restype = C.c_char_p
     lib.slod_last_create_error.restype = C.c_char_p
     lib.slod_set_coefficient.argtypes = [vp, C.c_int, C.c_int, P(dbl), C.c_size_t]
+    lib.slod_set_coefficient_tensor.argtypes = [vp, C.c_int, P(dbl), C.c_size_t]
     lib.slod_patch_count.argtypes = [vp, P(i64)]
     lib.slod_get_plan.argtypes = [vp, P(i32)]
     lib.slod_fine_size.argtypes = [vp, P(i64)]
@@ -240,6 +242,15 @@ class SlodContext:
     def set_coefficient(self, field, eta_refinement, values):
         v = np.ascontiguousarray(values, dtype=np.float64).ravel()
         self._ck(self.lib.slod_set_coefficient(self.h, field, eta_refinement, _dp(v), v.size))
+
+    def set_coefficient_tensor(self, eta_refinement, values):
+        """Tensor-diffusion coefficient: values (n_cells, dim (dim + 1) / 2), one symmetric tensor per cell in Voigt order
+        (2-D a_xx, a_yy, a_xy; 3-D a_xx, a_yy, a_zz, a_yz, a_xz, a_xy)."""
+        v = np.ascontiguousarray(values, dtype=np.float64)
+        ncomp = self.dim * (self.dim + 1) // 2
+        if v.ndim != 2 or v.shape[1] != ncomp:
+            raise ValueError(f"values must have shape (n_cells, {ncomp})")
+        self._ck(self.lib.slod_set_coefficient_tensor(self.h, eta_refinement, _dp(v), v.shape[0]))
 
     def plan(self):
         """The kernels slod_create chose (slod_get_plan): {key: int} over PLAN_KEYS."""

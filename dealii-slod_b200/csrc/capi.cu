@@ -37,10 +37,11 @@ struct slod_ctx {
   int device = 0;
   int n_sm = 148;
   int64_t n_patches = 0;
-  int n_fields = 1;
-  bool coef_set[2] = {false, false};
-  std::vector<double> coef_table[2];  // caller's cell-wise tables
-  int coef_r[2] = {0, 0};
+  int n_fields = 1;                   // 1 diffusion, 2 elasticity, dim (dim + 1) / 2 tensor diffusion
+  static constexpr int kMaxFields = 6;
+  bool coef_set[kMaxFields] = {};
+  std::vector<double> coef_table[kMaxFields];  // caller's cell-wise tables
+  int coef_r[kMaxFields] = {};
   bool coef_dirty = true;
   double *d_coef = nullptr;  // [n_fields][nsub^dim]
   size_t d_coef_elems = 0;
@@ -57,6 +58,8 @@ struct slod_ctx {
   int64_t ids_cap = 0;   // capacity of d_ids (patches of one range)
   int *d_ids = nullptr;
   double *d_X = nullptr, *d_Minv = nullptr, *d_G = nullptr, *d_cvec = nullptr, *d_Lws = nullptr, *d_W = nullptr, *d_coefws = nullptr;
+  double *d_coefws_finish = nullptr;
+  bool finish_coef_gmem = false;  // k_patch_finish keeps the patch coefficients in a global scratch (very large patches)
   FluxLayout xl{};
   size_t smem_flux = 0;
   int grid_flux = 0;
@@ -68,6 +71,7 @@ struct slod_ctx {
   int mma_nip = 0, mma_stw = 0;
   bool split_solver = false;      // factor + triangular-solve kernels instead of the fused solver (large 3-D patches)
   size_t smem_factor = 0, smem_tri = 0;
+  int split_coef_doubles = 0;     // coefficient window of k_patch_factor: one field
   double *d_Lrec = nullptr;       // factor records of a chunk
   double *d_stw = nullptr;        // per-CTA stencil scratch of k_patch_factor
   cudaEvent_t ev_split = nullptr;
@@ -282,6 +286,9 @@ int ipow(int b, int e) {
   return r;
 }
 
+// Voigt order of the tensor components: 2-D a_xx, a_yy, a_xy; 3-D a_xx, a_yy, a_zz, a_yz, a_xz, a_xy
+constexpr int kVoigt[2][6][2] = {{{0, 0}, {1, 1}, {0, 1}}, {{0, 0}, {1, 1}, {2, 2}, {1, 2}, {0, 2}, {0, 1}}};
+
 // Reference sub-cell matrices with the 2-point Gauss rule per axis (QIterated(QGauss<1>(2), n),
 // source/LOD.cc:91-92); local dof = s * (lx + 2 ly + 4 lz) + comp.
 void reference_matrices(Params &P) {
@@ -315,6 +322,14 @@ void reference_matrices(Params &P) {
           P.Kref[i * nl + j] += d * jxw;
           P.Kq[q][i * nl + j] = d * jxw;
         }
+    } else if (P.problem == SLOD_PROBLEM_DIFFUSION_TENSOR) {
+      // Kq[f]: the matrix of Voigt component f = (a, b), d_a phi_i d_b phi_j (+ d_b phi_i d_a phi_j for a != b)
+      for (int f = 0; f < tensor_fields(dim); ++f) {
+        const int a = kVoigt[dim - 2][f][0], b = kVoigt[dim - 2][f][1];
+        for (int i = 0; i < nn; ++i)
+          for (int j = 0; j < nn; ++j)
+            P.Kq[f][i * nl + j] += (a == b ? G[i][a] * G[j][a] : G[i][a] * G[j][b] + G[i][b] * G[j][a]) * jxw;
+      }
     } else {
       // 2 eps(phi_i):eps(phi_j) and div phi_i div phi_j   (include/Elasticity.h:236-250)
       for (int i = 0; i < nn; ++i)
@@ -503,8 +518,9 @@ void free_workspace(slod_ctx *c) {
     if (p) cudaFree(p);
     p = nullptr;
   };
-  F(c->d_counter); F(c->d_work_counter); F(c->d_ids); F(c->d_X); F(c->d_Minv); F(c->d_G); F(c->d_cvec); F(c->d_Lws); F(c->d_W); F(c->d_coefws);
+  F(c->d_counter); F(c->d_work_counter); F(c->d_ids); F(c->d_X); F(c->d_Minv); F(c->d_G); F(c->d_cvec); F(c->d_Lws); F(c->d_W); F(c->d_coefws); F(c->d_coefws_finish);
   c->dl.coef_ws = nullptr;
+  c->fl.coef_ws = nullptr;
   F(c->d_Lrec); F(c->d_stw);
   F(c->sb.eig_list); F(c->sb.jac_list); F(c->sb.H); F(c->sb.V); F(c->sb.rot_cs); F(c->sb.rot_i); F(c->sb.rot_n);
   c->chunk = 0;
@@ -549,6 +565,10 @@ int ensure_workspace(slod_ctx *ctx, int64_t n_range) {
     if (ctx->dense_coef_gmem) {
       CK(cudaMalloc(&ctx->d_coefws, sizeof(double) * (size_t)ctx->dl.coef_doubles * ctx->grid_dense));
       ctx->dl.coef_ws = ctx->d_coefws;
+    }
+    if (ctx->finish_coef_gmem) {
+      CK(cudaMalloc(&ctx->d_coefws_finish, sizeof(double) * (size_t)ctx->fl.coef_doubles * ctx->grid_finish));
+      ctx->fl.coef_ws = ctx->d_coefws_finish;
     }
     if (ctx->split_solver)
     {
@@ -603,7 +623,7 @@ int launch_patch_stages(slod_ctx *ctx, const int *ids, int nw, int *wc, cudaStre
   if (ctx->split_solver) {
     static const int factor_grid_env = getenv("SLOD_FACTOR_GRID") ? atoi(getenv("SLOD_FACTOR_GRID")) : 0;   // experiments
     CK(launch_patch_factor(std::min(nw, factor_grid_env > 0 ? factor_grid_env : 2 * ctx->n_sm), ctx->smem_factor, st, ids, nw, ctx->d_coef, ctx->d_Lrec,
-                           ctx->d_stw, status, ctx->sl.coef_doubles, ctx->mma_nip, ctx->sl.ldx, ctx->sl.x_stride, wc));
+                           ctx->d_stw, status, ctx->split_coef_doubles, ctx->mma_nip, ctx->sl.ldx, ctx->sl.x_stride, wc));
     if (ev_factor) CK(cudaEventRecord(ev_factor, st));
     CK(launch_patch_trisolve(std::min(nw, ctx->n_sm), ctx->smem_tri, st, ids, nw, ctx->d_Lrec, ctx->d_X,
                              ctx->sl.coef_doubles, ctx->mma_nip, ctx->sl.ldx, ctx->sl.x_stride, wc));
@@ -970,9 +990,12 @@ int slod_create(const slod_params *par, slod_ctx **out) {
   if (par->dim != 2 && par->dim != 3) return bad(SLOD_ERR_INVALID, "dim must be 2 or 3");
   if (par->problem == SLOD_PROBLEM_DIFFUSION && par->spacedim != 1)
     return bad(SLOD_ERR_INVALID, "diffusion needs spacedim 1");
+  if (par->problem == SLOD_PROBLEM_DIFFUSION_TENSOR && par->spacedim != 1)
+    return bad(SLOD_ERR_INVALID, "tensor diffusion needs spacedim 1");
   if (par->problem == SLOD_PROBLEM_ELASTICITY && (par->spacedim != par->dim || par->dim != 2))
     return bad(SLOD_ERR_UNSUPPORTED, "elasticity is implemented for dim = spacedim = 2 (as in the reference)");
-  if (par->problem != SLOD_PROBLEM_DIFFUSION && par->problem != SLOD_PROBLEM_ELASTICITY)
+  if (par->problem != SLOD_PROBLEM_DIFFUSION && par->problem != SLOD_PROBLEM_ELASTICITY &&
+      par->problem != SLOD_PROBLEM_DIFFUSION_TENSOR)
     return bad(SLOD_ERR_INVALID, "unknown problem");
   if (par->n_global_refinements < 0 || par->n_global_refinements * par->dim > 30)
     return bad(SLOD_ERR_INVALID, "n_global_refinements out of range");
@@ -1027,7 +1050,8 @@ int slod_create(const slod_params *par, slod_ctx **out) {
   P.has_presaved = 0;
   P.gauss_coef = 0;
   ctx->n_patches = (int64_t)ipow(P.N, P.dim);
-  ctx->n_fields = (P.problem == SLOD_PROBLEM_DIFFUSION) ? 1 : 2;
+  ctx->n_fields = (P.problem == SLOD_PROBLEM_DIFFUSION) ? 1
+                  : (P.problem == SLOD_PROBLEM_ELASTICITY) ? 2 : tensor_fields(P.dim);
   reference_matrices(P);
   // quirk B: the first full-size patch in patch-id order donates its matrix (source/LOD.cc:446-450)
   {
@@ -1075,8 +1099,10 @@ int slod_create(const slod_params *par, slod_ctx **out) {
   ctx->nb_max = nb_max;
   const bool big = (P.dim == 3);
   const int msub = P.n * mfull;
-  // room for one value per Gauss point (eta < h) where that is cheap (2-D); 3-D keeps one per sub-cell
-  const int coef_doubles = ctx->n_fields * ipow(msub, P.dim) * (P.dim == 2 ? 4 : 1);
+  // room for one value per Gauss point (eta < h) where that is cheap (2-D); 3-D and the tensor problem keep one per
+  // sub-cell
+  const int coef_doubles =
+      ctx->n_fields * ipow(msub, P.dim) * (P.dim == 2 && P.problem != SLOD_PROBLEM_DIFFUSION_TENSOR ? 4 : 1);
   // ---- layouts ----
   SolveLayout &sl = ctx->sl;
   sl.threads = big ? 512 : 128;
@@ -1092,9 +1118,22 @@ int slod_create(const slod_params *par, slod_ctx **out) {
   ctx->smem_solve = sizeof(double) * ((size_t)coef_doubles + (size_t)sl.R * sl.ldw + (size_t)sl.R * sl.ldr +
                                       (size_t)sl.R * kSolveNB + 2 * kSolveNB * kSolveNB + (size_t)kSolveNB * sl.ldr);
   sl.gmem_window = 0;
+  sl.gmem_coef = 0;
+  sl.gcoef_off = 0;
   sl.gwin_off = 0;
   const size_t smem_solve_small = sizeof(double) * ((size_t)coef_doubles + 2 * kSolveNB * kSolveNB + (size_t)kSolveNB * sl.ldr);
   const long long gwin_doubles = (long long)sl.R * sl.ldw + (long long)sl.R * sl.ldr + (long long)sl.R * kSolveNB;
+  // tiles of the tensor-core dense stage behind a solver whose X rows have leading dimension ldx (0: SIMT dense stage)
+  auto dense_tiles = [&](int variant, int ldx) {
+    const int nt_need = (P.NcdMax + 7) / 8;
+    int ntile = nt_need <= 4 ? 4 : (nt_need <= 8 ? 8 : (nt_need <= 16 ? 16 : 0));
+    if (getenv("SLOD_FORCE_SIMT_DENSE")) ntile = 0;
+    // the register/mma dense stage reads X rows with 16-byte loads: needs the padded layout of the mma solver
+    if (ntile && (variant < 0 || 8 * ntile != ldx)) ntile = 0;
+    if (ipow(P.n + 1, P.dim) > 27) ntile = 0;   // the gather table of M holds 27 local nodes per coarse cell
+    if (ntile && dense_mma_smem(ntile, coef_doubles, nb_max) > prop.sharedMemPerBlockOptin) ntile = 0;
+    return ntile;
+  };
   // tensor-core solver when the window (RB blocks of 8 rows) and the coarse columns (NW warps x 8) fit a variant
   {
     const int rb_need = (bw_max + 8 + 7) / 8, nw_need = (P.NcdMax + 7) / 8;
@@ -1103,9 +1142,16 @@ int slod_create(const slod_params *par, slod_ctx **out) {
     else if (rb_need <= 4 && nw_need <= 4) { variant = 1; rbmax = 4; nw = 4; }
     else if (rb_need <= 4 && nw_need <= 8) { variant = 2; rbmax = 4; nw = 8; }
     if (getenv("SLOD_FORCE_SIMT_SOLVER") || getenv("SLOD_FORCE_GMEM_SOLVER")) variant = -1;
-    // a variant whose shared-memory plan does not fit (large coefficient windows: many subdivisions) is no variant: the
-    // SIMT solver takes over, with its windows in global memory if need be
-    if (variant >= 0 && solve_mma_smem(variant, coef_doubles, ((P.NiMax + 7) / 8) * 8, P.s * ((P.dim == 3) ? 13 : 4) + P.s) >
+    // split factor + triangular-solve kernels for large 3-D scalar patches.  They keep their columns in z-major order,
+    // which only the tensor-core flux / dense kernels understand.  The factor kernel stages one coefficient field at a
+    // time (the tensor problem's components one after the other), so its window is one field whatever the problem.
+    const bool split = variant == 0 && P.dim == 3 && P.s == 1 &&
+                       (P.problem == SLOD_PROBLEM_DIFFUSION || P.problem == SLOD_PROBLEM_DIFFUSION_TENSOR) &&
+                       !getenv("SLOD_FUSED_SOLVER") && dense_tiles(variant, 8 * nw) > 0;
+    const int solve_coef = split ? coef_doubles / ctx->n_fields : coef_doubles;
+    // a variant whose shared-memory plan does not fit (large coefficient windows: many subdivisions or fields) is no
+    // variant: the SIMT solver takes over, with its windows in global memory if need be
+    if (variant >= 0 && solve_mma_smem(variant, solve_coef, ((P.NiMax + 7) / 8) * 8, P.s * ((P.dim == 3) ? 13 : 4) + P.s) >
                             prop.sharedMemPerBlockOptin)
       variant = -1;
     if (variant >= 0) {
@@ -1119,10 +1165,11 @@ int slod_create(const slod_params *par, slod_ctx **out) {
       sl.threads = ctx->mma_threads;
       ctx->mma_nip = nip;
       ctx->mma_stw = P.s * ((P.dim == 3) ? 13 : 4) + P.s;
-      ctx->smem_solve = solve_mma_smem(variant, coef_doubles, ctx->mma_nip, ctx->mma_stw);
-      if (variant == 0 && P.dim == 3 && P.s == 1 && P.problem == SLOD_PROBLEM_DIFFUSION && !getenv("SLOD_FUSED_SOLVER")) {
+      ctx->smem_solve = solve_mma_smem(variant, solve_coef, ctx->mma_nip, ctx->mma_stw);
+      if (split) {
         ctx->split_solver = true;
-        ctx->smem_factor = split_factor_smem(coef_doubles, nip);
+        ctx->split_coef_doubles = solve_coef;
+        ctx->smem_factor = split_factor_smem(solve_coef, nip);
         ctx->smem_tri = split_trisolve_smem(nip);
       }
     }
@@ -1133,6 +1180,14 @@ int slod_create(const slod_params *par, slod_ctx **out) {
     sl.gwin_off = sl.lws_per_cta;
     sl.lws_per_cta += gwin_doubles;
     ctx->smem_solve = smem_solve_small;
+    if (ctx->smem_solve > prop.sharedMemPerBlockOptin && P.problem == SLOD_PROBLEM_DIFFUSION_TENSOR) {
+      // the coefficient window does not fit either (the tensor problem's six fields on 3-D patches with 4 subdivisions):
+      // it goes to the CTA's slice of the workspace as well.  The other problems keep their envelope.
+      sl.gmem_coef = 1;
+      sl.gcoef_off = sl.lws_per_cta;
+      sl.lws_per_cta += coef_doubles;
+      ctx->smem_solve -= sizeof(double) * (size_t)coef_doubles;
+    }
   }
   DenseLayout &dl = ctx->dl;
   // the SIMT dense stage keeps kGEPT = 32 Gram entries per thread: 2-D patches with more than 64 coarse dofs need the
@@ -1144,21 +1199,10 @@ int slod_create(const slod_params *par, slod_ctx **out) {
   ctx->smem_dense = sizeof(double) * ((size_t)coef_doubles + (size_t)dl.m_stride + 2 * 16 * (size_t)P.NcdMax +
                                       2 * (size_t)P.NcdMax + 16 * 54) +
                     sizeof(int) * (16 * 54 + (size_t)nb_max + 8);
-  {
-    const int nt_need = (P.NcdMax + 7) / 8;
-    int ntile = nt_need <= 4 ? 4 : (nt_need <= 8 ? 8 : (nt_need <= 16 ? 16 : 0));
-    if (getenv("SLOD_FORCE_SIMT_DENSE")) ntile = 0;
-    // the register/mma dense stage reads X rows with 16-byte loads: needs the padded layout of the mma solver
-    if (ntile && (ctx->mma_variant < 0 || 8 * ntile != sl.ldx)) ntile = 0;
-    if (ipow(P.n + 1, P.dim) > 27) ntile = 0;   // the gather table of M holds 27 local nodes per coarse cell
-    if (ntile) {
-      const size_t sm = dense_mma_smem(ntile, coef_doubles, nb_max);
-      if (sm <= prop.sharedMemPerBlockOptin) {
-        ctx->dense_ntile = ntile;
-        ctx->smem_dense = sm;
-        dl.threads = 32 * ntile;
-      }
-    }
+  if (const int ntile = dense_tiles(ctx->mma_variant, sl.ldx)) {
+    ctx->dense_ntile = ntile;
+    ctx->smem_dense = dense_mma_smem(ntile, coef_doubles, nb_max);
+    dl.threads = 32 * ntile;
   }
   dl.coef_ws = nullptr;
   if (!ctx->dense_ntile && (ctx->smem_dense > prop.sharedMemPerBlockOptin || getenv("SLOD_FORCE_GMEM_SOLVER")) &&
@@ -1166,8 +1210,6 @@ int slod_create(const slod_params *par, slod_ctx **out) {
     ctx->dense_coef_gmem = true;   // the pointer is set when the workspace is allocated
     ctx->smem_dense -= sizeof(double) * (size_t)coef_doubles;
   }
-  // the split solver keeps its columns in z-major order, which only the tensor-core flux / dense kernels understand
-  if (ctx->split_solver && !ctx->dense_ntile) ctx->split_solver = false;
   if (ctx->dense_ntile) {
     FluxLayout &xl = ctx->xl;
     xl.coef_doubles = coef_doubles; xl.ldx = sl.ldx; xl.nb_max = nb_max; xl.x_stride = sl.x_stride;
@@ -1198,6 +1240,13 @@ int slod_create(const slod_params *par, slod_ctx **out) {
   fl.ell_width = P.ell_width;
   fl.coef_doubles = coef_doubles; fl.nf_max = P.NfMax; fl.ncd_max = P.NcdMax; fl.ldx = sl.ldx; fl.x_stride = sl.x_stride;
   ctx->smem_finish = sizeof(double) * ((size_t)coef_doubles + P.NfMax + P.NcdMax) + sizeof(int) * ((size_t)P.NiMax + 2);
+  fl.coef_ws = nullptr;
+  if (ctx->smem_finish > prop.sharedMemPerBlockOptin && P.problem == SLOD_PROBLEM_DIFFUSION_TENSOR) {
+    // as for the SIMT dense stage: the window in global memory (the tensor problem's six fields; the other problems
+    // keep their envelope)
+    ctx->finish_coef_gmem = true;   // the pointer is set when the workspace is allocated
+    ctx->smem_finish -= sizeof(double) * (size_t)coef_doubles;
+  }
   ctx->smem_coarse = sizeof(double) * ((size_t)P.s * P.NfMax);
   const size_t smem_cap = prop.sharedMemPerBlockOptin;
   {
@@ -1319,8 +1368,25 @@ void slod_destroy(slod_ctx *ctx) {
   delete ctx;
 }
 
+namespace {
+// field `field` of the handle := the n values cellwise[0], cellwise[stride], ...; prepare_coefficients expands it onto the
+// sub-cells before the next computation
+void store_coefficient(slod_ctx *ctx, int field, int eta_refinement, const double *cellwise, size_t n, size_t stride) {
+  std::vector<double> &tab = ctx->coef_table[field];
+  tab.resize(n);
+  for (size_t c = 0; c < n; ++c) tab[c] = cellwise[c * stride];
+  ctx->coef_r[field] = eta_refinement;
+  ctx->coef_set[field] = true;
+  ctx->coef_dirty = true;
+  ctx->basis_done = ctx->coarse_done = false;
+}
+}  // namespace
+
 int slod_set_coefficient(slod_ctx *ctx, int field, int eta_refinement, const double *cellwise, size_t n) {
   if (!ctx || !cellwise) return SLOD_ERR_INVALID;
+  if (ctx->P.problem == SLOD_PROBLEM_DIFFUSION_TENSOR)
+    return fail(ctx, SLOD_ERR_INVALID,
+                "a tensor-diffusion handle takes its coefficient as whole tensors: use slod_set_coefficient_tensor");
   NEED_DEVICE();
   const Params &P = ctx->P;
   if (field < 0 || field >= ctx->n_fields) return fail(ctx, SLOD_ERR_INVALID, "coefficient field index out of range");
@@ -1329,13 +1395,61 @@ int slod_set_coefficient(slod_ctx *ctx, int field, int eta_refinement, const dou
   size_t want = 1;
   for (int a = 0; a < P.dim; ++a) want <<= eta_refinement;
   if (want != n) return fail(ctx, SLOD_ERR_INVALID, "coefficient table size != (2^r)^dim");
-  ctx->coef_table[field].assign(cellwise, cellwise + n);
-  ctx->coef_r[field] = eta_refinement;
-  ctx->coef_set[field] = true;
-  ctx->coef_dirty = true;
-  ctx->basis_done = ctx->coarse_done = false;
+  store_coefficient(ctx, field, eta_refinement, cellwise, n, 1);
   for (slod_ctx *sub : ctx->subs) {
     const int rc = slod_set_coefficient(sub, field, eta_refinement, cellwise, n);
+    if (rc) return fail(ctx, rc, sub->err);
+  }
+  return SLOD_OK;
+}
+
+int slod_set_coefficient_tensor(slod_ctx *ctx, int eta_refinement, const double *cells, size_t n_cells) {
+  if (!ctx || !cells) return SLOD_ERR_INVALID;
+  const Params &P = ctx->P;
+  if (P.problem != SLOD_PROBLEM_DIFFUSION_TENSOR)
+    return fail(ctx, SLOD_ERR_INVALID, "slod_set_coefficient_tensor needs a SLOD_PROBLEM_DIFFUSION_TENSOR handle: use "
+                                       "slod_set_coefficient");
+  if (eta_refinement < 0 || eta_refinement * P.dim > 30)
+    return fail(ctx, SLOD_ERR_INVALID, "eta_refinement out of range ((2^r)^dim must stay below 2^31)");
+  size_t want = 1;
+  for (int a = 0; a < P.dim; ++a) want <<= eta_refinement;
+  if (want != n_cells) return fail(ctx, SLOD_ERR_INVALID, "n_cells != (2^eta_refinement)^dim");
+  const int nc = ctx->n_fields;
+  for (size_t c = 0; c < n_cells; ++c) {
+    const double *t = cells + c * nc;
+    for (int f = 0; f < nc; ++f)
+      if (!std::isfinite(t[f])) return fail(ctx, SLOD_ERR_INVALID, "tensor of cell " + std::to_string(c) + " is not finite");
+    // Cholesky with positive pivots of the symmetric tensor (Voigt order: the diagonal first)
+    double A[3][3];
+    for (int f = 0; f < nc; ++f) {
+      const int a = kVoigt[P.dim - 2][f][0], b = kVoigt[P.dim - 2][f][1];
+      A[a][b] = A[b][a] = t[f];
+    }
+    bool spd = true;
+    for (int j = 0; j < P.dim && spd; ++j) {
+      double d = A[j][j];
+      for (int k = 0; k < j; ++k) d -= A[j][k] * A[j][k];
+      if (!(d > 0.0)) {
+        spd = false;
+        break;
+      }
+      A[j][j] = std::sqrt(d);
+      for (int i = j + 1; i < P.dim; ++i) {
+        double v = A[i][j];
+        for (int k = 0; k < j; ++k) v -= A[i][k] * A[j][k];
+        A[i][j] = v / A[j][j];
+      }
+    }
+    if (!spd) return fail(ctx, SLOD_ERR_INVALID, "tensor of cell " + std::to_string(c) + " is not positive definite");
+  }
+  if ((1 << eta_refinement) > P.nsub)
+    return fail(ctx, SLOD_ERR_UNSUPPORTED, "a tensor table finer than the fine sub-cells (eta < h) is not supported: "
+                                           "the per-Gauss-point mode exists for scalar coefficients only");
+  NEED_DEVICE();
+  // each component is a cell-wise table of its own, expanded like a slod_set_coefficient field
+  for (int f = 0; f < nc; ++f) store_coefficient(ctx, f, eta_refinement, cells + f, n_cells, nc);
+  for (slod_ctx *sub : ctx->subs) {
+    const int rc = slod_set_coefficient_tensor(sub, eta_refinement, cells, n_cells);
     if (rc) return fail(ctx, rc, sub->err);
   }
   return SLOD_OK;

@@ -16,6 +16,10 @@
 namespace slod {
 
 constexpr int kMaxLocal = 8;  // (2^dim * spacedim) <= 8 : 2-D elasticity, 3-D diffusion
+constexpr int kProblemTensor = 2;   // SLOD_PROBLEM_DIFFUSION_TENSOR (include/slod.h)
+
+// coefficient fields of the tensor problem: the components of a symmetric dim x dim tensor in Voigt order
+SLOD_HD int tensor_fields(int dim) { return dim * (dim + 1) / 2; }
 
 struct Params {
   int dim, s, ref, n, ell, N;  // N = 2^ref coarse cells per axis
@@ -33,7 +37,8 @@ struct Params {
   double Kref[kMaxLocal * kMaxLocal];   // diffusion: Laplace * h^(d-2);  elasticity: 2 eps:eps
   double Klam[kMaxLocal * kMaxLocal];   // elasticity: div div
   // coefficient finer than the sub-cells (eta < h, e.g. tests/Poisson_LOD_Example): one value per Gauss
-  // point of QIterated(QGauss<1>(2), n) and the per-Gauss-point matrices (q = qx + 2 qy + 4 qz)
+  // point of QIterated(QGauss<1>(2), n) and the per-Gauss-point matrices (q = qx + 2 qy + 4 qz).
+  // Tensor problem (never per Gauss point): Kq[f] is the matrix of Voigt component f, whose coefficient is field f.
   int gauss_coef;
   double Kq[kMaxLocal][kMaxLocal * kMaxLocal];
   double Klamq[kMaxLocal][kMaxLocal * kMaxLocal];
@@ -201,6 +206,14 @@ SLOD_HD double proj_entry(const Params &P, const Geom &g, const int a[3], int ca
   return wgt;
 }
 
+// Entry idx of the tensor problem's matrix of sub-cell sc: the sum over the Voigt components
+template <typename CoefT>
+SLOD_HD double tensor_subcell_entry(const Params &P, const CoefT *coef, int nsubp, int sc, int idx) {
+  double acc = 0.0;
+  for (int f = 0; f < tensor_fields(P.dim); ++f) acc += (double)coef[f * nsubp + sc] * P.Kq[f][idx];
+  return acc;
+}
+
 // Entry of the unconstrained patch stiffness matrix between (node a, comp ca) and (node a+dl, comp cb)
 // (include/Diffusion.h:143-193 / include/Elasticity.h:211-284 summed over the sub-cells containing both
 // nodes).  `coef` holds the patch's sub-cell coefficients, field-major, x fastest.
@@ -228,7 +241,9 @@ SLOD_HD double stiff_entry(const Params &P, const Geom &g, const CoefT *coef, co
         const int la = (a[0] - ox) + 2 * (a[1] - oy) + ((P.dim == 3) ? 4 * (a[2] - oz) : 0);
         const int lb = (a[0] + dl[0] - ox) + 2 * (a[1] + dl[1] - oy) + ((P.dim == 3) ? 4 * (a[2] + dl[2] - oz) : 0);
         const int idx = (la * P.s + ca) * nl + (lb * P.s + cb);
-        if (!P.gauss_coef) {
+        if (P.problem == kProblemTensor) {
+          acc += tensor_subcell_entry(P, coef, nsubp, sc, idx);
+        } else if (!P.gauss_coef) {
           if (P.problem == 0)
             acc += (double)coef[sc] * P.Kref[idx];
           else

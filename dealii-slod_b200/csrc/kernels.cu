@@ -30,10 +30,14 @@ cudaError_t upload_params(const Params &p, cudaStream_t st) {
 // ------------------------------------------------------------------------------------------------
 // helpers
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ int nfields() { return cP.problem == 0 ? 1 : 2; }
+__device__ __forceinline__ int nfields() {
+  return cP.problem == 0 ? 1 : (cP.problem == 1 ? 2 : tensor_fields(cP.dim));
+}
 
 // copy the patch's sub-cell coefficients (window origin g.clo) into shared memory, field-major
 // t0 / nt: index and number of the threads taking part (default: the whole CTA)
+// kOneField: only the field d_coef points to (k_patch_factor stages the tensor problem's components one at a time)
+template <bool kOneField = false>
 __device__ void load_coef(const Geom &g, const double *__restrict__ d_coef, double *sCoef, int t0 = -1, int nt = 0) {
   if (t0 < 0) { t0 = threadIdx.x; nt = blockDim.x; }
   const int n = cP.n;
@@ -41,7 +45,7 @@ __device__ void load_coef(const Geom &g, const double *__restrict__ d_coef, doub
   const int nsubp = msx * msy * msz;
   const long long nsub = cP.nsub;
   const long long fstride = (cP.dim == 3) ? nsub * nsub * nsub : nsub * nsub;
-  const int nf = nfields();
+  const int nf = kOneField ? 1 : nfields();
   const int nq = cP.gauss_coef ? (1 << cP.dim) : 1;   // values per sub-cell
   for (int idx = t0; idx < nf * nsubp * nq; idx += nt) {
     const int q = idx % nq;
@@ -143,14 +147,14 @@ k_patch_solve(const int *__restrict__ patch_ids, int n_work, const double *__res
               double *__restrict__ Xbuf, double *__restrict__ Lws, int *__restrict__ status, SolveLayout lay) {
   extern __shared__ double smem[];
   double *myL = Lws + (size_t)blockIdx.x * lay.lws_per_cta;
-  double *sCoef = smem;
+  double *sCoef = lay.gmem_coef ? myL + lay.gcoef_off : smem;
   // Large patches (e.g. 3-D, 4 subdivisions, oversampling 2: half band width 381): the three windows do not fit shared
   // memory and live in the CTA's slice of the global workspace (L2 resident); block barriers order the accesses as
   // they do for shared memory.  Slower, but every configuration the reference's direct solver accepts runs.
   double *sW = lay.gmem_window ? myL + lay.gwin_off : sCoef + lay.coef_doubles;
   double *sR = sW + (size_t)lay.R * lay.ldw;
   double *sLp = sR + (size_t)lay.R * lay.ldr;
-  double *sLd = lay.gmem_window ? sCoef + lay.coef_doubles : sLp + (size_t)lay.R * NB;
+  double *sLd = lay.gmem_window ? (lay.gmem_coef ? smem : sCoef + lay.coef_doubles) : sLp + (size_t)lay.R * NB;
   double *sLinv = sLd + NB * NB;
   double *sYd = sLinv + NB * NB;
   const int tid = threadIdx.x, NT = blockDim.x, lane = tid & 31, warp = tid >> 5;
@@ -564,13 +568,16 @@ namespace slod {
 // ------------------------------------------------------------------------------------------------
 // k_patch_finish : phi = X c (zero on every boundary dof), normalise, A phi
 // ------------------------------------------------------------------------------------------------
+// kGmemCoef: the coefficient window lives in the CTA's slice of lay.coef_ws (patches whose window does not fit shared
+// memory); a template parameter, so that the usual instantiation keeps its registers
+template <bool kGmemCoef>
 __global__ void __launch_bounds__(256, 3)
 k_patch_finish(const int *__restrict__ patch_ids, int n_work, const double *__restrict__ d_coef,
                const double *__restrict__ Xbuf, const double *__restrict__ cvec, double *__restrict__ phi_out,
                double *__restrict__ aphi_out, FinishLayout lay) {
   extern __shared__ double smem[];
-  double *sCoef = smem;
-  double *sPhi = sCoef + lay.coef_doubles;  // [Nf]
+  double *sCoef = kGmemCoef ? lay.coef_ws + (size_t)blockIdx.x * lay.coef_doubles : smem;
+  double *sPhi = kGmemCoef ? smem : sCoef + lay.coef_doubles;  // [Nf]
   double *sC = sPhi + lay.nf_max;           // [ncd]
   int *sRowDof = (int *)(sC + lay.ncd_max);  // [Ni] patch dof of every interior row
   __shared__ double sRed[32];
@@ -693,6 +700,34 @@ k_patch_finish(const int *__restrict__ patch_ids, int n_work, const double *__re
               }
               if (in) av += sCoef[(oz * msy + oy) * msx + ox] * racc;
             }
+          } else if (cP.dim == 3 && cP.problem == kProblemTensor) {
+            // tensor problem in 3-D: the unrolled form of the scalar branch above, one reference-matrix row per Voigt
+            // component (immediate constant-bank operands), weighted by that component's coefficient
+            const int msx = g.m[0] * cP.n, msy = g.m[1] * cP.n, msz = g.m[2] * cP.n;
+            const int nsubp = msx * msy * msz;
+            double pn[27];
+#pragma unroll
+            for (int e = 0; e < 27; ++e) {
+              const int bx = a[0] + e % 3 - 1, by = a[1] + (e / 3) % 3 - 1, bz = a[2] + e / 9 - 1;
+              const bool in = bx >= 0 && bx < g.p[0] && by >= 0 && by < g.p[1] && bz >= 0 && bz < g.p[2];
+              pn[e] = in ? sPhi[(bz * g.p[1] + by) * g.p[0] + bx] : 0.0;
+            }
+#pragma unroll
+            for (int oc = 0; oc < 8; ++oc) {
+              const int ox = a[0] - (oc & 1), oy = a[1] - ((oc >> 1) & 1), oz = a[2] - ((oc >> 2) & 1);
+              if (ox < 0 || ox >= msx || oy < 0 || oy >= msy || oz < 0 || oz >= msz) continue;
+              const int sc = (oz * msy + oy) * msx + ox;
+#pragma unroll
+              for (int f = 0; f < 6; ++f) {
+                double racc = 0.0;
+#pragma unroll
+                for (int lb = 0; lb < 8; ++lb) {
+                  const int ex = (lb & 1) - (oc & 1) + 1, ey = ((lb >> 1) & 1) - ((oc >> 1) & 1) + 1, ez = ((lb >> 2) & 1) - ((oc >> 2) & 1) + 1;
+                  racc += cP.Kq[f][oc * 8 + lb] * pn[(ez * 3 + ey) * 3 + ex];
+                }
+                av += sCoef[f * nsubp + sc] * racc;
+              }
+            }
           } else {
             // sub-cell-wise application of the patch operator: for every sub-cell that contains the node, its local
             // matrix row times the local phi values (include/Diffusion.h:143-193 / include/Elasticity.h:211-284)
@@ -706,7 +741,16 @@ k_patch_finish(const int *__restrict__ patch_ids, int n_work, const double *__re
               const int sc = (oz * msy + oy) * msx + ox;
               const int rowi = (oc * s + ca) * nl;
               double cacc = 0.0;
-              if (!cP.gauss_coef) {
+              if (cP.problem == kProblemTensor) {
+                for (int f = 0; f < tensor_fields(dimv); ++f) {
+                  double racc = 0.0;
+                  for (int lb = 0; lb < nn; ++lb) {
+                    const int nb_ = ((oz + ((lb >> 2) & 1)) * g.p[1] + (oy + ((lb >> 1) & 1))) * g.p[0] + ox + (lb & 1);
+                    racc += cP.Kq[f][rowi + lb] * sPhi[nb_];
+                  }
+                  cacc += sCoef[f * nsubp + sc] * racc;
+                }
+              } else if (!cP.gauss_coef) {
                 double racc = 0.0, lacc = 0.0;
                 for (int lb = 0; lb < nn; ++lb) {
                   const int nb_ = ((oz + ((lb >> 2) & 1)) * g.p[1] + (oy + ((lb >> 1) & 1))) * g.p[0] + ox + (lb & 1);
@@ -1203,9 +1247,10 @@ cudaError_t launch_select_pipeline(const SelectPlan &pl, cudaStream_t st, const 
 cudaError_t launch_patch_finish(int grid, size_t smem, cudaStream_t st, const int *ids, int n_work, const double *coef,
                                 const double *X, const double *cvec, double *phi, double *aphi,
                                 const FinishLayout &lay) {
-  cudaError_t e = cudaFuncSetAttribute(k_patch_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  auto kern = lay.coef_ws ? k_patch_finish<true> : k_patch_finish<false>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  k_patch_finish<<<grid, 256, smem, st>>>(ids, n_work, coef, X, cvec, phi, aphi, lay);
+  kern<<<grid, 256, smem, st>>>(ids, n_work, coef, X, cvec, phi, aphi, lay);
   return cudaGetLastError();
 }
 __global__ void __launch_bounds__(256)

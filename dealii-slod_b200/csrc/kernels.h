@@ -20,6 +20,8 @@ struct SolveLayout {
   long long lws_per_cta;  // doubles of L workspace per CTA
   int gmem_window;        // patches too large for shared memory: the band / RHS / panel windows live in the CTA's
   long long gwin_off;     //   slice of the L workspace instead, at this offset (doubles)
+  int gmem_coef;          // with gmem_window: the coefficient window too (six tensor fields of a large 3-D patch), at
+  long long gcoef_off;    //   this offset of the CTA's slice
 };
 struct DenseLayout {
   long long w_stride;  // doubles per patch in the flux buffer W
@@ -52,6 +54,7 @@ struct FinishLayout {
   int nf_max, ncd_max;
   int ldx;
   long long x_stride;
+  double *coef_ws;     // very large patches: per-CTA coefficient window in global memory (else nullptr)
 };
 
 cudaError_t upload_params(const Params &p, cudaStream_t st);   // stream-ordered upload of the __constant__ block

@@ -294,6 +294,13 @@ k_cg_direction(int nrows, int it, const double *__restrict__ r, const double *__
 // use (geom.h: Kref / Klam / Kq), so the fine FEM problem of assemble_and_solve_fem_problem (source/LOD.cc:1004-1094)
 // is exactly the operator the patch problems restrict.
 
+__device__ __forceinline__ double fine_tensor_entry(const double *__restrict__ d_coef, long long sc, long long fstride,
+                                                 int idx) {
+  double v = 0.0;
+  for (int f = 0; f < tensor_fields(cP.dim); ++f) v += d_coef[f * fstride + sc] * cP.Kq[f][idx];
+  return v;
+}
+
 __device__ __forceinline__ double fine_stiff_entry(const double *__restrict__ d_coef, long long sc, long long fstride,
                                                    int la, int lb, int ca, int cb) {
   const int dim = cP.dim, s = cP.s;
@@ -301,6 +308,7 @@ __device__ __forceinline__ double fine_stiff_entry(const double *__restrict__ d_
   const int idx = (la * s + ca) * nl + (lb * s + cb);
   if (!cP.gauss_coef) {
     if (cP.problem == 0) return d_coef[sc] * cP.Kref[idx];
+    if (cP.problem == kProblemTensor) return fine_tensor_entry(d_coef, sc, fstride, idx);   // never per Gauss point
     return d_coef[fstride + sc] * cP.Kref[idx] + d_coef[sc] * cP.Klam[idx];
   }
   const int nq = 1 << dim;

@@ -116,6 +116,29 @@ __device__ __forceinline__ double stiff_entry_3d(const Geom &g, const double *sC
   return acc;
 }
 
+// The tensor problem's lower-stencil entries, components 1 .. 5 (component 0 is in stw already): each one's field through
+// the same one-field coefficient window and 8 x 8 reference matrix, added to the entry by the thread that wrote it.  Six
+// fields in shared memory would halve k_patch_factor's occupancy; this way its shared-memory plan is the scalar one.
+__device__ __forceinline__ void tensor_stencil_components(const Geom &geo, const double *__restrict__ d_coef, double *sCoef,
+                                                       double *sK, const int *sRowPk, double *stw, int NBLK) {
+  constexpr int nlow = 13;
+  for (int f = 1; f < tensor_fields(3); ++f) {
+    __syncthreads();
+    load_coef<true>(geo, d_coef + (size_t)f * cP.nsub * cP.nsub * cP.nsub, sCoef);
+    for (int i = threadIdx.x; i < 64; i += blockDim.x) sK[i] = cP.Kq[f][i];
+    __syncthreads();
+    for (int item = threadIdx.x; item < NBLK * 8 * (nlow + 1); item += blockDim.x) {
+      const int i = item & 7, e = (item % (8 * (nlow + 1))) >> 3;
+      const int pk = sRowPk[8 * (item / (8 * (nlow + 1))) + i];
+      if (pk >= 0 || !((pk >> (16 + e)) & 1)) continue;   // padding row (keeps its identity entry) or outside the patch
+      const int a[3] = {pk & 31, (pk >> 5) & 31, (pk >> 10) & 31};
+      int dl[3];
+      lower_offset(e, dl);
+      __stcg(stw + item, __ldcg(stw + item) + stiff_entry_3d(geo, sCoef, sK, cP.n, a, dl));
+    }
+  }
+}
+
 // =====================================================================================================================
 // k_patch_factor
 // =====================================================================================================================
@@ -148,7 +171,9 @@ k_patch_factor(const int *__restrict__ patch_ids, int n_work, const double *__re
     while ((offI + 1) * offI / 2 <= tt) ++offI;
     sTileTab[tt] = offI | ((tt - offI * (offI - 1) / 2 + 1) << 8);
   }
-  for (int i = tid; i < 64; i += NT) sK[i] = cP.Kref[i];
+  const bool tensor = cP.problem == kProblemTensor;
+  if (!tensor)
+    for (int i = tid; i < 64; i += NT) sK[i] = cP.Kref[i];
 
   unsigned long long table_key = ~0ull;   // shape key (geom.h) of the patch sRowPk / sDOff were built for
   __shared__ int sNextWork;
@@ -168,7 +193,10 @@ k_patch_factor(const int *__restrict__ patch_ids, int n_work, const double *__re
     // slides -- computing them on the fly in the loop put 1.2 k cycles per step on one warp
     double *stw = stencil_ws + (size_t)blockIdx.x * lay.nip_max * (nlow + 1);
     __syncthreads();
-    load_coef(geo, d_coef, sCoef);
+    // one coefficient field in the window (the scalar problem's only one, the tensor problem's first component)
+    load_coef<true>(geo, d_coef, sCoef);
+    if (tensor)
+      for (int i = tid; i < 64; i += NT) sK[i] = cP.Kq[0][i];
     if (rebuild)
     for (int r = tid; r < 8 * NBLK; r += NT) {
       int pk = 0;
@@ -232,6 +260,7 @@ k_patch_factor(const int *__restrict__ patch_ids, int n_work, const double *__re
     for (int b = 0; b < RB && b < NBLK; ++b) zero_block_row(b);
     for (int item = tid; item < NBLK * 8 * (nlow + 1); item += NT)
       __stcg(stw + item, stencil_item(item / (8 * (nlow + 1)), item % (8 * (nlow + 1))));
+    if (tensor) tensor_stencil_components(geo, d_coef, sCoef, sK, sRowPk, stw, NBLK);
     __syncthreads();
     for (int b = 0; b < RB && b < NBLK; ++b) {   // the first RB block rows of the window
       for (int item = tid; item < 8 * (nlow + 1); item += NT) {

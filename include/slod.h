@@ -67,7 +67,9 @@ enum {
   SLOD_ERR_NUMERIC = 5       /* a patch problem was not SPD / an eigen-solver or CG did not converge */
 };
 
-enum { SLOD_PROBLEM_DIFFUSION = 0, SLOD_PROBLEM_ELASTICITY = 1 };
+/* SLOD_PROBLEM_DIFFUSION_TENSOR: -div(A grad u) with a symmetric positive definite dim x dim tensor A per coefficient
+ * cell (laminates, fibre composites, layered media), dim 2 or 3, spacedim 1; set with slod_set_coefficient_tensor. */
+enum { SLOD_PROBLEM_DIFFUSION = 0, SLOD_PROBLEM_ELASTICITY = 1, SLOD_PROBLEM_DIFFUSION_TENSOR = 2 };
 /* slod_params.device: -1 = current CUDA device; SLOD_DEVICE_NONE = no device, integer maps only
  * (patch lists, DoF maps, CSR pattern) -- every compute call on such a handle returns SLOD_ERR_CUDA. */
 enum { SLOD_DEVICE_CURRENT = -1, SLOD_DEVICE_NONE = -2 };
@@ -75,7 +77,7 @@ enum { SLOD_DEVICE_CURRENT = -1, SLOD_DEVICE_NONE = -2 };
 /* Mirrors LODParameters (include/LOD.h:85-157) + the template arguments <dim, spacedim>. */
 typedef struct {
   int dim;                  /* 2 or 3 (3 only with spacedim 1)                                   */
-  int spacedim;             /* 1 diffusion, 2 = dim elasticity                                    */
+  int spacedim;             /* 1 diffusion (scalar or tensor), 2 = dim elasticity                 */
   int n_global_refinements; /* "Number of global refinements"                 include/LOD.h:95   */
   int n_subdivisions;       /* "Number of subdivisions" (power of two)        include/LOD.h:94   */
   int oversampling;         /* "Oversampling"                                 include/LOD.h:93   */
@@ -101,6 +103,22 @@ const char *slod_last_create_error(void);
  * field 1 = mu.  If the table is finer than the fine sub-cells (eta < h, as in tests/Poisson_LOD_Example)
  * it is sampled at the Gauss points like the reference does; that mode is available in 2-D. */
 int slod_set_coefficient(slod_ctx *ctx, int field, int eta_refinement, const double *cellwise, size_t n);
+
+/* the coefficient of a SLOD_PROBLEM_DIFFUSION_TENSOR handle: `cells` is [n_cells][dim (dim + 1) / 2], one symmetric
+ * tensor per cell of the (2^eta_refinement)^dim grid, lexicographic x fastest, each in Voigt order
+ *   2-D: a_xx, a_yy, a_xy          3-D: a_xx, a_yy, a_zz, a_yz, a_xz, a_xy.
+ * Sub-cell matrices are sum_f a_f K_f with K_f = d_a phi_i d_b phi_j (+ d_b phi_i d_a phi_j for a != b) for component
+ * f = (a, b), integrated like the scalar problem's.  Every argument is checked before the device (a maps-only handle
+ * checks them too): another problem, n_cells != (2^eta_refinement)^dim, a non-finite entry or a cell that is not
+ * positive definite (a Cholesky factorisation with positive pivots) -> SLOD_ERR_INVALID, and slod_last_error names the
+ * first offending cell; a table finer than the fine sub-cells (eta < h) -> SLOD_ERR_UNSUPPORTED (the per-Gauss-point mode
+ * is scalar only).  slod_set_coefficient on a tensor handle returns SLOD_ERR_INVALID: setting one component at a time
+ * could leave an indefinite tensor between calls.  Each component is then stored and expanded onto the sub-cells like a
+ * slod_set_coefficient field.  slod_update_basis compares every component (a changed off-diagonal entry marks its
+ * cell), and a checkpoint records the problem, so it loads only into a tensor handle.  Where the six-field window of a
+ * 3-D patch fits no shared-memory plan (4 subdivisions), the SIMT solver and the finish kernel read it from global
+ * memory: such handles have the scalar handle's plan. */
+int slod_set_coefficient_tensor(slod_ctx *ctx, int eta_refinement, const double *cells, size_t n_cells);
 
 /* the kernel plan slod_create chose from the largest patch shape (read only; a maps-only handle plans for 227 KB of
  * shared memory per block, as on a B200).  out[8]:
